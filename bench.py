@@ -10,6 +10,7 @@ world > 1).  Point sampling, rhs evaluation and Adam are outside the step (SURVE
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference            # the reference's own CPU path on the host cores
+    python bench.py --dump-outputs out/         # also save the last timed step's loss and gradients as .npy
 
 The one JSON line carries, besides the contract's keys: ``roofline`` (tensor pipe), ``cpu_baseline`` (the reference's
 CPU path in the same run), ``parity`` (loss / gradient of the first 2^16 benchmarked points against the reference
@@ -460,7 +461,13 @@ def main():
     ap.add_argument("--points", type=int, default=N_PER_GPU, help="points per GPU (default 2^22, the metric's config)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and parameter gradients of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs saves the outputs of --impl b200 only")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -537,7 +544,7 @@ def main():
     barrier()
     e0.record()
     for i in range(args.steps):
-        step(i)
+        loss = step(i)
     e1.record()
     barrier()
     launches = ops.launch_count() - launches0      # counted by the library at its launch sites
@@ -547,6 +554,14 @@ def main():
     ops.KERNEL_EVENTS = None
     kernel_ms = [a.elapsed_time(b) for a, b in kev]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives from its last step: the loss and every parameter's .grad (the
+        # gradient is all-reduced, so rank 0 holds the global result); copied before the end-to-end steps reuse them
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        outs = {"loss": loss, **{f"grad.{n}": p.grad for n, p in model.named_parameters()}}
+        for name, t in outs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.detach().float().cpu().numpy())
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import assert_grads_close, flat, grads_from, load_golden, net_from
+from conftest import assert_grads_close, flat, grads_from, load_golden, net_from, stored_entries
 from oracle import autograd_ref as AR
 from oracle import jets_numpy as O
 
@@ -435,11 +435,11 @@ def test_numpy_oracle_config5_kh1d():
     env = dict(kind=O.ENV_EXPWIN, lo=-L, hi=L)
     loss, gWs, gbs, dE = O.eigen_pinn_loss(uW, ub, X, O.SIN, env, alpha=-0.5, beta=V, E=E)
     assert abs(loss - g["pinn_loss"]) <= TOL * max(1, abs(g["pinn_loss"]))
-    assert_grads_close((gWs, gbs), grads_from(g, "pinn_"), TOL, "pinn")
+    assert_grads_close(stored_entries((gWs, gbs), g, "pinn_"), grads_from(g, "pinn_"), TOL, "pinn")
     assert abs(dE - float(g["pinn_gE"])) <= TOL * max(1, abs(float(g["pinn_gE"])))
     loss, gWs, gbs, _ = O.rayleigh_loss(uW, ub, X, O.SIN, env, a=0.5, beta=V, eps_out=1e-12, scale=2 * L)
     assert abs(loss - g["drm_loss"]) <= TOL * max(1, abs(g["drm_loss"]))
-    assert_grads_close((gWs, gbs), grads_from(g, "drm_"), TOL, "drm")
+    assert_grads_close(stored_entries((gWs, gbs), g, "drm_"), grads_from(g, "drm_"), TOL, "drm")
     raw = dict(kind=O.ENV_NONE)
     m, Gu, Gv, dE1 = O.wan_means(dict(Ws=wW, bs=wb, act=O.SIN, env=raw), dict(Ws=vW, bs=vb, act=O.SIN, env=raw), X, None,
                                  -L, L, a=0.5, beta=V, E=E, eps_den=1e-10)
@@ -449,8 +449,8 @@ def test_numpy_oracle_config5_kh1d():
     assert abs(ratio ** 2 - g["wan_pde"]) <= TOL * max(1, abs(g["wan_pde"]))
     assert abs((2 * L * m3 - 1.0) ** 2 - g["wan_norm"]) <= TOL * max(1, abs(g["wan_norm"]))
     d = [2 * ratio * 2 * L / den, -2 * ratio * 2 * L * m1 * 2 * L / den ** 2, 2 * (2 * L * m3 - 1.0) * 2 * L, 0.0]
-    assert_grads_close(_combine(Gu, d), grads_from(g, "wan_u_"), TOL, "wan/u")
-    assert_grads_close(_combine(Gv, d), grads_from(g, "wan_v_"), TOL, "wan/v")
+    assert_grads_close(stored_entries(_combine(Gu, d), g, "wan_u_"), grads_from(g, "wan_u_"), TOL, "wan/u")
+    assert_grads_close(stored_entries(_combine(Gv, d), g, "wan_v_"), grads_from(g, "wan_v_"), TOL, "wan/v")
     assert abs(d[0] * dE1 - float(g["wan_gE"])) <= TOL * max(1, abs(float(g["wan_gE"])))
 
 
@@ -467,8 +467,8 @@ def test_numpy_oracle_config5_qho1d_wan():
     assert abs(m1 * m1 / (m2 + 1e-8) - g["loss_pde"]) <= TOL * max(1, abs(g["loss_pde"]))
     assert abs((2 * L * m3 - 1.0) ** 2 - g["loss_norm"]) <= TOL * max(1, abs(g["loss_norm"]))
     dtot = _wan_dtot(m1, m2, m3, 2 * L)
-    assert_grads_close(_combine(Gu, dtot), grads_from(g, "tot_u_"), TOL, "tot/u")
-    assert_grads_close(_combine(Gv, dtot), grads_from(g, "tot_v_"), TOL, "tot/v")
+    assert_grads_close(stored_entries(_combine(Gu, dtot), g, "tot_u_"), grads_from(g, "tot_u_"), TOL, "tot/u")
+    assert_grads_close(stored_entries(_combine(Gv, dtot), g, "tot_v_"), grads_from(g, "tot_v_"), TOL, "tot/v")
     assert abs(dtot[0] * dE1 - float(g["tot_gE"])) <= TOL * max(1, abs(float(g["tot_gE"])))
 
 
