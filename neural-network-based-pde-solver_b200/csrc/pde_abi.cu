@@ -55,6 +55,12 @@ struct Plan {
 
 inline long long rup(long long x, long long m) { return (x + m - 1) / m * m; }
 
+// Scalar parameters of a validated network: W0 [H][D], b0 [H], (n_h - 1) x (W [H][H], b [H]), wL [H], bL.
+inline long long param_count(const pde_net* net) {
+  const long long H = net->widths[1], D = net->dim, n_h = net->n_linear - 1;
+  return H * D + H + (n_h - 1) * (H * H + H) + H + 1;
+}
+
 int validate_net(const pde_net* net) {
   if (!net) return PDE_ERR_INVALID;
   if (net->dtype != PDE_F32 && net->dtype != PDE_F64) return PDE_ERR_INVALID;
@@ -114,7 +120,7 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
   p.off_gwL = p.off_gW + (long long)(p.n_h - 1) * (HH + p.Hp);
   p.off_gbL = p.off_gwL + p.Hp;
   p.PP = rup(p.off_gbL + 1, 4);
-  p.n_params = (long long)p.H * p.D + p.H + (long long)(p.n_h - 1) * ((long long)p.H * p.H + p.H) + p.H + 1;
+  p.n_params = param_count(net);
 
   KernelInfo ki = net_kernel_info<T>(p.D, order);
   if (!ki.fn) return PDE_ERR_UNSUPPORTED;
@@ -258,6 +264,23 @@ int run_net(const pde_net* net, int order, int mode, const pde_envelope* env, co
   return PDE_OK;
 }
 
+template <typename T>
+cudaError_t run_wan(const pde_wan* wan, const void* X, long long n, const void* Ju, const void* Jv, const void* seed,
+                    double inv_n, void* sums, void* Jbar_u, void* Jbar_v, void* workspace, int blocks, cudaStream_t st) {
+  WanArgs<T> a;
+  memset(&a, 0, sizeof(a));
+  a.D = wan->dim; a.n = n;
+  a.X = static_cast<const T*>(X); a.Ju = static_cast<const T*>(Ju); a.Jv = static_cast<const T*>(Jv);
+  a.f = static_cast<const T*>(wan->f); a.beta = static_cast<const T*>(wan->beta);
+  a.energy = static_cast<const T*>(wan->energy); a.seed = static_cast<const T*>(seed);
+  a.alpha = (T)wan->alpha; a.beta_const = (T)wan->beta_const; a.energy_const = (T)wan->energy_const;
+  a.w_lo = (T)wan->w_lo; a.w_hi = (T)wan->w_hi; a.eps_den = (T)wan->eps_den; a.inv_n = (T)inv_n;
+  fill_env<T>(&wan->env_u, &a.env_u); fill_env<T>(&wan->env_v, &a.env_v);
+  a.Jbar_u = static_cast<T*>(Jbar_u); a.Jbar_v = static_cast<T*>(Jbar_v);
+  a.psums = static_cast<double*>(workspace); a.sums = static_cast<T*>(sums); a.blocks = blocks;
+  return launch_wan<T>(st, a);
+}
+
 }  // namespace
 
 extern "C" {
@@ -280,8 +303,7 @@ int pde_param_count(const pde_net* net, int64_t* n_params) {
   int st = validate_net(net);
   if (st) return st;
   if (!n_params) return PDE_ERR_INVALID;
-  const long long H = net->widths[1], D = net->dim, n_h = net->n_linear - 1;
-  *n_params = H * D + H + (n_h - 1) * (H * H + H) + H + 1;
+  *n_params = param_count(net);
   return PDE_OK;
 }
 
@@ -433,34 +455,10 @@ int pde_wan_pointwise(const pde_wan* wan, const void* X, int64_t n_points, const
   if (blocks > dv.sms * 4) blocks = dv.sms * 4;
   if (workspace_bytes < (size_t)blocks * 8 * sizeof(double)) return PDE_ERR_WORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  cudaError_t err;
-  if (wan->dtype == PDE_F64) {
-    WanArgs<double> a;
-    memset(&a, 0, sizeof(a));
-    a.D = wan->dim; a.n = n_points;
-    a.X = (const double*)X; a.Ju = (const double*)Ju; a.Jv = (const double*)Jv;
-    a.f = (const double*)wan->f; a.beta = (const double*)wan->beta; a.energy = (const double*)wan->energy;
-    a.seed = (const double*)seed;
-    a.alpha = wan->alpha; a.beta_const = wan->beta_const; a.energy_const = wan->energy_const;
-    a.w_lo = wan->w_lo; a.w_hi = wan->w_hi; a.eps_den = wan->eps_den; a.inv_n = inv_n;
-    fill_env<double>(&wan->env_u, &a.env_u); fill_env<double>(&wan->env_v, &a.env_v);
-    a.Jbar_u = (double*)Jbar_u; a.Jbar_v = (double*)Jbar_v;
-    a.psums = (double*)workspace; a.sums = (double*)sums; a.blocks = blocks;
-    err = launch_wan<double>(st, a);
-  } else {
-    WanArgs<float> a;
-    memset(&a, 0, sizeof(a));
-    a.D = wan->dim; a.n = n_points;
-    a.X = (const float*)X; a.Ju = (const float*)Ju; a.Jv = (const float*)Jv;
-    a.f = (const float*)wan->f; a.beta = (const float*)wan->beta; a.energy = (const float*)wan->energy;
-    a.seed = (const float*)seed;
-    a.alpha = (float)wan->alpha; a.beta_const = (float)wan->beta_const; a.energy_const = (float)wan->energy_const;
-    a.w_lo = (float)wan->w_lo; a.w_hi = (float)wan->w_hi; a.eps_den = (float)wan->eps_den; a.inv_n = (float)inv_n;
-    fill_env<float>(&wan->env_u, &a.env_u); fill_env<float>(&wan->env_v, &a.env_v);
-    a.Jbar_u = (float*)Jbar_u; a.Jbar_v = (float*)Jbar_v;
-    a.psums = (double*)workspace; a.sums = (float*)sums; a.blocks = blocks;
-    err = launch_wan<float>(st, a);
-  }
+  const cudaError_t err =
+      wan->dtype == PDE_F64
+          ? run_wan<double>(wan, X, n_points, Ju, Jv, seed, inv_n, sums, Jbar_u, Jbar_v, workspace, blocks, st)
+          : run_wan<float>(wan, X, n_points, Ju, Jv, seed, inv_n, sums, Jbar_u, Jbar_v, workspace, blocks, st);
   return err == cudaSuccess ? PDE_OK : PDE_ERR_CUDA;
 }
 

@@ -17,6 +17,7 @@ equals the single big batch exactly, also for functions of means (SURVEY.md §8e
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 from dataclasses import dataclass, field
 from typing import Optional, Sequence
 
@@ -221,6 +222,10 @@ def _stream(device):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
 _unflatten = getattr(torch._C._nn, "unflatten_dense_tensors", None)
 
 
@@ -297,9 +302,10 @@ def combine_forward(buf, nparam, n_tot, group, fused):
     reverse sweep was fused into the same launch, else the sums only) makes every rank hold the
     single-big-batch values; returns the means.  (SURVEY.md §8e: sums and gradient vectors are
     reduced, never per-rank losses.)"""
+    sums = _row_sums(buf, nparam)
     if group is not None:
-        _all_reduce(buf if fused else buf[nparam + 1:], group)
-    return buf[nparam + 1:] / n_tot
+        _all_reduce(buf if fused else sums, group)
+    return sums / n_tot
 
 
 def combine_backward(buf, nparam, group):
@@ -365,13 +371,49 @@ class ProgramSpec:
     beta_const: float = 0.0
     energy_const: float = 0.0
 
+    def to_c(self, f=None, beta=None, energy=None) -> L.Program:
+        """The pde_program descriptor; ``f`` / ``beta`` / ``energy``: per-point (scalar) device tensors or None."""
+        p = L.Program()
+        p.kind, p.alpha, p.beta_const, p.energy_const = self.kind, self.alpha, self.beta_const, self.energy_const
+        p.f, p.beta, p.energy = _ptr(f), _ptr(beta), _ptr(energy)
+        return p
+
+
+_MSE = ProgramSpec(L.PROG_MSE)
+
+
+def _row_sums(row, nparam):
+    """The sums of a [grad (nparam) | dE (1) | sums (K)] row."""
+    return row[nparam + 1:]
+
+
+def _residual_row(cnet, cenv, prog, X, n, inv_n, ws, row, nparam, seed=None, sums=None, want_grad=True, ar=None):
+    """One residual-program launch into ``row`` = [grad (nparam) | dE (1) | sums (K)] (1-D, contiguous): the layout
+    that pde_residual_loss_grad writes and that the all-reduce and pde_residual_loss_grad_exchange carry.
+
+    ``seed``: device cotangents of the means (seeded reverse sweep); ``sums``: write the sums there instead of into
+    the row; ``want_grad=False``: sums only (``row`` may then be None); ``ar``: an ``NvlinkAllReduce`` whose exchange
+    of the whole row is folded into the reduction launch."""
+    lib, st = L.load(), _stream(X.device)
+    if ar is not None:
+        L.check(lib.pde_residual_loss_grad_exchange(C.byref(cnet), C.byref(cenv), C.byref(prog), X.data_ptr(), n,
+                                                    _ptr(seed), inv_n, row.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                    C.byref(ar.peers), ar.slot, ar.seq.data_ptr(), st),
+                "pde_residual_loss_grad_exchange")
+        return
+    es = X.element_size()
+    gptr = row.data_ptr() if want_grad else None
+    sptr = sums.data_ptr() if sums is not None else row.data_ptr() + (nparam + 1) * es
+    L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(prog), X.data_ptr(), n, _ptr(seed), inv_n,
+                                       sptr, gptr, gptr + nparam * es if want_grad else None, ws.data_ptr(), ws.numel(),
+                                       st), "pde_residual_loss_grad")
+
 
 class _Residual(torch.autograd.Function):
     """means[K] of a residual program; backward = sum_k gbar_k * d(mean_k)/d(theta, E)."""
 
     @staticmethod
     def forward(ctx, net, env, spec, group, n_global, need_grad, X, f, beta, energy, *params):
-        lib = L.load()
         ps = [p.detach().contiguous() for p in params]
         cnet = net.to_c(ps)
         n = X.shape[0]
@@ -384,29 +426,13 @@ class _Residual(torch.autograd.Function):
         fused = (K == 1) and need_grad
         # one buffer [grad (nparam) | dE (1) | sums (K)] so that one all-reduce covers everything
         buf = torch.zeros(nparam + 1 + K, dtype=dt, device=dev)
-        prog = L.Program()
-        prog.kind, prog.alpha, prog.beta_const, prog.energy_const = spec.kind, spec.alpha, spec.beta_const, spec.energy_const
-        prog.f = f.data_ptr() if f is not None else None
-        prog.beta = beta.data_ptr() if beta is not None else None
         e_dev = energy.detach().reshape(1).to(dt) if energy is not None else None
-        prog.energy = e_dev.data_ptr() if e_dev is not None else None
-        cenv = env.to_c()
+        prog, cenv = spec.to_c(f, beta, e_dev), env.to_c()
         ws = _ws_for(cnet, order, n, dev)
-        gptr = buf.data_ptr() if fused else None
-        eptr = buf.data_ptr() + nparam * buf.element_size() if fused else None
-        sptr = buf.data_ptr() + (nparam + 1) * buf.element_size()
+        # exchange folded into the reduction of the per-CTA partials: no separate all-reduce launch
         ar = _exchange_for(buf, group) if (fused and FUSE_EXCHANGE) else None
         with torch.cuda.device(dev), _timed(dev):
-            if ar is not None:
-                # exchange folded into the reduction of the per-CTA partials: no separate all-reduce launch
-                L.check(lib.pde_residual_loss_grad_exchange(C.byref(cnet), C.byref(cenv), C.byref(prog), X.data_ptr(), n, None,
-                                                            1.0 / n_tot, buf.data_ptr(), ws.data_ptr(), ws.numel(),
-                                                            C.byref(ar.peers), ar.slot, ar.seq.data_ptr(), _stream(dev)),
-                        "pde_residual_loss_grad_exchange")
-            else:
-                L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(prog), X.data_ptr(), n, None,
-                                                   1.0 / n_tot, sptr, gptr, eptr, ws.data_ptr(), ws.numel(), _stream(dev)),
-                        "pde_residual_loss_grad")
+            _residual_row(cnet, cenv, prog, X, n, 1.0 / n_tot, ws, buf, nparam, want_grad=fused, ar=ar)
         means = combine_forward(buf, nparam, n_tot, None if ar is not None else group, fused)
         ctx.fused = fused
         ctx.has_energy = energy is not None
@@ -428,28 +454,16 @@ class _Residual(torch.autograd.Function):
             gE = (buf[nparam] * gmeans[0]) if ctx.has_energy else None
             grads = _split_flat(flat, ctx.ps)
         else:
-            lib = L.load()
             X, f, beta, e_dev, *ps = ctx.saved_tensors
             cnet = net.to_c(ps)
             n = X.shape[0]
             dev, dt = X.device, X.dtype
             nparam = sum(p.numel() for p in ps)
             buf = torch.zeros(nparam + 1 + ctx.K, dtype=dt, device=dev)
-            prog = L.Program()
-            prog.kind, prog.alpha, prog.beta_const, prog.energy_const = spec.kind, spec.alpha, spec.beta_const, spec.energy_const
-            prog.f = f.data_ptr() if f is not None else None
-            prog.beta = beta.data_ptr() if beta is not None else None
-            prog.energy = e_dev.data_ptr() if e_dev is not None else None
-            cenv = env.to_c()
-            order = _program_info(spec.kind)[1]
             seed = gmeans.detach().to(dt).contiguous()
-            ws = _ws_for(cnet, order, n, dev)
+            ws = _ws_for(cnet, _program_info(spec.kind)[1], n, dev)
             with torch.cuda.device(dev):
-                L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(prog), X.data_ptr(), n,
-                                                   seed.data_ptr(), 1.0 / n_tot,
-                                                   buf.data_ptr() + (nparam + 1) * buf.element_size(), buf.data_ptr(),
-                                                   buf.data_ptr() + nparam * buf.element_size(), ws.data_ptr(),
-                                                   ws.numel(), _stream(dev)), "pde_residual_loss_grad")
+                _residual_row(cnet, env.to_c(), spec.to_c(f, beta, e_dev), X, n, 1.0 / n_tot, ws, buf, nparam, seed=seed)
             flat, dE = combine_backward(buf, nparam, group)
             grads = _split_flat(flat, ps)
             gE = dE if ctx.has_energy else None
@@ -470,15 +484,10 @@ def _global_count(n, group, n_global):
     return n * dist.get_world_size(group)
 
 
-def residual_means(model, X, spec: ProgramSpec, env: EnvelopeSpec = NO_ENVELOPE, f=None, beta=None, energy=None,
-                   group=None, n_global: Optional[int] = None) -> torch.Tensor:
-    """Means of the program's per-point quantities, differentiable w.r.t. the network parameters
-    (and the scalar ``energy`` when it is a tensor that requires grad)."""
-    X = _points(X)
-    net = _Net(model, X)
-    n = X.shape[0]
-    n_global = _global_count(n, group, n_global)
-
+def _coefficients(spec, X, f, beta, energy):
+    """(spec, f, beta, energy) of one call: a float ``beta`` / ``energy`` folded into the spec's constants, per-point
+    ``f`` / ``beta`` as flat contiguous tensors of the points' dtype with one value per point, a tensor ``energy`` as
+    given.  Already conforming coefficients are passed through without a copy."""
     def coef(t):
         if t is None:
             return None
@@ -488,23 +497,29 @@ def residual_means(model, X, spec: ProgramSpec, env: EnvelopeSpec = NO_ENVELOPE,
         t = t.reshape(-1)
         if not t.is_contiguous():
             t = t.contiguous()
-        if t.numel() != n or t.device != X.device:
+        if t.numel() != X.shape[0] or t.device != X.device:
             raise ValueError("per-point coefficient must have one value per point on the points' device")
         return t
 
-    e = None
-    if energy is not None:
-        if torch.is_tensor(energy):
-            e = energy
-        else:
-            spec = ProgramSpec(spec.kind, spec.alpha, spec.beta_const, float(energy))
+    if energy is not None and not torch.is_tensor(energy):
+        spec, energy = dataclasses.replace(spec, energy_const=float(energy)), None
     if beta is not None and not torch.is_tensor(beta):
-        spec = ProgramSpec(spec.kind, spec.alpha, float(beta), spec.energy_const)
-        beta = None
+        spec, beta = dataclasses.replace(spec, beta_const=float(beta)), None
+    return spec, coef(f), coef(beta), energy
+
+
+def residual_means(model, X, spec: ProgramSpec, env: EnvelopeSpec = NO_ENVELOPE, f=None, beta=None, energy=None,
+                   group=None, n_global: Optional[int] = None) -> torch.Tensor:
+    """Means of the program's per-point quantities, differentiable w.r.t. the network parameters
+    (and the scalar ``energy`` when it is a tensor that requires grad)."""
+    X = _points(X)
+    net = _Net(model, X)
+    n_global = _global_count(X.shape[0], group, n_global)
+    spec, f, beta, e = _coefficients(spec, X, f, beta, energy)
     # (grad mode is off inside Function.forward, so decide here whether the fused reverse sweep runs)
     need_grad = torch.is_grad_enabled() and (any(p.requires_grad for p in net.params) or
                                              (e is not None and e.requires_grad))
-    return _Residual.apply(net, env, spec, group, n_global, need_grad, X, coef(f), coef(beta), e, *net.params)
+    return _Residual.apply(net, env, spec, group, n_global, need_grad, X, f, beta, e, *net.params)
 
 
 def residual_mean(model, X, spec: ProgramSpec, env: EnvelopeSpec = NO_ENVELOPE, **kw) -> torch.Tensor:
@@ -528,6 +543,18 @@ class WanSpec:
     w_hi: float = 2.0
     eps_den: float = 0.0
 
+    def to_c(self, dtype, dim, env_u, env_v, f=None, beta=None, energy=None) -> L.Wan:
+        """The pde_wan descriptor for points of ``dtype`` / ``dim``; ``f`` / ``beta`` / ``energy``: per-point (scalar)
+        device tensors or None."""
+        w = L.Wan()
+        w.dtype = L.F64 if dtype == torch.float64 else L.F32
+        w.dim = dim
+        w.alpha, w.beta_const, w.energy_const = self.alpha, self.beta_const, self.energy_const
+        w.w_lo, w.w_hi, w.eps_den = self.w_lo, self.w_hi, self.eps_den
+        w.f, w.beta, w.energy = _ptr(f), _ptr(beta), _ptr(energy)
+        w.env_u, w.env_v = env_u.to_c(), env_v.to_c()
+        return w
+
 
 class _WanPoint(torch.autograd.Function):
     """means[4] (+ d mean0/dE) from the two networks' jets; backward produces jet cotangents."""
@@ -538,16 +565,8 @@ class _WanPoint(torch.autograd.Function):
         n, d = X.shape
         dev, dt = X.device, X.dtype
         n_tot = float(n if n_global is None else n_global)
-        w = L.Wan()
-        w.dtype = L.F64 if dt == torch.float64 else L.F32
-        w.dim = d
-        w.alpha, w.beta_const, w.energy_const = spec.alpha, spec.beta_const, spec.energy_const
-        w.w_lo, w.w_hi, w.eps_den = spec.w_lo, spec.w_hi, spec.eps_den
-        w.f = f.data_ptr() if f is not None else None
-        w.beta = beta.data_ptr() if beta is not None else None
         e_dev = energy.detach().reshape(1).to(dt) if energy is not None else None
-        w.energy = e_dev.data_ptr() if e_dev is not None else None
-        w.env_u, w.env_v = env_u.to_c(), env_v.to_c()
+        w = spec.to_c(dt, d, env_u, env_v, f, beta, e_dev)
         sums = torch.empty(5, dtype=dt, device=dev)    # all five written by the launch (wan_finish_kernel)
         ws = _workspace(dev, 1 << 20)
         Juc, Jvc = Ju.detach().contiguous(), Jv.detach().contiguous()
@@ -569,15 +588,7 @@ class _WanPoint(torch.autograd.Function):
         X, f, beta, e_dev, Ju, Jv, sums = ctx.saved_tensors
         n, d = X.shape
         dev, dt = X.device, X.dtype
-        w = L.Wan()
-        w.dtype = L.F64 if dt == torch.float64 else L.F32
-        w.dim = d
-        w.alpha, w.beta_const, w.energy_const = spec.alpha, spec.beta_const, spec.energy_const
-        w.w_lo, w.w_hi, w.eps_den = spec.w_lo, spec.w_hi, spec.eps_den
-        w.f = f.data_ptr() if f is not None else None
-        w.beta = beta.data_ptr() if beta is not None else None
-        w.energy = e_dev.data_ptr() if e_dev is not None else None
-        w.env_u, w.env_v = env_u.to_c(), env_v.to_c()
+        w = spec.to_c(dt, d, env_u, env_v, f, beta, e_dev)
         seed = gmeans.detach().to(dt).contiguous()
         Jbu, Jbv = torch.empty_like(Ju), torch.empty_like(Jv)
         scratch = torch.empty(5, dtype=dt, device=dev)
@@ -607,30 +618,11 @@ def wan_means(u_model, v_model, X, spec: WanSpec, env_u=NO_ENVELOPE, env_v=NO_EN
     points with the other network's parameters switched off (IPW_1D_WAN.py:186-194, KH_1D.py:343-352).
     """
     X = _points(X)
-    n = X.shape[0]
-    n_global = _global_count(n, group, n_global)
-
-    def coef(t):
-        if t is None:
-            return None
-        t = t.detach().to(X.dtype).reshape(-1).contiguous()
-        if t.numel() != n or t.device != X.device:
-            raise ValueError("per-point coefficient must have one value per point on the points' device")
-        return t
-
-    e = None
-    if energy is not None:
-        if torch.is_tensor(energy):
-            e = energy
-        else:
-            spec = WanSpec(spec.alpha, spec.beta_const, float(energy), spec.w_lo, spec.w_hi, spec.eps_den)
-    if beta is not None and not torch.is_tensor(beta):
-        spec = WanSpec(spec.alpha, float(beta), spec.energy_const, spec.w_lo, spec.w_hi, spec.eps_den)
-        beta = None
+    n_global = _global_count(X.shape[0], group, n_global)
+    spec, f, beta, e = _coefficients(spec, X, f, beta, energy)
     Ju = mlp_jets(u_model, X, 1) if u_jets is None else _check_jets(u_jets, X)
     Jv = mlp_jets(v_model, X, 1) if v_jets is None else _check_jets(v_jets, X)
-    means = _WanPoint.apply(spec, env_u, env_v, group, n_global, X, coef(f), coef(beta), e, Ju, Jv)
-    return means
+    return _WanPoint.apply(spec, env_u, env_v, group, n_global, X, f, beta, e, Ju, Jv)
 
 
 class _WanScalars(torch.autograd.Function):
@@ -691,7 +683,5 @@ def all_reduce_grads(params, group=None):
         return
     flat = torch.cat([g.reshape(-1) for g in gs])
     dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
-    o = 0
-    for g in gs:
-        k = g.numel()
-        g.copy_(flat[o:o + k].view_as(g)); o += k
+    for g, r in zip(gs, _split_flat(flat, gs)):
+        g.copy_(r)

@@ -118,12 +118,8 @@ def boundary_loss_dirichlet(model, L, N_b_per_face, dim, device, *, group=None):
         for at_L in (False, True):
             X = torch.rand(N_b_per_face, dim, device=device, dtype=dtype) * L
             X[:, i] = L if at_L else 0.0
-            n_glob = None
-            if group is not None:
-                import torch.distributed as dist
-                n_glob = N_b_per_face * dist.get_world_size(group)
-            losses.append(residual_mean(model, X, ProgramSpec(_lib.PROG_MSE), _envelope(model, L), group=group,
-                                        n_global=n_glob))
+            # (with group, residual_mean counts N_b_per_face points on every rank)
+            losses.append(residual_mean(model, X, ProgramSpec(_lib.PROG_MSE), _envelope(model, L), group=group))
     return sum(losses) / len(losses)
 
 

@@ -23,7 +23,7 @@ from typing import Optional, Sequence
 import torch
 
 from . import _lib as L
-from .ops import NO_ENVELOPE, EnvelopeSpec, ProgramSpec, _Net, _stream, _ws_for
+from .ops import _MSE, EnvelopeSpec, ProgramSpec, _Net, _residual_row, _row_sums, _split_flat, _stream, _ws_for
 
 
 def sample_points_rhs(n, dim, L_box, ks=None, *, dtype=torch.float32, device="cuda", seed=0, offset=0, lo=0.0,
@@ -65,6 +65,51 @@ def rank_offset(rank):
     epoch count, so that every rank draws its own points (the reference is single-process; with the default seed
     identical draws on every rank would make the global batch n points repeated world times)."""
     return int(rank) << 40
+
+
+TERMS = ('pde', 'bc', 'data', 'norm')
+
+
+def _term_weights(weights, rb, has_data, pde=1.0):
+    """Weights of the loss terms like the reference's ``weights`` argument (Poisson_ND.py:169-173): bc 1e4 for a soft
+    Dirichlet constraint (``rb``), data 1e3 when data points are given, norm 0; ``weights`` overrides them and may
+    only name the terms in ``TERMS``."""
+    w = {'pde': float(pde), 'bc': 1e4 if rb else 0.0, 'data': 1e3 if has_data else 0.0, 'norm': 0.0}
+    if weights:
+        unknown = set(weights) - set(TERMS)
+        if unknown:
+            raise ValueError(f"unknown loss terms {sorted(unknown)}")
+        w.update({k: float(v) for k, v in weights.items()})
+    return w
+
+
+class _FacePoints:
+    """``n_boundary`` points split evenly over the 2d faces of [0, L]^dim (Poisson_ND.py:225), redrawn into ``X`` by
+    ``draw``: one uniform draw, then face k = (coordinate k // 2, side k % 2) gets that coordinate replaced by 0 or L
+    (:133-139).  Equal counts per face, so the mean over all face points is the mean of the per-face means."""
+    KEY = 0x5851F42D4C957F2D   # xor-ed into the seed: the face draws are independent of the interior draws
+
+    def __init__(self, n_boundary, dim, L_box, dtype, device):
+        per_face = max(1, int(n_boundary) // (2 * dim))
+        self.n, self.dim, self.L = 2 * dim * per_face, dim, float(L_box)
+        self.X = torch.empty(self.n, dim, dtype=dtype, device=device)
+        keep = torch.ones(2 * dim, 1, dim, dtype=dtype, device=device)
+        put = torch.zeros(2 * dim, 1, dim, dtype=dtype, device=device)
+        for k in range(2 * dim):
+            keep[k, 0, k // 2] = 0.0
+            put[k, 0, k // 2] = self.L if k % 2 else 0.0
+        self._keep = keep.expand(-1, per_face, -1).reshape(self.n, dim).contiguous()
+        self._put = put.expand(-1, per_face, -1).reshape(self.n, dim).contiguous()
+
+    def draw(self, seed, offset, counter, advance=False):
+        """Fresh face points from Philox block ``offset`` + ``counter`` (a device int64 draw counter, incremented
+        after the uniform draw when ``advance``)."""
+        sample_points_rhs(self.n, self.dim, self.L, None, dtype=self.X.dtype, device=self.X.device, seed=seed ^ self.KEY,
+                          offset=offset, offset_add=counter, out=(self.X, None, None))
+        if advance:
+            counter.add_(1)
+        torch.addcmul(self._put, self.X, self._keep, out=self.X)
+        return self.X
 
 
 class FusedAdam:
@@ -222,7 +267,7 @@ class FusedTrainer:
                peer memory; 'nccl': torch.distributed.all_reduce)
     """
 
-    TERMS = ('pde', 'bc', 'data', 'norm')
+    TERMS = TERMS
 
     def __init__(self, model, L_box=2.0, ks=None, method='PINN', n_interior=20000, lr=1e-3, betas=(0.9, 0.999), eps=1e-8,
                  weight_pde=1.0, X=None, f=None, resample=False, seed=0, n_test=0, history=0, graph=True, group=None,
@@ -256,14 +301,8 @@ class FusedTrainer:
             self.f = (f if f is not None else sample_points_rhs(0, 0, self.L, self.ks, X=self.X)[2]).detach().to(self.dtype).reshape(-1).contiguous()
             if self.resample:
                 raise ValueError("resample=True draws its own points; do not pass X")
-        # term weights (Poisson_ND.py:169-173)
         rb = getattr(model, "bc_mode", "FBC") == 'RB' and envelope is None
-        self.w = {'pde': float(weight_pde), 'bc': 1e4 if rb else 0.0, 'data': 1e3 if X_data is not None else 0.0, 'norm': 0.0}
-        if weights:
-            unknown = set(weights) - set(self.TERMS)
-            if unknown:
-                raise ValueError(f"unknown loss terms {sorted(unknown)}")
-            self.w.update({k: float(v) for k, v in weights.items()})
+        self.w = _term_weights(weights, rb, X_data is not None, pde=weight_pde)
         self.norm_mode = norm_mode
         self.use = {'pde': True, 'bc': self.w['bc'] != 0.0, 'data': self.w['data'] != 0.0, 'norm': self.w['norm'] > 0.0}
         if self.use['data'] and (X_data is None or u_data is None):
@@ -276,11 +315,9 @@ class FusedTrainer:
         self.params = [p for p in self.net.params]
         self.nparam = sum(p.numel() for p in self.params)
         self.opt = FusedAdam([p.data for p in self.params], lr=lr, betas=betas, eps=eps)
-        self.weight_pde = self.w['pde']
         self._ar = None
         # one row per active term: [grad (nparam) | dE (1) | sum (1)] — the layout pde_residual_loss_grad writes
         self.G = torch.zeros(len(self.rows), self.nparam + 2, dtype=self.dtype, device=self.dev)
-        self.buf = self.G[0]
         if group is not None:
             if exchange == 'nvlink':     # one-kernel all-reduce over peer memory (pde_allreduce_oneshot)
                 from .comm import NvlinkAllReduce
@@ -291,17 +328,8 @@ class FusedTrainer:
             self.total = torch.zeros(self.nparam + 2, dtype=self.dtype, device=self.dev)
             self.wvec = torch.tensor([self.w[t] for t in self.rows], dtype=self.dtype, device=self.dev)
         if self.use['bc']:
-            per_face = max(1, int(n_boundary) // (2 * self.dim))       # Poisson_ND.py:225
-            self.nb = 2 * self.dim * per_face
-            self.Xb = torch.empty(self.nb, self.dim, dtype=self.dtype, device=self.dev)
-            # face k = (coordinate k // 2, side k % 2): that coordinate is replaced by 0 or L  (:133-139)
-            keep = torch.ones(2 * self.dim, 1, self.dim, dtype=self.dtype, device=self.dev)
-            put = torch.zeros(2 * self.dim, 1, self.dim, dtype=self.dtype, device=self.dev)
-            for k in range(2 * self.dim):
-                keep[k, 0, k // 2] = 0.0
-                put[k, 0, k // 2] = self.L if k % 2 else 0.0
-            self._face_keep = keep.expand(-1, per_face, -1).reshape(self.nb, self.dim).contiguous()
-            self._face_put = put.expand(-1, per_face, -1).reshape(self.nb, self.dim).contiguous()
+            self.faces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev)
+            self.nb, self.Xb = self.faces.n, self.faces.X
         if self.use['data']:
             self.Xd = X_data.detach().to(self.dtype).to(self.dev).contiguous()
             self.ud = u_data.detach().to(self.dtype).to(self.dev).reshape(-1).contiguous()
@@ -319,7 +347,6 @@ class FusedTrainer:
             self.best_step = torch.full((1,), -1, dtype=torch.int64, device=self.dev)
         self.hist_loss = torch.zeros(max(int(history), 0), dtype=self.dtype, device=self.dev)
         self.hist_l2sq = torch.zeros(max(int(history), 0) if self.n_test else 0, dtype=self.dtype, device=self.dev)
-        self._karr = (C.c_double * self.dim)(*self.ks)
         self._order = self.lib.pde_program_order(self.spec.kind)
         cnet = self.net.to_c([p.data for p in self.params])
         n_big = max(self.n, self.n_test, getattr(self, "nb", 1), self.Xd.shape[0] if self.use['data'] else 1)
@@ -329,102 +356,62 @@ class FusedTrainer:
         self.epochs_done = 0
 
     # ---- the launches of one epoch (enqueued on the current stream, no host sync)
-    def _mse(self, cnet, cenv, X, n, target, inv_n, row, seed=None, sums=None, want_grad=True):
-        """mean((u - target)^2) (target None: mean u^2) with gradient into row ``row`` of self.G."""
-        lib, st = self.lib, _stream(self.dev)
-        es = self.G.element_size()
-        base = self.G.data_ptr() + row * self.G.shape[1] * es
-        ev = L.Program()
-        ev.kind, ev.alpha = L.PROG_MSE, 1.0
-        ev.f = target.data_ptr() if target is not None else None
-        L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(ev), X.data_ptr(), n,
-                                           seed.data_ptr() if seed is not None else None, inv_n,
-                                           sums.data_ptr() if sums is not None else base + (self.nparam + 1) * es,
-                                           base if want_grad else None, None, self._ws.data_ptr(), self._ws.numel(), st),
-                "pde_residual_loss_grad(mse)")
+    def _mse(self, cnet, cenv, X, target, term, seed=None, sums=None, want_grad=True):
+        """mean((u - target)^2) over the global batch (target None: mean u^2) into the row of ``term``."""
+        n = X.shape[0]
+        _residual_row(cnet, cenv, _MSE.to_c(f=target), X, n, 1.0 / (n * self.world), self._ws,
+                      self.G[self.rows.index(term)], self.nparam, seed=seed, sums=sums, want_grad=want_grad)
 
     def _enqueue(self):
-        lib, dev = self.lib, self.dev
-        st = _stream(dev)
-        ps = [p.data for p in self.params]
-        cnet = self.net.to_c(ps)
+        cnet = self.net.to_c([p.data for p in self.params])
         cenv = self.env.to_c()
-        dt = L.F64 if self.dtype == torch.float64 else L.F32
-        es = self.G.element_size()
-        P = self.nparam
+        P, step = self.nparam, self.opt.step_count
         if self.resample:
-            L.check(lib.pde_sample_points_rhs(dt, self.dim, self.n, 0.0, self.L, self.seed, rank_offset(self.rank),
-                                              self.opt.step_count.data_ptr(), self._karr, self.L, None, self.X.data_ptr(), None,
-                                              self.f.data_ptr(), st), "pde_sample_points_rhs")
-        prog = L.Program()
-        prog.kind, prog.alpha = self.spec.kind, self.spec.alpha
-        prog.f = self.f.data_ptr()
+            sample_points_rhs(self.n, self.dim, self.L, self.ks, dtype=self.dtype, device=self.dev, seed=self.seed,
+                              offset=rank_offset(self.rank), offset_add=step, out=(self.X, None, self.f))
         inv_n = 1.0 / (self.n * self.world)
         row = self.rows.index('pde')
-        base = self.G.data_ptr() + row * self.G.shape[1] * es
-        fused_exchange = self._ar is not None and len(self.rows) == 1
-        if fused_exchange:     # exchange folded into the reduction of the per-CTA partials (one launch fewer)
-            L.check(lib.pde_residual_loss_grad_exchange(C.byref(cnet), C.byref(cenv), C.byref(prog), self.X.data_ptr(), self.n, None,
-                                                        inv_n, base, self._ws.data_ptr(), self._ws.numel(), C.byref(self._ar.peers),
-                                                        self._ar.slot, self._ar.seq.data_ptr(), st),
-                    "pde_residual_loss_grad_exchange")
-        else:
-            L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(prog), self.X.data_ptr(), self.n, None, inv_n,
-                                               base + (P + 1) * es, base, base + P * es, self._ws.data_ptr(), self._ws.numel(), st),
-                    "pde_residual_loss_grad")
+        # a single row: its exchange folded into the reduction of the per-CTA partials (one launch fewer)
+        fused_ar = self._ar if len(self.rows) == 1 else None
+        _residual_row(cnet, cenv, self.spec.to_c(f=self.f), self.X, self.n, inv_n, self._ws, self.G[row], P, ar=fused_ar)
         if self.use['bc']:
-            # fresh face points every epoch: one uniform draw, face coordinate replaced by 0 / L; the mean over
-            # the faces of the per-face means (equal counts) is the mean over all face points
-            L.check(lib.pde_sample_points_rhs(dt, self.dim, self.nb, 0.0, self.L, self.seed ^ 0x5851F42D4C957F2D, rank_offset(self.rank),
-                                              self.opt.step_count.data_ptr(), None, self.L, None, self.Xb.data_ptr(), None, None, st),
-                    "pde_sample_points_rhs(faces)")
-            torch.addcmul(self._face_put, self.Xb, self._face_keep, out=self.Xb)
-            self._mse(cnet, cenv, self.Xb, self.nb, None, 1.0 / (self.nb * self.world), self.rows.index('bc'))
+            self._mse(cnet, cenv, self.faces.draw(self.seed, rank_offset(self.rank), step), None, 'bc')
         if self.use['data']:
-            self._mse(cnet, cenv, self.Xd, self.Xd.shape[0], self.ud, 1.0 / (self.Xd.shape[0] * self.world), self.rows.index('data'))
+            self._mse(cnet, cenv, self.Xd, self.ud, 'data')
         if self.use['norm']:
-            r = self.rows.index('norm')
             if self.norm_mode == 'l2':
-                self._mse(cnet, cenv, self.X, self.n, None, inv_n, r)
+                self._mse(cnet, cenv, self.X, None, 'norm')
             else:
                 # F = 1 / (m + 1e-8), m = mean u^2: the mean first, then the reverse sweep seeded with dF/dm
-                self._mse(cnet, cenv, self.X, self.n, None, inv_n, r, sums=self.nsum, want_grad=False)
+                self._mse(cnet, cenv, self.X, None, 'norm', sums=self.nsum, want_grad=False)
                 m = self.nsum * inv_n
                 torch.neg(torch.reciprocal((m + 1e-8) ** 2), out=self.nseed)
-                self._mse(cnet, cenv, self.X, self.n, None, inv_n, r, seed=self.nseed)
+                self._mse(cnet, cenv, self.X, None, 'norm', seed=self.nseed)
                 self.norm_value.copy_(torch.reciprocal(m + 1e-8)[0])
-        if fused_exchange:
-            pass
-        elif self._ar is not None:
-            self._ar.all_reduce_(self.G.view(-1))
+        if self._ar is not None:
+            if fused_ar is None:
+                self._ar.all_reduce_(self.G.view(-1))
         elif self.group is not None:
             import torch.distributed as dist
             dist.all_reduce(self.G, group=self.group)
         if self.hist_loss.numel():
-            self.hist_loss.index_copy_(0, self.opt.step_count.clamp(max=self.hist_loss.numel() - 1), self.G[row, P + 1:] * inv_n)
+            self.hist_loss.index_copy_(0, step.clamp(max=self.hist_loss.numel() - 1), _row_sums(self.G[row], P) * inv_n)
         if len(self.rows) > 1:
             torch.mv(self.G.t(), self.wvec, out=self.total)      # sum of weight x term gradient
-            gflat, gscale = self.total, 1.0
+            self.opt.step(self.total)
         else:
-            gflat, gscale = self.G[0], self.w['pde']
-        cfg = self.opt.config(gscale)
-        L.check(lib.pde_adam_step(C.byref(cfg), gflat.data_ptr(), self.opt.exp_avg.data_ptr(), self.opt.exp_avg_sq.data_ptr(),
-                                  self.opt.step_count.data_ptr(), st), "pde_adam_step")
+            self.opt.step(self.G[0], self.w['pde'])
         if self.n_test:
             # fresh test points every epoch (Poisson_ND.py:282), a different Philox key than the interior draw
-            L.check(lib.pde_sample_points_rhs(dt, self.dim, self.n_test, 0.0, self.L, self.seed ^ 0x9E3779B97F4A7C15, 0,
-                                              self.opt.step_count.data_ptr(), self._karr, self.L, None, self.Xt.data_ptr(),
-                                              self.ut.data_ptr(), None, st), "pde_sample_points_rhs")
-            ev = L.Program()
-            ev.kind, ev.alpha = L.PROG_MSE, 1.0
-            ev.f = self.ut.data_ptr()
-            L.check(lib.pde_residual_loss_grad(C.byref(cnet), C.byref(cenv), C.byref(ev), self.Xt.data_ptr(), self.n_test, None,
-                                               1.0 / self.n_test, self.esum.data_ptr(), None, None, self._ws.data_ptr(),
-                                               self._ws.numel(), st), "pde_residual_loss_grad(eval)")
-            L.check(lib.pde_keep_best(C.byref(cfg), self.esum.data_ptr(), self.best_metric.data_ptr(), self.best_flat.data_ptr(),
-                                      self.opt.step_count.data_ptr(), self.best_step.data_ptr(), st), "pde_keep_best")
+            sample_points_rhs(self.n_test, self.dim, self.L, self.ks, dtype=self.dtype, device=self.dev,
+                              seed=self.seed ^ 0x9E3779B97F4A7C15, offset_add=step, out=(self.Xt, self.ut, None))
+            _residual_row(cnet, cenv, _MSE.to_c(f=self.ut), self.Xt, self.n_test, 1.0 / self.n_test, self._ws, None, P,
+                          sums=self.esum, want_grad=False)
+            L.check(self.lib.pde_keep_best(C.byref(self.opt.config()), self.esum.data_ptr(), self.best_metric.data_ptr(),
+                                           self.best_flat.data_ptr(), step.data_ptr(), self.best_step.data_ptr(),
+                                           _stream(self.dev)), "pde_keep_best")
             if self.hist_l2sq.numel():
-                self.hist_l2sq.index_copy_(0, (self.opt.step_count - 1).clamp(min=0, max=self.hist_l2sq.numel() - 1),
+                self.hist_l2sq.index_copy_(0, (step - 1).clamp(min=0, max=self.hist_l2sq.numel() - 1),
                                            self.esum / self.n_test)
 
     def step(self, n_epochs=1):
@@ -454,26 +441,29 @@ class FusedTrainer:
         if self._ar is not None:
             self._ar.check()
 
+    def _mean(self, term, n):
+        """The mean over the global batch of ``n`` points per rank that the row of ``term`` holds."""
+        return _row_sums(self.G[self.rows.index(term)], self.nparam)[0] / (n * self.world)
+
     @property
     def loss(self):
         """PDE loss of the last evaluated epoch (mean over the global batch), 0-d device tensor."""
         self.check()
-        return (self.G[self.rows.index('pde'), self.nparam + 1] / (self.n * self.world)).clone()
+        return self._mean('pde', self.n)
 
     @property
     def terms(self):
         """{'pde','bc','data','norm','total'} of the last evaluated epoch as 0-d device tensors
         (what train_poisson_nd appends to its history, Poisson_ND.py:288-293)."""
         self.check()
-        P = self.nparam
         out = {t: torch.zeros((), dtype=self.dtype, device=self.dev) for t in self.TERMS}
-        out['pde'] = self.G[self.rows.index('pde'), P + 1] / (self.n * self.world)
+        out['pde'] = self._mean('pde', self.n)
         if self.use['bc']:
-            out['bc'] = self.G[self.rows.index('bc'), P + 1] / (self.nb * self.world)
+            out['bc'] = self._mean('bc', self.nb)
         if self.use['data']:
-            out['data'] = self.G[self.rows.index('data'), P + 1] / (self.Xd.shape[0] * self.world)
+            out['data'] = self._mean('data', self.Xd.shape[0])
         if self.use['norm']:
-            out['norm'] = (self.G[self.rows.index('norm'), P + 1] / (self.n * self.world)) if self.norm_mode == 'l2' else self.norm_value
+            out['norm'] = self._mean('norm', self.n) if self.norm_mode == 'l2' else self.norm_value
         out['total'] = sum(self.w[t] * out[t] for t in self.TERMS)
         return out
 
@@ -491,11 +481,9 @@ class FusedTrainer:
     def load_best(self, model=None):
         """Copy the best parameters seen so far into ``model`` (default: the trained model)."""
         tgt = self.params if model is None else _Net(model, self.X).params
-        o = 0
         with torch.no_grad():
-            for p in tgt:
-                k = p.numel()
-                p.copy_(self.best_flat[o:o + k].view_as(p)); o += k
+            for p, b in zip(tgt, _split_flat(self.best_flat, tgt)):
+                p.copy_(b)
 
 
 class WanTrainer:
@@ -521,10 +509,7 @@ class WanTrainer:
         self.dim = model.dim
         self.ks = [1.0] * self.dim if ks is None else [float(k) for k in ks]
         self.n, self.critic_steps, self.wan_reg = int(n_interior), int(critic_steps), float(wan_reg)
-        rb = getattr(model, "bc_mode", "FBC") == 'RB'
-        self.w = {'pde': 1.0, 'bc': 1e4 if rb else 0.0, 'data': 1e3 if X_data is not None else 0.0, 'norm': 0.0}
-        if weights:
-            self.w.update({k: float(v) for k, v in weights.items()})
+        self.w = _term_weights(weights, getattr(model, "bc_mode", "FBC") == 'RB', X_data is not None)
         self.norm_mode = norm_mode
         self.seed = int(seed)
         self.opt_u = Adam(model.parameters(), lr=lr)      # torch.optim.Adam's update, one launch per step
@@ -536,16 +521,7 @@ class WanTrainer:
                         torch.empty(n, 1, dtype=self.dtype, device=self.dev))
         self.bufs = [mk(self.n) for _ in range(self.critic_steps + 1)]
         if self.w['bc'] != 0.0:
-            per_face = max(1, int(n_boundary) // (2 * self.dim))
-            self.nb = 2 * self.dim * per_face
-            self.Xb = torch.empty(self.nb, self.dim, dtype=self.dtype, device=self.dev)
-            keep = torch.ones(2 * self.dim, 1, self.dim, dtype=self.dtype, device=self.dev)
-            put = torch.zeros(2 * self.dim, 1, self.dim, dtype=self.dtype, device=self.dev)
-            for k in range(2 * self.dim):
-                keep[k, 0, k // 2] = 0.0
-                put[k, 0, k // 2] = self.L if k % 2 else 0.0
-            self._face_keep = keep.expand(-1, per_face, -1).reshape(self.nb, self.dim).contiguous()
-            self._face_put = put.expand(-1, per_face, -1).reshape(self.nb, self.dim).contiguous()
+            self.faces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev)
         self.Xd = X_data.detach().to(self.dev, self.dtype).contiguous() if X_data is not None else None
         self.ud = u_data.detach().to(self.dev, self.dtype).contiguous() if u_data is not None else None
         self.record = bool(record_points) and not graph
@@ -576,13 +552,10 @@ class WanTrainer:
         zero = torch.zeros((), dtype=self.dtype, device=self.dev)
         bc_l = data_l = norm_l = zero
         if self.w['bc'] != 0.0:                                              # :255-259 on device-drawn face points
-            sample_points_rhs(self.nb, self.dim, self.L, None, dtype=self.dtype, device=self.dev,
-                              seed=self.seed ^ 0x5851F42D4C957F2D, offset_add=self.draws, out=(self.Xb, None, None))
-            self.draws.add_(1)
-            torch.addcmul(self._face_put, self.Xb, self._face_keep, out=self.Xb)
+            Xb = self.faces.draw(self.seed, 0, self.draws, advance=True)
             if self.record:
-                self.drawn.append(('bc', self.Xb.clone(), None))
-            bc_l = P.data_loss(self.model, self.Xb, None, self.L)
+                self.drawn.append(('bc', Xb.clone(), None))
+            bc_l = P.data_loss(self.model, Xb, None, self.L)
         if self.w['data'] != 0.0:                                            # :261-265
             data_l = P.data_loss(self.model, self.Xd, self.ud, self.L)
         if self.w['norm'] > 0.0:                                             # :267-268

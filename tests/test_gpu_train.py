@@ -321,6 +321,8 @@ def test_trainer_rb_bc_data_norm_terms_match_reference_loop(method, norm_mode, g
     with pytest.raises(ValueError):
         pb.train.FusedTrainer(model, L, ks, weights={"bogus": 1.0})
     with pytest.raises(ValueError):
+        pb.train.WanTrainer(model, pb.poisson.CriticNet(dim, 8, 2).double().cuda(), L, ks, weights={"bogus": 1.0})
+    with pytest.raises(ValueError):
         pb.train.FusedTrainer(model, L, ks, weights={"data": 1.0})      # data weight without data points
 
 
