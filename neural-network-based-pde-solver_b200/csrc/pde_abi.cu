@@ -144,9 +144,15 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
     }
     return best;
   };
-  int P2 = largest_P(budget2, max_threads_regs / 2 >= p.UG ? max_threads_regs / 2 : p.UG);
   int P1 = largest_P(budget1, max_threads_regs);
+  // Wide, deep fp64 nets (d = 5, order 2, 7 hidden layers of 256) leave no room for one point next to the default
+  // K-chunk of W: stream W through smaller chunks (multiples of 4) before refusing the shape.
+  while (P1 < 1 && p.KC > 4) {
+    p.KC -= 4;
+    P1 = largest_P(budget1, max_threads_regs);
+  }
   if (P1 < 1) return PDE_ERR_UNSUPPORTED;
+  int P2 = largest_P(budget2, max_threads_regs / 2 >= p.UG ? max_threads_regs / 2 : p.UG);
   int P = (P2 >= 8) ? P2 : P1;
   // do not make tiles larger than what fills the machine
   long long fill = (n + dv.sms - 1) / dv.sms;
