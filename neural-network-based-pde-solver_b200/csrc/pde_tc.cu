@@ -42,54 +42,10 @@ namespace tc {
 
 constexpr int TP = 64;        // points per tile = UMMA M
 constexpr int HP = 64;        // padded hidden width = UMMA N / K
-// Epilogue warps: quarter q = w % 4 (16 points), column half h = (w / 4) % 2 and, with 16 warps, row half
-// rh = w / 8: the two warps of a (q, h) pair read the same 16x256b accumulator fragments and each keeps
-// one of its two rows, so a thread carries NE = 2 instead of 4 elements per chunk (half the registers)
-// and every scheduler has four instead of two epilogue warps to hide latencies with.
-#ifndef PDE_TC_NEPI
-#define PDE_TC_NEPI 8
-#endif
-constexpr int NEPI = PDE_TC_NEPI;
-constexpr int RS = NEPI / 8;    // row split
-constexpr int NE = 4 / RS;      // elements per thread and chunk: NR rows x 2 adjacent units
-constexpr int NR = 2 / RS;      // rows per thread
-static_assert(NEPI == 8 || NEPI == 16, "8 or 16 epilogue warps");
+// Epilogue warps: quarter q = w % 4 (16 points), column half h = w / 4 (8 of the 16 columns of a chunk).
+constexpr int NEPI = 8;
+constexpr int NE = 4;         // elements per thread and chunk: 2 rows x 2 adjacent units
 constexpr int NTHREADS = (NEPI + 4) * 32;   // + one warpgroup whose first warp issues the MMAs (rest idle, registers donated)
-#ifndef PDE_TC_STASH_EARLY
-#define PDE_TC_STASH_EARLY 1    // forward: stash stores at the top of the chunk instead of after its proxy fence
-#endif
-#ifndef PDE_TC_LD_EARLY
-#define PDE_TC_LD_EARLY 1       // forward: next chunk's accumulators fetched before this chunk's operand stores (needs STASH_EARLY)
-#endif
-#ifndef PDE_TC_PAIR
-#define PDE_TC_PAIR 1           // forward / dgrad GEMMs: two channels per M = 128 instruction (see ch_paired)
-#endif
-#ifndef PDE_TC_F32X2
-#define PDE_TC_F32X2 1          // sin/cos polynomials in packed fp32 pairs (FFMA2): half the issue slots
-#endif
-#ifndef PDE_TC_FENCE_MASK
-#define PDE_TC_FENCE_MASK 0xF   // bit j: chunk j gets its own fence + barrier arrival (bit 3 must be set)
-#endif
-#ifndef PDE_TC_SHADOW
-#define PDE_TC_SHADOW 2         // chunk-0 shadow of the adjoint operand set (see SmemMap); 1: rebuilt A chunk 0 in a fifth pass, 2: parked in TMEM
-#endif
-#ifndef PDE_TC_PARKQ
-#define PDE_TC_PARKQ 1          // six-channel variants: the residual stage's running sums live in TMEM (see PARK_Q)
-#endif
-#define PDE_TC_STR2(x) #x
-#define PDE_TC_STR(x) PDE_TC_STR2(x)
-#if PDE_TC_NEPI == 16
-#define PDE_TC_EPI_REGS 104     // 640 threads launch at 96 registers; setmaxnreg only redistributes those 61 440
-#define PDE_TC_ISS_REGS 64
-#else
-#ifndef PDE_TC_EPI_REGS
-#define PDE_TC_EPI_REGS 208
-#endif
-#ifndef PDE_TC_ISS_REGS
-#define PDE_TC_ISS_REGS 88      // 256 x 208 + 128 x 88 = the 384 x 168 registers the CTA launches with
-#endif
-#endif
-using StashV = std::conditional<RS == 1, float4, float2>::type;   // one stashed value of a thread's NE elements
 constexpr int MAXC = 6;       // jet channels the TMEM / smem budget covers
 constexpr int COL_R0 = 0;     // TMEM columns: activation / adjoint accumulators (3 interleaved pairs)
 constexpr int COL_G = 384;    // gW accumulators: slot s at column COL_G + 64 (s / 2), lane half s % 2
@@ -220,7 +176,7 @@ __device__ __forceinline__ void act_eval(int act, const float (&z)[N], bool big,
 #pragma unroll
       for (int e = 0; e < N; ++e) sincosf(z[e], &v0[e], &v1[e]);
     } else {
-      if constexpr (PDE_TC_F32X2 && N % 2 == 0) {
+      if constexpr (N % 2 == 0) {
 #pragma unroll
         for (int e = 0; e < N; e += 2) sincos_cw2(z[e], z[e + 1], v0[e], v1[e], v0[e + 1], v1[e + 1]);
       } else {
@@ -344,7 +300,7 @@ struct SmemMap {
   static constexpr int LIMIT = 232448;                    // dynamic shared memory a CTA can opt in to
   static constexpr int set_bytes = 2 * C * TILE_BYTES;
   static constexpr int par_floats = D * 64 + 4 * 64 + 64 + 4;
-  static constexpr int red_floats = (2 * 64 * C > 256 * RS) ? 2 * 64 * C : 256 * RS;   // also [4 RS][64] at the end
+  static constexpr int red_floats = (2 * 64 * C > 256) ? 2 * 64 * C : 256;   // also [4][64] at the end
   // everything but the operand sets, W and the chunk-0 shadow
   static constexpr int rest = 4096 + 1024 * (D > 0 ? D : 1) + par_floats * 4 + 64 * D * 4 + 64 * C * 4 + red_floats * 4 + 128;
   // Chunk-0 shadow of the adjoint set (reverse sweep): columns 0..15 of the 2 C adjoint tiles in an unswizzled K-major
@@ -353,12 +309,8 @@ struct SmemMap {
   static constexpr int shadow_if = 2 * C * 2048;
   static constexpr bool fits3 = 2 * set_bytes + 3 * 2 * TILE_BYTES + shadow_if + rest <= LIMIT;
   static constexpr bool fits2 = 2 * set_bytes + 2 * 2 * TILE_BYTES + shadow_if + rest <= LIMIT;
-  static constexpr bool shadow = (PDE_TC_SHADOW != 0) && (NEPI == 8) && (C <= 5) && (fits3 || fits2);
-#ifdef PDE_TC_FORCE_WS2
-  static constexpr int w_slots = (C <= 5) ? 2 : 1;   // development: two W slots whether the shadow needs them or not
-#else
+  static constexpr bool shadow = (C <= 5) && (fits3 || fits2);
   static constexpr int w_slots = (C <= 5) ? ((shadow && !fits3) ? 2 : 3) : 1;   // 3: every hidden W resident
-#endif
   static constexpr int off_T1 = 0;                        // activations A_l (operand of fwd / wgrad)
   static constexpr int off_T2 = off_T1 + set_bytes;       // adjoints Zb_l (operand of dgrad / wgrad)
   static constexpr int off_W = off_T2 + set_bytes;        // W_l hi, lo per slot
@@ -381,15 +333,8 @@ __device__ __forceinline__ void stsm_x4(uint32_t addr, uint32_t r0, uint32_t r1,
   asm volatile("stmatrix.sync.aligned.m8n8.x4.shared.b16 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(r0), "r"(r1), "r"(r2), "r"(r3) : "memory");
 }
 // The stash is rewritten every tile and dead after the tile's reverse sweep, but an L2 line that is merely dirty is
-// still written back to HBM when it is evicted.  PDE_TC_STASH_POLICY: 0 = plain st.global.cg / ld.global.cg;
-// 1 = stash traffic carries an L2 evict_last policy and the streamed inputs (X, f, beta) evict_first, so that the
-// one-pass inputs do not push stash lines out; 2 = 1 + every stash line is discarded (discard.global.L2: dropped
-// without write-back) once the reverse sweep has consumed it; 3 = discard only.
-#ifndef PDE_TC_STASH_POLICY
-#define PDE_TC_STASH_POLICY 1
-#endif
-constexpr bool STASH_HINT = (PDE_TC_STASH_POLICY == 1 || PDE_TC_STASH_POLICY == 2);
-constexpr bool STASH_DISCARD = (PDE_TC_STASH_POLICY >= 2);
+// still written back to HBM when it is evicted.  Stash traffic carries an L2 evict_last policy and the streamed
+// inputs (X, f, beta) evict_first, so that the one-pass inputs do not push stash lines out.
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t p;
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
@@ -401,74 +346,37 @@ __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   return p;
 }
 __device__ __forceinline__ void stash_store(float4* p, float4 v, uint64_t pol) {
-  if constexpr (STASH_HINT)
-    asm volatile("st.global.cg.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
-  else
-    __stcg(p, v);
-}
-__device__ __forceinline__ void stash_store(float2* p, float2 v, uint64_t pol) {
-  if constexpr (STASH_HINT)
-    asm volatile("st.global.cg.L2::cache_hint.v2.f32 [%0], {%1,%2}, %3;" ::"l"(p), "f"(v.x), "f"(v.y), "l"(pol) : "memory");
-  else
-    __stcg(p, v);
+  asm volatile("st.global.cg.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
 }
 __device__ __forceinline__ float4 stash_load(const float4* p, uint64_t pol) {
-  if constexpr (STASH_HINT) {
-    float4 v;
-    asm volatile("ld.global.cg.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
-    return v;
-  } else {
-    return __ldcg(p);
-  }
-}
-__device__ __forceinline__ float2 stash_load(const float2* p, uint64_t pol) {
-  if constexpr (STASH_HINT) {
-    float2 v;
-    asm volatile("ld.global.cg.L2::cache_hint.v2.f32 {%0,%1}, [%2], %3;" : "=f"(v.x), "=f"(v.y) : "l"(p), "l"(pol));
-    return v;
-  } else {
-    return __ldcg(p);
-  }
+  float4 v;
+  asm volatile("ld.global.cg.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
+  return v;
 }
 // one-pass inputs
 __device__ __forceinline__ float stream_load(const float* p, uint64_t pol) {
-  if constexpr (STASH_HINT) {
-    float v;
-    asm volatile("ld.global.cg.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol));
-    return v;
-  } else {
-    return *p;
-  }
+  float v;
+  asm volatile("ld.global.cg.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol));
+  return v;
 }
 // the same under a predicate (0 when it is false).  One asm block, so that the register is written by the predicated
 // load itself: a select after the load would make the warp wait for the DRAM round trip right where it was issued.
 __device__ __forceinline__ float stream_load_if(const float* p, uint64_t pol, bool pred) {
-  if constexpr (STASH_HINT) {
-    float v;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %3, 0;\n\t"
-        "mov.f32 %0, 0f00000000;\n\t"
-        "@p ld.global.cg.L2::cache_hint.f32 %0, [%1], %2;\n\t"
-        "}"
-        : "=f"(v)
-        : "l"(p), "l"(pol), "r"((int)pred));
-    return v;
-  } else {
-    return pred ? *p : 0.f;
-  }
-}
-// 128-byte line at p (128-byte aligned) will not be read again before it is rewritten: drop it from L2
-__device__ __forceinline__ void stash_discard(const void* p) { asm volatile("discard.global.L2 [%0], 128;" ::"l"(p) : "memory"); }
-__device__ __forceinline__ void stsm_x2(uint32_t addr, uint32_t r0, uint32_t r1) {
-  asm volatile("stmatrix.sync.aligned.m8n8.x2.shared.b16 [%0], {%1,%2};" ::"r"(addr), "r"(r0), "r"(r1) : "memory");
+  float v;
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %3, 0;\n\t"
+      "mov.f32 %0, 0f00000000;\n\t"
+      "@p ld.global.cg.L2::cache_hint.f32 %0, [%1], %2;\n\t"
+      "}"
+      : "=f"(v)
+      : "l"(p), "l"(pol), "r"((int)pred));
+  return v;
 }
 // stashed vector <-> the thread's element array
 __device__ __forceinline__ void to_arr(const float4& sv, float (&v)[4]) { v[0] = sv.x; v[1] = sv.y; v[2] = sv.z; v[3] = sv.w; }
-__device__ __forceinline__ void to_arr(const float2& sv, float (&v)[2]) { v[0] = sv.x; v[1] = sv.y; }
 __device__ __forceinline__ float4 from_arr(const float (&v)[4]) { return make_float4(v[0], v[1], v[2], v[3]); }
-__device__ __forceinline__ float2 from_arr(const float (&v)[2]) { return make_float2(v[0], v[1]); }
 __device__ __forceinline__ void named_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
 // UMMA descriptors as "constant high word + 14-bit start address (16-byte units) in the low word":
@@ -477,14 +385,14 @@ constexpr uint32_t DESC_HI = (1024u >> 4) | (1u << 14) | (2u << 29);   // SBO | 
 constexpr uint32_t DESC_HI_G2 = (2048u >> 4) | (1u << 14) | (2u << 29);   // MN-major view of a paired channel: 8-row groups 2 KB apart
 constexpr uint32_t DESC_K_LBO = (16u >> 4) << 16;      // low word, next to the start address
 constexpr uint32_t DESC_MN_LBO = (8192u >> 4) << 16;
-// Channel pairs stacked along M (PDE_TC_PAIR).  A tcgen05.mma whose operands both come from shared memory costs what its A
+// Channel pairs stacked along M.  A tcgen05.mma whose operands both come from shared memory costs what its A
 // tile costs to read, and an M = 128 instruction (52 cycles) is cheaper than two M = 64 ones (2 x 39): channels 2p and 2p+1
 // of an operand set share a pair of 16 KB blocks (hi, lo) with their 8-row groups interleaved (channel c & 1 of point
 // group g at row group 2g + (c & 1)), so that one M = 128 K-major descriptor covers both in the forward and dgrad GEMMs;
 // the accumulator rows land in TMEM exactly where the two M = 64 accumulators used to be interleaved by hand, only with
 // the roles of (lane half, row half) swapped (pick_ch).  An odd last channel keeps the plain (hi tile, lo tile) layout.
 // In the MN-major views (wgrad, first layer, biases) a paired channel simply has its row groups 2 KB apart.
-__host__ __device__ constexpr bool ch_paired(int c, int C) { return PDE_TC_PAIR && RS == 1 && ((c | 1) < C); }   // 8-warp epilogue only
+__host__ __device__ constexpr bool ch_paired(int c, int C) { return (c | 1) < C; }
 __host__ __device__ constexpr uint32_t ch_base(int c, int C) {   // bytes from the set's start to channel c's first row group (hi part)
   return ch_paired(c, C) ? (uint32_t)(c >> 1) * 4u * TILE_BYTES + (uint32_t)(c & 1) * 1024u : (uint32_t)c * 2u * TILE_BYTES;
 }
@@ -546,7 +454,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
   constexpr int WS = SM::w_slots;
   constexpr bool WRES = (WS == 3);
   constexpr bool SHADOW = SM::shadow;
-  constexpr bool SHADOW_TAIL = SHADOW && (PDE_TC_SHADOW == 1);   // fifth pass + bar_fix hand-shake
 
   extern __shared__ __align__(1024) unsigned char sm[];
   float* sPar = reinterpret_cast<float*>(sm + SM::off_par);
@@ -563,7 +470,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
   uint64_t* bar_wt = bar_chunk + 7;    // bulk copy of a W tile pair has landed (non-resident W only)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_chunk + 8);
   int* sTileEnd = reinterpret_cast<int*>(bar_chunk + 14);   // the epilogue's loop bound (see there)
-  uint64_t* bar_fix = bar_chunk + 9;   // 8 arrivals, epilogue -> issuer: chunk 0 of both operand sets is in place (shadow builds)
+  // (bar_chunk + 9 is unused)
   float* sMx = reinterpret_cast<float*>(bar_chunk + 10);   // per-tile maximum cotangent of warps 0 and 1
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -610,7 +517,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     mbar_init(bar_w, 1);
     mbar_init(bar_own, 1);
     mbar_init(bar_wt, 1);
-    mbar_init(bar_fix, NEPI);
     fence_mbar_init();
     if (sbase & 1023u) __trap();   // SWIZZLE_128B tiles need the 1024-byte alignment the declaration asks for
   }
@@ -656,7 +562,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     // MMA issuer (warp NEPI); its warpgroup hands its registers to the epilogue.  The warp runs
     // the loops convergently and one elected lane issues, so descriptor arithmetic stays uniform.
     // =====================================================================================
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 " PDE_TC_STR(PDE_TC_ISS_REGS) ";");
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 88;");   // 256 x 208 + 128 x 88 = the 384 x 168 registers the CTA launches with
     if (warp == NEPI) {
       constexpr uint32_t ID_FWD = make_idesc(64, 64, 0, 0);   // A K-major, B K-major
       constexpr uint32_t ID_FWD2 = make_idesc(128, 64, 0, 0), ID_DG2 = make_idesc(128, 64, 0, 1);   // channel pairs
@@ -669,7 +575,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
       const uint32_t kT1K = (sT1 >> 4) | DESC_K_LBO, kT1M = (sT1 >> 4) | DESC_MN_LBO;
       const uint32_t kT2K = (sT2 >> 4) | DESC_K_LBO, kT2M = (sT2 >> 4) | DESC_MN_LBO;
       const uint32_t kXT0 = (sXT >> 4) | DESC_K_LBO, kETK = (sET >> 4) | DESC_K_LBO;
-      uint32_t ph_chunk = 0, ph_own = 0, ph_wt = 0, ph_fix = 0;
+      uint32_t ph_chunk = 0, ph_own = 0, ph_wt = 0;
       int reg = 0;   // region the next D-producing GEMM writes
       int cur_w = 1;   // layer whose W sits in the shared slot (non-resident W)
       // chunk-0 shadow (unswizzled K-major: LBO 128 = next core matrix along K, SBO 256 = next 8 rows)
@@ -800,12 +706,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           __syncwarp();
           ph_chunk ^= 1;
           reg ^= 1;
-          if (SHADOW_TAIL && l < n_h - 1) {
-            // chunk 0 of the adjoints has been copied from the shadow and chunk 0 of A_{l-1} rebuilt
-            mbar_wait(bar_fix, ph_fix);
-            ph_fix ^= 1;
-            tc_fence_after();
-          }
           // wgrad: gW_l(tile) = sum_c Zb_{l,c}^T A_{l-1,c}   (K = 64 points);  bias: gb_l(tile) = Zb_{l,0}^T 1.
           // The accumulators start from zero every tile (the epilogue adds them to the running fp32
           // sums, see flush_grads) and the small cross terms go first: the tensor core truncates
@@ -854,10 +754,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           if constexpr (C <= 4) asm volatile("" : "+r"(kT1K_), "+r"(kT1M_), "+r"(kT2K_), "+r"(kT2M_), "+r"(kXT0_), "+r"(kETK_), "+r"(kZ0_));
 #pragma unroll
           for (int j = 0; j < 4; ++j) mbar_wait(&bar_chunk[j], ph_chunk);
-          if (SHADOW_TAIL) {
-            mbar_wait(bar_fix, ph_fix);
-            ph_fix ^= 1;
-          }
           tc_fence_after();
           ph_chunk ^= 1;
           if (elect_one()) {
@@ -894,30 +790,24 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     // =====================================================================================
     // epilogue warps
     // =====================================================================================
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 " PDE_TC_STR(PDE_TC_EPI_REGS) ";");
-    const int q = warp & 3, h = (warp >> 2) & 1, rh = warp >> 3;
-    int rows[NR];                                       // this thread's points (tile rows)
-    rows[0] = 16 * q + (lane >> 2) + (RS == 2 ? 8 * rh : 0);
-    if constexpr (NR == 2) rows[1] = rows[0] + 8;
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 208;");
+    const int q = warp & 3, h = (warp >> 2) & 1;
+    int rows[2];                                        // this thread's points (tile rows)
+    rows[0] = 16 * q + (lane >> 2);
+    rows[1] = rows[0] + 8;
     const int cq = 2 * (lane & 3);                      // column offset inside an 8-column block
-    // stmatrix row address of this thread.  8 warps: matrix i = lane/8 = (hi r0-rows, hi r1-rows, lo r0-rows,
-    // lo r1-rows); 16 warps (.x2): (hi rows, lo rows) of this warp's row half
-    const int sm_row = (RS == 1) ? 16 * q + 8 * ((lane >> 3) & 1) + (lane & 7) : 16 * q + 8 * rh + (lane & 7);
-    const int sm_tile = (RS == 1) ? (lane >> 4) : ((lane >> 3) & 1);
+    // stmatrix row address of this thread: matrix i = lane/8 = (hi r0-rows, hi r1-rows, lo r0-rows, lo r1-rows)
+    const int sm_row = 16 * q + 8 * ((lane >> 3) & 1) + (lane & 7);
+    const int sm_tile = lane >> 4;
     const uint32_t sm_base = (uint32_t)(sm_tile * TILE_BYTES) + ((sm_row >> 3) << 10) + ((sm_row & 7) << 7);
     const int sm_r7 = sm_row & 7;
     float* part = a.partial + (long long)blockIdx.x * a.PP;
-    StashV* stash = reinterpret_cast<StashV*>(a.stash + (long long)blockIdx.x * a.stash_f4) + warp * (NV * 32) + lane;
+    float4* stash = a.stash + (long long)blockIdx.x * a.stash_f4 + warp * (NV * 32) + lane;
     // this thread's part of a 16x256b accumulator fragment (rows lane/4 and lane/4 + 8, two columns each);
     // only valid after tcgen05.wait::ld
     auto pick = [&](const float (&t)[4], float (&v)[NE]) {
-      if constexpr (RS == 1) {
 #pragma unroll
-        for (int e = 0; e < 4; ++e) v[e] = t[e];
-      } else {
-        v[0] = rh ? t[2] : t[0];
-        v[1] = rh ? t[3] : t[1];
-      }
+      for (int e = 0; e < 4; ++e) v[e] = t[e];
     };
     // accumulator fragments of channel c from the raw 16x256b loads (one per channel slot, as issued): a paired channel's
     // two rows come from the two loads of its pair (lane halves = row halves), its columns from word pair c & 1
@@ -929,11 +819,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
         pick(t[c], v);
       }
     };
+    // (zeroed, then set: initialising them in the declaration swaps two issuer registers of the 5- and 6-channel variants)
     uint64_t pol_stash = 0, pol_stream = 0;
-    if constexpr (STASH_HINT) {
-      pol_stash = l2_policy_evict_last();
-      pol_stream = l2_policy_evict_first();
-    }
+    pol_stash = l2_policy_evict_last();
+    pol_stream = l2_policy_evict_first();
     uint32_t ph_d = 0, ph_w = 0;
     int reg = 0;   // region the next D-consuming step reads
     bool w_pending = false;   // a bar_w commit has been issued that nobody waited for yet
@@ -943,7 +832,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     // Six-channel variants are over the register budget and ptxas would keep these running sums (used once per tile, by
     // the residual stage of warps 0 and 1) in local memory, whose reloads miss L1 behind the stash traffic.  They are kept
     // in the last free TMEM columns instead (lane half 1 of the small accumulators' slot, columns 32..47).
-    constexpr bool PARK_Q = (PDE_TC_PARKQ != 0) && (C == 6) && (NEPI == 8);
+    constexpr bool PARK_Q = (C == 6);
     const uint32_t qpark = taddr_of(tmem, 32 * q + 16, COL_SMALL + 32);
     auto q_load = [&](double (&t)[4], double& g) {
       uint32_t w0[4], w1[4];
@@ -976,12 +865,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     auto pack_chunk = [&](const float (&v)[C][NE], uint32_t (&pk)[C][NE]) {
 #pragma unroll
       for (int c = 0; c < C; ++c) {
-        if constexpr (RS == 1) {
-          split2(v[c][0], v[c][1], pk[c][0], pk[c][2]);
-          split2(v[c][2], v[c][3], pk[c][1], pk[c][3]);
-        } else {
-          split2(v[c][0], v[c][1], pk[c][0], pk[c][1]);
-        }
+        split2(v[c][0], v[c][1], pk[c][0], pk[c][2]);
+        split2(v[c][2], v[c][3], pk[c][1], pk[c][3]);
       }
     };
     // paired channels: the lo part is a pair block (two tiles) further, the 8-row groups are 2 KB apart
@@ -991,18 +876,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
       for (int c = 0; c < C; ++c) {
         const uint32_t ac = addr + ch_base(c, C) + (ch_paired(c, C) ? pair_extra : 0u);
-        if constexpr (RS == 1) stsm_x4(ac, pk[c][0], pk[c][1], pk[c][2], pk[c][3]);
-        else stsm_x2(ac, pk[c][0], pk[c][1]);
+        stsm_x4(ac, pk[c][0], pk[c][1], pk[c][2], pk[c][3]);
       }
     };
     // chunk 0 of the adjoints into the shadow (unswizzled: 8-row group g at 256 g, K half h at +128, row at +16 (row & 7))
     const uint32_t z0_base = sZ0 + (uint32_t)(sm_tile * 2048) + ((sm_row >> 3) << 8) + (h << 7) + ((sm_row & 7) << 4);
     auto put_shadow = [&](const uint32_t (&pk)[C][NE]) {
-      if constexpr (RS == 1) {
 #pragma unroll
-        for (int c = 0; c < C; ++c)
-          stsm_x4(z0_base + z0_base_of(c, C) + (ch_paired(c, C) ? (pair_extra >> 2) : 0u), pk[c][0], pk[c][1], pk[c][2], pk[c][3]);
-      }
+      for (int c = 0; c < C; ++c)
+        stsm_x4(z0_base + z0_base_of(c, C) + (ch_paired(c, C) ? (pair_extra >> 2) : 0u), pk[c][0], pk[c][1], pk[c][2], pk[c][3]);
     };
     // ... and from there into the adjoint set proper: every warp moves the 16 rows x 16 bytes per tile it wrote itself
     auto copy_shadow = [&]() {
@@ -1025,11 +907,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
       pack_chunk(v, pk);
       put_chunk(set, j, pk);
     };
-    // Chunks whose bit is clear in PDE_TC_FENCE_MASK are published together with the next chunk that has
-    // its bit set: one proxy fence (MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC, ~200 cycles) covers several chunks.
+    // One proxy fence (MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC, ~200 cycles) publishes every chunk written since the last
+    // one.  The first layer's shadow path (SHP0 in bwd_layer) skips chunks 0 and 1 and publishes 0..2 with chunk_done(2).
     int chunk_pending = 0;   // first chunk written but not yet published
     auto chunk_done = [&](int j) {
-      if (!((PDE_TC_FENCE_MASK >> j) & 1)) return;
       fence_proxy_async();
       tc_fence_before();
       __syncwarp();
@@ -1046,7 +927,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
     // element of `part` is owned by one thread, so the fire-and-forget adds are applied in tile order
     // (deterministic).  Precondition: bar_w of the tile's last step has been waited for.
     float accW[3][4][NE];  // running sums of gW_l: [layer slot][8-column block][fragment]
-    float accB[3][NR];     // gb_l (lanes with lane % 4 == 0 of the h == 0 warps)
+    float accB[3][2];      // gb_l (lanes with lane % 4 == 0 of the h == 0 warps)
     float acc0[NE];        // [gW0 | gb0] fragment (h == 0 warps)
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
@@ -1055,7 +936,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
         for (int e = 0; e < NE; ++e) accW[i][b][e] = 0.f;
 #pragma unroll
-      for (int r = 0; r < NR; ++r) accB[i][r] = 0.f;
+      for (int r = 0; r < 2; ++r) accB[i][r] = 0.f;
     }
 #pragma unroll
     for (int e = 0; e < NE; ++e) acc0[e] = 0.f;
@@ -1079,7 +960,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           float t[NE];
           pick(w, t);
 #pragma unroll
-          for (int r = 0; r < NR; ++r) accB[sl][r] += t[2 * r];
+          for (int r = 0; r < 2; ++r) accB[sl][r] += t[2 * r];
         }
       }
       {
@@ -1146,9 +1027,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
       }
 
       TS(5);
-      float outacc[NR][C];
+      float outacc[2][C];
 #pragma unroll
-      for (int r = 0; r < NR; ++r)
+      for (int r = 0; r < 2; ++r)
 #pragma unroll
         for (int c = 0; c < C; ++c) outacc[r][c] = 0.f;
 
@@ -1178,10 +1059,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           tc_fence_after();
         }
         TS(20 + l);
-        float xr[NR][D > 0 ? D : 1];   // first layer: this thread's point coordinates (loop-invariant)
+        float xr[2][D > 0 ? D : 1];   // first layer: this thread's point coordinates (loop-invariant)
         if constexpr (L0) {
 #pragma unroll
-          for (int r = 0; r < NR; ++r)
+          for (int r = 0; r < 2; ++r)
 #pragma unroll
             for (int jd = 0; jd < D; ++jd) xr[r][jd] = sX[rows[r] * D + jd];
         }
@@ -1217,7 +1098,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
             for (int e = 0; e < NE; ++e) z[0][e] += (e & 1) ? b1v : b0v;
           }
-#if PDE_TC_STASH_EARLY
           // Stash stores first: by the time the chunk's proxy fence (whose MEMBAR waits for outstanding
           // stores) is reached they have been acknowledged, and their source registers are free again.
           if (do_bwd) {
@@ -1226,20 +1106,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
               for (int c = 1; c < C; ++c) stash_store(stash_at(l, j, 1 + c), from_arr(z[c]), pol_stash);
             }
           }
-#endif
           float av[C][NE], sv0[NE], sv1[NE];
           float zmax = 0.f;
 #pragma unroll
           for (int e = 0; e < NE; ++e) zmax = fmaxf(zmax, fabsf(z[0][e]));
           const bool big = (act == 0) && __any_sync(0xffffffffu, zmax > 32768.f);
           act_eval<NE>(act, z[0], big, sv0, sv1);
-#if PDE_TC_STASH_EARLY
           if (do_bwd) {
             stash_store(stash_at(l, j, 0), from_arr(sv0), pol_stash);
             stash_store(stash_at(l, j, 1), from_arr(sv1), pol_stash);
           }
-#endif
-          if constexpr (PDE_TC_F32X2 && NE % 2 == 0 && ND >= 1) {
+          if constexpr (ND >= 1) {
             // chain rule on element pairs in packed fp32 arithmetic
 #pragma unroll
             for (int e = 0; e < NE; e += 2) {
@@ -1273,16 +1150,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
               if constexpr (LAP) av[1 + ND][e] = fmaf(s1, z[1 + ND][e], s2 * S);
             }
           }
-#if PDE_TC_LD_EARLY
           if (!L0 && j < 3) {
             // z has been consumed by the chain rule: the accumulators of the next chunk are fetched under this
             // chunk's operand stores and proxy fence
 #pragma unroll
             for (int c = 0; c < C; ++c) tmem_ld_16x256b(zsrc + ((16 * (c & 1)) << 16) + 64 * (c >> 1) + 16 * (j + 1), zr[c]);
           }
-#endif
-          // Operand tile first: its fence (MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC) would otherwise also wait
-          // for the stash stores below to be acknowledged by L2.
           if constexpr (!LAST) {
             if (l == 1) TS(320 + j);
             store_chunk(sT1, j, av);
@@ -1294,26 +1167,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
             for (int c = 0; c < C; ++c) {
 #pragma unroll
-              for (int r = 0; r < NR; ++r) outacc[r][c] = fmaf(w0v, av[c][2 * r], fmaf(w1v, av[c][2 * r + 1], outacc[r][c]));
+              for (int r = 0; r < 2; ++r) outacc[r][c] = fmaf(w0v, av[c][2 * r], fmaf(w1v, av[c][2 * r + 1], outacc[r][c]));
             }
           }
-#if !PDE_TC_STASH_EARLY
-          if (do_bwd) {
-            stash_store(stash_at(l, j, 0), from_arr(sv0), pol_stash);
-            stash_store(stash_at(l, j, 1), from_arr(sv1), pol_stash);
-            if constexpr (!L0) {
-#pragma unroll
-              for (int c = 1; c < C; ++c) stash_store(stash_at(l, j, 1 + c), from_arr(z[c]), pol_stash);
-            }
-          }
-#endif
-#if !PDE_TC_LD_EARLY
-          if (!L0 && j < 3) {
-            // z has been consumed: fetch the accumulators of the next chunk now
-#pragma unroll
-            for (int c = 0; c < C; ++c) tmem_ld_16x256b(zsrc + ((16 * (c & 1)) << 16) + 64 * (c >> 1) + 16 * (j + 1), zr[c]);
-          }
-#endif
         }
         if constexpr (!L0) reg ^= 1;
       };
@@ -1323,7 +1179,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 
       // ================= output layer + envelope + residual program =================
 #pragma unroll
-      for (int r = 0; r < NR; ++r)
+      for (int r = 0; r < 2; ++r)
 #pragma unroll
         for (int c = 0; c < C; ++c) {
           float v = outacc[r][c];
@@ -1335,7 +1191,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
         for (int c = 0; c < C; ++c) {
 #pragma unroll
-          for (int r = 0; r < NR; ++r) sRed[(h * 64 + rows[r]) * C + c] = outacc[r][c];
+          for (int r = 0; r < 2; ++r) sRed[(h * 64 + rows[r]) * C + c] = outacc[r][c];
         }
       }
       TSW(2);
@@ -1424,7 +1280,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
                 for (int e = 0; e < NE; ++e) accW[i][b][e] *= ratio;
 #pragma unroll
-              for (int r = 0; r < NR; ++r) accB[i][r] *= ratio;
+              for (int r = 0; r < 2; ++r) accB[i][r] *= ratio;
             }
 #pragma unroll
             for (int e = 0; e < NE; ++e) acc0[e] *= ratio;
@@ -1445,7 +1301,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
         // Stash of this layer (activation values, pre-activation jets) and of the layer below (whose
         // activations are this layer's wgrad operand).  Software pipeline: the registers of chunk j+1
         // are fetched as soon as chunk j has consumed them (no rotation copies).
-        StashV cur[NV], prv[NV];
+        float4 cur[NV], prv[NV];
         auto load_cur = [&](int j) {
           cur[0] = stash_load(stash_at(l, j, 0), pol_stash); cur[1] = stash_load(stash_at(l, j, 1), pol_stash);
           if constexpr (LK >= 1) {
@@ -1465,13 +1321,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           }
         };
         // Shadow builds, below the top layer (SH): chunk 0 of the adjoints goes to the shadow, so nothing waits for
-        // the previous layer's wgrad before chunk 1; chunk 0 of the rebuilt A_{l-1} is made last (a fifth pass that
-        // also copies the shadow into the adjoint set), in the shadow of the last dgrad K step.
+        // the previous layer's wgrad before chunk 1; chunk 0 of the rebuilt A_{l-1} is parked in TMEM until the sets
+        // are free.
         constexpr bool SH = SHADOW && !TOP;
-        constexpr bool SHT = SHADOW_TAIL && !TOP;   // chunk 0 of A_{l-1} rebuilt in a fifth pass
-        constexpr bool SHP = SH && !SHT;            // ... rebuilt in the first pass and parked in TMEM until the sets are free
         load_cur(0);
-        load_prv(SHT ? 1 : 0);
+        load_prv(0);
         TS(30 + l);
         if constexpr (!TOP) {
           mbar_wait(bar_d, ph_d);   // Ab_l is complete
@@ -1479,10 +1333,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           tc_fence_after();
         }
         TS(40 + l);
-        float nbr[NR][C];   // top layer: cotangents of this thread's points (loop-invariant)
+        float nbr[2][C];   // top layer: cotangents of this thread's points (loop-invariant)
         if constexpr (TOP) {
 #pragma unroll
-          for (int r = 0; r < NR; ++r)
+          for (int r = 0; r < 2; ++r)
 #pragma unroll
             for (int c = 0; c < C; ++c) nbr[r][c] = sNb[rows[r] * C + c] * cur_scale;
         }
@@ -1511,7 +1365,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
               if constexpr (LAP) zp[1 + ND][e] = 0.f;
             }
           }
-          if constexpr (PDE_TC_F32X2 && NE % 2 == 0 && ND >= 1) {
+          if constexpr (ND >= 1) {
 #pragma unroll
             for (int e = 0; e < NE; e += 2) {
               float s0a, s1a, s2a, s3a, s0b, s1b, s2b, s3b;
@@ -1555,7 +1409,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
             for (int c = 0; c < C; ++c) {
 #pragma unroll
-              for (int r = 0; r < NR; ++r) {
+              for (int r = 0; r < 2; ++r) {
                 const float nv = nbr[r][c];
                 ab[c][2 * r] = w0v * nv; ab[c][2 * r + 1] = w1v * nv;
               }
@@ -1583,7 +1437,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
                 if constexpr (LAP) zj[1 + ND][e] = 0.f;
               }
             }
-            if constexpr (PDE_TC_F32X2 && NE % 2 == 0 && ND >= 1) {
+            if constexpr (ND >= 1) {
               // the same recurrences on element pairs in packed fp32 arithmetic
 #pragma unroll
               for (int e = 0; e < NE; e += 2) {
@@ -1672,23 +1526,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             }
             load_cur(j + 1);
           }
-          if constexpr (STASH_DISCARD) {
-            // layer l's stash lines of chunk j have been consumed (as `cur` here, as `prv` one layer up)
-            if ((lane & 7) == 0) {
-#pragma unroll
-              for (int v = 0; v < ((LK >= 1) ? NV : 2); ++v) stash_discard(stash_at(l, j, v));
-            }
-          }
           pack_chunk(zb, zk);
           }
           float ap[C][NE];
-          if (REFILL && (!SHT || j > 0)) {
+          if (REFILL) {
             refill(u0, ap);
-            if constexpr (SHT) load_prv(j < 3 ? j + 1 : 0);
-            else if (j < 3) load_prv(j + 1);
+            if (j < 3) load_prv(j + 1);
           }
           // first layer (no GEMM consumes its chunks one by one): chunk 1 is parked as well and the wait moves to chunk 2
-          constexpr bool SHP0 = SHP && LK == 0;
+          constexpr bool SHP0 = SH && LK == 0;
           if (j == (SH ? (SHP0 ? 2 : 1) : 0) && w_pending) {
             // the previous layer's wgrad still reads both operand sets: the results of this chunk are
             // computed before waiting for it, the stores come after
@@ -1698,7 +1544,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             w_pending = false;
             TS(60 + l);
           }
-          if constexpr (SHP0) {   // (shadow builds have the 8-warp epilogue: NE == 4)
+          if constexpr (SHP0) {
             if (j <= 2) {
               if (j == 0) {
                 put_shadow(zk);
@@ -1721,7 +1567,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           }
           if (SH && j == 0) {
             put_shadow(zk);
-            if constexpr (SHP && REFILL) {
+            if constexpr (REFILL) {
               // park the split A_{l-1} chunk in the unused accumulator slot of region h (lane half 1, columns 128..)
               uint32_t pk[C][NE];
               pack_chunk(ap, pk);
@@ -1732,7 +1578,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           } else {
             put_chunk(sT2, j, zk);
             if constexpr (REFILL) store_chunk(sT1, j, ap);
-            if constexpr (SHP) if (j == 1) {
+            if constexpr (SH) if (j == 1) {
               // the sets are free: chunk 0 moves from the shadow / TMEM to its place
               if constexpr (REFILL) {
                 uint32_t pk[C][NE];
@@ -1745,19 +1591,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             }
           }
           chunk_done(j);
-        }
-        if constexpr (SHT) {
-          // chunk 0 of both operand sets, in the shadow of the last dgrad K step
-          if constexpr (REFILL) {
-            float ap[C][NE];
-            refill(8 * h + cq, ap);
-            store_chunk(sT1, 0, ap);
-          }
-          copy_shadow();
-          fence_proxy_async();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_fix);
         }
         if constexpr (!TOP) reg ^= 1;
         w_pending = true;   // the issuer commits bar_w after this step's wgrad / first-layer MMAs
@@ -1790,12 +1623,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           for (int b = 0; b < 4; ++b) {
             const int i0 = 32 * h + 8 * b + cq;
 #pragma unroll
-            for (int r = 0; r < NR; ++r)
+            for (int r = 0; r < 2; ++r)
               *reinterpret_cast<float2*>(gW + rows[r] * HP + i0) = make_float2(accW[sl][b][2 * r] * inv, accW[sl][b][2 * r + 1] * inv);
           }
           if (h == 0 && (lane & 3) == 0) {
 #pragma unroll
-            for (int r = 0; r < NR; ++r) gW[HP * HP + rows[r]] = accB[sl][r] * inv;
+            for (int r = 0; r < 2; ++r) gW[HP * HP + rows[r]] = accB[sl][r] * inv;
           }
         }
       }
@@ -1820,19 +1653,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           gwl[j][k] = v;
         }
       named_sync(1, NEPI * 32);
-      float* sRedW = sRed;   // [4 RS row groups][64 columns]
+      float* sRedW = sRed;   // [4 row groups][64 columns]
       if (lane < 4) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          sRedW[(q + 4 * rh) * 64 + 16 * j + 8 * h + cq] = gwl[j][0];
-          sRedW[(q + 4 * rh) * 64 + 16 * j + 8 * h + cq + 1] = gwl[j][1];
+          sRedW[q * 64 + 16 * j + 8 * h + cq] = gwl[j][0];
+          sRedW[q * 64 + 16 * j + 8 * h + cq + 1] = gwl[j][1];
         }
       }
       named_sync(1, NEPI * 32);
       // ... then over the row groups in fixed order
       if (tid < 64) {
-        float v = (sRedW[tid] + sRedW[64 + tid]) + (sRedW[128 + tid] + sRedW[192 + tid]);
-        if constexpr (RS == 2) v += (sRedW[256 + tid] + sRedW[320 + tid]) + (sRedW[384 + tid] + sRedW[448 + tid]);
+        const float v = (sRedW[tid] + sRedW[64 + tid]) + (sRedW[128 + tid] + sRedW[192 + tid]);
         part[a.off_gwL + tid] = v * inv;
       }
       named_sync(1, NEPI * 32);
