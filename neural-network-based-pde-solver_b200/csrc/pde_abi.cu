@@ -17,49 +17,40 @@ static std::atomic<unsigned long long> g_launches{0};
 static thread_local int g_last_path = -1;
 void count_launch(int k) { g_launches.fetch_add((unsigned long long)k, std::memory_order_relaxed); }
 void set_last_path(int path) { g_last_path = path; }
+
+DevInfo device_info() {
+  // Per-device cache (devices of one box are identical, but be exact).  Threads that fill the same entry at once
+  // store the same values; `have` is published last, so a thread that sees it set also sees the attributes.
+  static std::atomic<int> sms[64], smem_optin[64], cc_major[64];
+  static std::atomic<bool> have[64];
+  int dev = 0;
+  DevInfo d{0, 0, 0, 0};
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return d; }
+  if (!have[dev].load(std::memory_order_acquire)) {
+    if (cudaDeviceGetAttribute(&d.sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return d;
+    if (cudaDeviceGetAttribute(&d.smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return d;
+    if (cudaDeviceGetAttribute(&d.cc_major, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess) return d;
+    sms[dev].store(d.sms, std::memory_order_relaxed);
+    smem_optin[dev].store(d.smem_optin, std::memory_order_relaxed);
+    cc_major[dev].store(d.cc_major, std::memory_order_relaxed);
+    have[dev].store(true, std::memory_order_release);
+  }
+  return DevInfo{1, sms[dev].load(std::memory_order_relaxed), smem_optin[dev].load(std::memory_order_relaxed),
+                 cc_major[dev].load(std::memory_order_relaxed)};
+}
 }  // namespace pde
 
 namespace {
 
 using namespace pde;
 
-struct DevInfo {
-  int ok, sms, smem_optin, cc_major;
-};
-
-DevInfo device_info() {
-  // per-device cache (devices of one box are identical, but be exact)
-  static DevInfo cache[64];
-  static int have[64];
-  int dev = 0;
-  DevInfo d{0, 0, 0, 0};
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return d; }
-  if (have[dev]) return cache[dev];
-  if (cudaDeviceGetAttribute(&d.sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return d;
-  if (cudaDeviceGetAttribute(&d.smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return d;
-  if (cudaDeviceGetAttribute(&d.cc_major, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess) return d;
-  d.ok = 1;
-  cache[dev] = d;
-  have[dev] = 1;
-  return d;
-}
-
 struct Plan {
   int D, order, C, n_lin, n_h, H, Hp, UG, P, KC, pitchP, nthreads, grid, num_tiles, max_grid;
   size_t elem, smem_bytes;
   long long packed_elems, off_W0t, off_b, off_Wt, off_Wn, off_wL, off_bL;
-  long long PP, off_gW0, off_gb0, off_gW, off_gwL, off_gbL;
-  long long n_params;
+  GradLayout g;
   size_t ws_packed, ws_partial, ws_psums, ws_total;
 };
-
-inline long long rup(long long x, long long m) { return (x + m - 1) / m * m; }
-
-// Scalar parameters of a validated network: W0 [H][D], b0 [H], (n_h - 1) x (W [H][H], b [H]), wL [H], bL.
-inline long long param_count(const pde_net* net) {
-  const long long H = net->widths[1], D = net->dim, n_h = net->n_linear - 1;
-  return H * D + H + (n_h - 1) * (H * H + H) + H + 1;
-}
 
 int validate_net(const pde_net* net) {
   if (!net) return PDE_ERR_INVALID;
@@ -72,12 +63,6 @@ int validate_net(const pde_net* net) {
   if (H < 1 || H > PDE_MAX_WIDTH) return PDE_ERR_UNSUPPORTED;
   for (int l = 1; l < net->n_linear; ++l)
     if (net->widths[l] != H) return PDE_ERR_UNSUPPORTED;
-  return PDE_OK;
-}
-
-int check_ptrs(const pde_net* net) {
-  for (int l = 0; l < net->n_linear; ++l)
-    if (!net->W[l] || !net->b[l]) return PDE_ERR_INVALID;
   return PDE_OK;
 }
 
@@ -113,14 +98,7 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
   p.off_wL = p.off_Wn + (long long)(p.n_h - 1) * HH;
   p.off_bL = p.off_wL + p.Hp;
   p.packed_elems = rup(p.off_bL + 1, 4);
-  // per-CTA partial gradient layout (padded natural layout)
-  p.off_gW0 = 0;
-  p.off_gb0 = (long long)p.Hp * p.D;
-  p.off_gW = p.off_gb0 + p.Hp;
-  p.off_gwL = p.off_gW + (long long)(p.n_h - 1) * (HH + p.Hp);
-  p.off_gbL = p.off_gwL + p.Hp;
-  p.PP = rup(p.off_gbL + 1, 4);
-  p.n_params = param_count(net);
+  p.g = grad_layout(p.D, p.n_h, p.H, p.Hp);
 
   KernelInfo ki = net_kernel_info<T>(p.D, order);
   if (!ki.fn) return PDE_ERR_UNSUPPORTED;
@@ -169,7 +147,7 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
     occ = 1;
   }
   if (occ < 1) occ = 1;
-  const size_t pbytes = (size_t)p.PP * sizeof(T);
+  const size_t pbytes = (size_t)p.g.PP * sizeof(T);
   int cap = pbytes <= (128u << 10) ? 4 : (pbytes <= (512u << 10) ? 2 : 1);
   if (occ > cap) occ = cap;
   p.max_grid = dv.sms * cap;
@@ -177,22 +155,10 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
   if (g > p.num_tiles) g = p.num_tiles;
   p.grid = (int)g;
   p.ws_packed = (size_t)rup(p.packed_elems * (long long)sizeof(T), 256);
-  p.ws_partial = (size_t)rup((long long)p.max_grid * p.PP * (long long)sizeof(T), 256);
+  p.ws_partial = (size_t)rup((long long)p.max_grid * p.g.PP * (long long)sizeof(T), 256);
   p.ws_psums = (size_t)rup((long long)p.max_grid * 8 * (long long)sizeof(double), 256);
   p.ws_total = p.ws_packed + p.ws_partial + p.ws_psums;
   return PDE_OK;
-}
-
-template <typename T>
-void fill_env(const pde_envelope* env, EnvDev<T>* e) {
-  memset(e, 0, sizeof(*e));
-  if (!env) return;
-  e->kind = env->kind;
-  e->lo = (T)env->lo; e->hi = (T)env->hi;
-  for (int i = 0; i < PDE_MAX_DIM; ++i) {
-    e->n_nodes[i] = env->n_nodes[i];
-    for (int k = 0; k < PDE_MAX_NODES; ++k) e->nodes[i][k] = (T)env->nodes[i][k];
-  }
 }
 
 int validate_env(const pde_envelope* env) {
@@ -218,6 +184,14 @@ int run_net(const pde_net* net, int order, int mode, const pde_envelope* env, co
   T* packed = reinterpret_cast<T*>(wsb);
   T* partial = reinterpret_cast<T*>(wsb + p.ws_packed);
   double* psums = reinterpret_cast<double*>(wsb + p.ws_packed + p.ws_partial);
+  const bool program = mode == MODE_PROGRAM;
+  const int n_q = program ? pde_program_quantities(prog->kind) : 0;
+  ReduceArgs<T> r;
+  if (mode != MODE_JETS_FWD &&
+      (rc = make_reduce_args<T>(p.g, partial, psums, p.grid, 0, n_q, false, static_cast<T*>(grad),
+                                program ? static_cast<T*>(sums) : nullptr, program ? static_cast<T*>(energy_grad) : nullptr,
+                                ex, &r)))
+    return rc;
 
   PackArgs<T> pa;
   memset(&pa, 0, sizeof(pa));
@@ -236,36 +210,21 @@ int run_net(const pde_net* net, int order, int mode, const pde_envelope* env, co
   a.X = static_cast<const T*>(X); a.n = n; a.num_tiles = p.num_tiles;
   a.mode = mode; a.want_grad = (grad != nullptr) || (energy_grad != nullptr);
   a.J = static_cast<T*>(J); a.Jbar = static_cast<const T*>(Jbar);
-  a.n_q = 0;
-  if (mode == MODE_PROGRAM) {
-    a.prog = prog->kind; a.n_q = pde_program_quantities(prog->kind);
+  a.n_q = n_q;
+  if (program) {
+    a.prog = prog->kind;
     fill_env<T>(env, &a.env);
     a.alpha = (T)prog->alpha; a.beta_const = (T)prog->beta_const; a.energy_const = (T)prog->energy_const;
     a.inv_n = (T)inv_n;
     a.f = static_cast<const T*>(prog->f); a.beta = static_cast<const T*>(prog->beta);
     a.energy = static_cast<const T*>(prog->energy); a.seed = static_cast<const T*>(seed);
   }
-  a.partial = partial; a.psums = psums; a.PP = p.PP;
-  a.off_gW0 = p.off_gW0; a.off_gb0 = p.off_gb0; a.off_gW = p.off_gW; a.off_gwL = p.off_gwL; a.off_gbL = p.off_gbL;
+  a.partial = partial; a.psums = psums; a.PP = p.g.PP;
+  a.off_gW0 = p.g.off_gW0; a.off_gb0 = p.g.off_gb0; a.off_gW = p.g.off_gW; a.off_gwL = p.g.off_gwL; a.off_gbL = p.g.off_gbL;
   if (launch_net<T>(p.D, order, p.grid, p.nthreads, p.smem_bytes, st, a) != cudaSuccess) return PDE_ERR_CUDA;
   set_last_path(0);
 
   if (mode == MODE_JETS_FWD) return PDE_OK;
-  ReduceArgs<T> r;
-  memset(&r, 0, sizeof(r));
-  r.partial = partial; r.psums = psums; r.PP = p.PP; r.grid = p.grid; r.n_lin = p.n_lin; r.D = p.D; r.H = p.H; r.Hp = p.Hp;
-  r.n_q = a.n_q;
-  r.off_gW0 = p.off_gW0; r.off_gb0 = p.off_gb0; r.off_gW = p.off_gW; r.off_gwL = p.off_gwL; r.off_gbL = p.off_gbL;
-  r.n_params = p.n_params;
-  r.grad = static_cast<T*>(grad);
-  r.sums = (mode == MODE_PROGRAM) ? static_cast<T*>(sums) : nullptr;
-  r.energy_grad = (mode == MODE_PROGRAM) ? static_cast<T*>(energy_grad) : nullptr;
-  if (ex) {
-    if (mode != MODE_PROGRAM || !r.grad || !r.sums || !r.energy_grad) return PDE_ERR_INVALID;
-    rc = comm_fill_args(ex->peers, sizeof(T) == 8 ? PDE_F64 : PDE_F32, p.n_params + 1 + a.n_q, ex->slot_elems, ex->seq, &r.comm);
-    if (rc) return rc;
-    r.have_comm = 1;
-  }
   if (launch_reduce<T>(st, r) != cudaSuccess) return PDE_ERR_CUDA;
   return PDE_OK;
 }
@@ -309,7 +268,7 @@ int pde_param_count(const pde_net* net, int64_t* n_params) {
   int st = validate_net(net);
   if (st) return st;
   if (!n_params) return PDE_ERR_INVALID;
-  *n_params = param_count(net);
+  *n_params = param_count(net->dim, net->n_linear - 1, net->widths[1]);
   return PDE_OK;
 }
 

@@ -37,8 +37,7 @@
 
 #include "../../include/pde_b200.h"
 #include "pde_comm.cuh"
-
-namespace pde { void count_launch(int k); }   // pde_abi.cu: launch counter behind pde_launch_count()
+#include "pde_launch.h"
 
 namespace {
 

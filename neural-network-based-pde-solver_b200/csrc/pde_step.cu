@@ -14,8 +14,7 @@
 #include <stdint.h>
 
 #include "../../include/pde_b200.h"
-
-namespace pde { void count_launch(int k); }   // pde_abi.cu: launch counter behind pde_launch_count()
+#include "pde_launch.h"
 
 namespace {
 

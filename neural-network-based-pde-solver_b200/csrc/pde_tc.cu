@@ -1794,11 +1794,10 @@ struct TcPlan {
   int D, order, C, NV, n_lin, n_h, H, grid, num_tiles, sms;
   int ndir;   // derivative directions of this launch (= D except in the dimension-split passes)
   size_t smem_bytes;
-  long long PP, off_gW0, off_gb0, off_gW, off_gwL, off_gbL, n_params, stash_f4;
+  GradLayout g;
+  long long stash_f4;
   size_t ws_params, ws_wimg, ws_partial, ws_psums, ws_stash, ws_total;
 };
-
-static inline long long rup(long long x, long long m) { return (x + m - 1) / m * m; }
 
 template <int D, int ORDER, int ACT, int NDIR = D>
 static cudaError_t launch_one(const TcPlan& p, const TcArgs& a, cudaStream_t st) {
@@ -1919,21 +1918,12 @@ static bool shape_ok(const pde_net* net, int order, long long n, int ndir = -1) 
 
 static int make_plan(const pde_net* net, int order, long long n, TcPlan* pl, int ndir = -1) {
   if (!shape_ok(net, order, n, ndir)) return PDE_ERR_UNSUPPORTED;
-  static std::atomic<int> sms_cached[64];   // per device ordinal
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return PDE_ERR_NO_DEVICE; }
-  int sms_dev = sms_cached[dev].load(std::memory_order_relaxed);
-  if (!sms_dev) {
-    int sms = 0, cc = 0;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return PDE_ERR_NO_DEVICE;
-    if (cudaDeviceGetAttribute(&cc, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess) return PDE_ERR_NO_DEVICE;
-    if (cc != 10) return PDE_ERR_UNSUPPORTED;
-    sms_cached[dev].store(sms, std::memory_order_relaxed);
-    sms_dev = sms;
-  }
+  const DevInfo dv = device_info();
+  if (!dv.ok) return PDE_ERR_NO_DEVICE;
+  if (dv.cc_major != 10) return PDE_ERR_UNSUPPORTED;
   TcPlan& p = *pl;
   memset(&p, 0, sizeof(p));
-  p.sms = sms_dev;
+  p.sms = dv.sms;
   p.D = net->dim; p.order = order;
   p.ndir = ndir < 0 ? p.D : ndir;
   p.C = 1 + (order >= 1 ? p.ndir : 0) + (order == 2);
@@ -1941,22 +1931,72 @@ static int make_plan(const pde_net* net, int order, long long n, TcPlan* pl, int
   p.n_lin = net->n_linear; p.n_h = p.n_lin - 1; p.H = net->widths[1];
   p.num_tiles = (int)((n + TP - 1) / TP);
   p.grid = p.num_tiles < p.sms ? p.num_tiles : p.sms;
-  const long long HH = (long long)HP * HP;
-  p.off_gW0 = 0;
-  p.off_gb0 = (long long)HP * p.D;
-  p.off_gW = p.off_gb0 + HP;
-  p.off_gwL = p.off_gW + (long long)(p.n_h - 1) * (HH + HP);
-  p.off_gbL = p.off_gwL + HP;
-  p.PP = rup(p.off_gbL + 1, 4);
-  p.n_params = (long long)p.H * p.D + p.H + (long long)(p.n_h - 1) * ((long long)p.H * p.H + p.H) + p.H + 1;
+  p.g = grad_layout(p.D, p.n_h, p.H, HP);
   p.stash_f4 = (long long)p.n_h * 4 * 8 * p.NV * 32;   // 16 bytes per thread of 8 warps (or 8 bytes x 16 warps)
   p.ws_params = (size_t)rup((p.D * 64 + p.n_h * 64 + 64 + 1) * 4, 256);
   p.ws_wimg = (size_t)(p.n_h - 1) * 2 * TILE_BYTES;
-  p.ws_partial = (size_t)rup((long long)p.sms * p.PP * 4, 256);
+  p.ws_partial = (size_t)rup((long long)p.sms * p.g.PP * 4, 256);
   p.ws_psums = (size_t)rup((long long)p.sms * 8 * 8, 256);
   p.ws_stash = (size_t)rup((long long)p.sms * p.stash_f4 * 16, 256);
   p.ws_total = p.ws_params + p.ws_wimg + p.ws_partial + p.ws_psums + p.ws_stash;
   return PDE_OK;
+}
+
+// The workspace pieces every tensor-core sequence uses, as make_plan sized them.
+struct TcBufs {
+  float* params;
+  unsigned char* wimg;
+  float* partial;
+  double* psums;
+  float4* stash;
+};
+
+static TcBufs carve(const TcPlan& p, void* workspace) {
+  unsigned char* wsb = static_cast<unsigned char*>(workspace);
+  TcBufs b;
+  b.params = reinterpret_cast<float*>(wsb);
+  b.wimg = wsb + p.ws_params;
+  b.partial = reinterpret_cast<float*>(wsb + p.ws_params + p.ws_wimg);
+  b.psums = reinterpret_cast<double*>(wsb + p.ws_params + p.ws_wimg + p.ws_partial);
+  b.stash = reinterpret_cast<float4*>(wsb + p.ws_params + p.ws_wimg + p.ws_partial + p.ws_psums);
+  return b;
+}
+
+static int launch_tc_pack(const pde_net* net, const TcPlan& p, float* params, unsigned char* wimg, cudaStream_t st) {
+  TcPackArgs pa;
+  memset(&pa, 0, sizeof(pa));
+  for (int l = 0; l < p.n_lin; ++l) { pa.W[l] = static_cast<const float*>(net->W[l]); pa.b[l] = static_cast<const float*>(net->b[l]); }
+  pa.n_lin = p.n_lin; pa.D = p.D; pa.H = p.H; pa.params = params; pa.wimg = wimg;
+  tc_pack_kernel<<<32, 256, 0, st>>>(pa);
+  if (cudaGetLastError() != cudaSuccess) return PDE_ERR_CUDA;
+  count_launch();
+  return PDE_OK;
+}
+
+// tc_kernel arguments of every mode: network, points, workspace and the partial-gradient layout.
+static TcArgs tc_args(const pde_net* net, const TcPlan& p, const TcBufs& b, const void* X, long long n, int mode,
+                      double inv_n) {
+  TcArgs a;
+  memset(&a, 0, sizeof(a));
+  a.n_h = p.n_h; a.act = net->activation; a.H = p.H;
+  a.params = b.params; a.wimg = b.wimg;
+  a.X = static_cast<const float*>(X); a.n = n; a.num_tiles = p.num_tiles;
+  a.mode = mode;
+  a.inv_n = (float)inv_n;
+  a.partial = b.partial; a.psums = b.psums; a.stash = b.stash;
+  a.PP = p.g.PP; a.stash_f4 = p.stash_f4;
+  a.off_gW0 = p.g.off_gW0; a.off_gb0 = p.g.off_gb0; a.off_gW = p.g.off_gW; a.off_gwL = p.g.off_gwL; a.off_gbL = p.g.off_gbL;
+  return a;
+}
+
+// What the envelope and residual-program stage reads (tc_kernel in mode 0, pinn_split_kernel).
+static void set_program(TcArgs& a, const pde_envelope* env, const pde_program* prog, const void* seed, double inv_n) {
+  a.prog = prog->kind; a.n_q = pde_program_quantities(prog->kind);
+  fill_env<float>(env, &a.env);
+  a.alpha = (float)prog->alpha; a.beta_const = (float)prog->beta_const; a.energy_const = (float)prog->energy_const;
+  a.inv_n = (float)inv_n;
+  a.f = static_cast<const float*>(prog->f); a.beta = static_cast<const float*>(prog->beta);
+  a.energy = static_cast<const float*>(prog->energy); a.seed = static_cast<const float*>(seed);
 }
 
 }  // namespace tc
@@ -1984,11 +2024,11 @@ static int make_split_plan(const pde_net* net, long long n, SplitPlan* sp) {
   sp->blocks = (int)(g < 4LL * sp->a.sms ? g : 4LL * sp->a.sms);
   sp->ws_common = sp->a.ws_total > sp->b.ws_total ? sp->a.ws_total : sp->b.ws_total;   // same layout, pass A's stash is the larger
   size_t o = sp->ws_common;
-  sp->off_JA = o; o += (size_t)tc::rup(n * 5 * 4, 256);
-  sp->off_JB = o; o += (size_t)tc::rup(n * 4 * 4, 256);
-  sp->off_JbA = o; o += (size_t)tc::rup(n * 5 * 4, 256);
-  sp->off_JbB = o; o += (size_t)tc::rup(n * 4 * 4, 256);
-  sp->off_ps = o; o += (size_t)tc::rup((long long)sp->blocks * 8 * 8, 256);
+  sp->off_JA = o; o += (size_t)rup(n * 5 * 4, 256);
+  sp->off_JB = o; o += (size_t)rup(n * 4 * 4, 256);
+  sp->off_JbA = o; o += (size_t)rup(n * 5 * 4, 256);
+  sp->off_JbB = o; o += (size_t)rup(n * 4 * 4, 256);
+  sp->off_ps = o; o += (size_t)rup((long long)sp->blocks * 8 * 8, 256);
   sp->ws_total = o;
   return PDE_OK;
 }
@@ -2027,51 +2067,23 @@ static int tc_run(const pde_net* net, int order, int mode, const pde_envelope* e
   TcPlan p;
   int rc = make_plan(net, order, n_points, &p);
   if (rc) return rc;
-  for (int l = 0; l < p.n_lin; ++l)
-    if (!net->W[l] || !net->b[l]) return PDE_ERR_INVALID;
+  if ((rc = check_ptrs(net))) return rc;
   if (!X || !workspace) return PDE_ERR_INVALID;
   if (workspace_bytes < p.ws_total) return PDE_ERR_WORKSPACE;
   if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) return PDE_ERR_INVALID;
-  unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  float* params = reinterpret_cast<float*>(wsb);
-  unsigned char* wimg = wsb + p.ws_params;
-  float* partial = reinterpret_cast<float*>(wsb + p.ws_params + p.ws_wimg);
-  double* psums = reinterpret_cast<double*>(wsb + p.ws_params + p.ws_wimg + p.ws_partial);
-  float4* stash = reinterpret_cast<float4*>(wsb + p.ws_params + p.ws_wimg + p.ws_partial + p.ws_psums);
-
-  TcPackArgs pa;
-  memset(&pa, 0, sizeof(pa));
-  for (int l = 0; l < p.n_lin; ++l) { pa.W[l] = static_cast<const float*>(net->W[l]); pa.b[l] = static_cast<const float*>(net->b[l]); }
-  pa.n_lin = p.n_lin; pa.D = p.D; pa.H = p.H; pa.params = params; pa.wimg = wimg;
-  tc_pack_kernel<<<32, 256, 0, st>>>(pa);
-  if (cudaGetLastError() != cudaSuccess) return PDE_ERR_CUDA;
-  count_launch();
-
-  TcArgs a;
-  memset(&a, 0, sizeof(a));
-  a.n_h = p.n_h; a.act = net->activation; a.H = p.H;
-  a.params = params; a.wimg = wimg;
-  a.X = static_cast<const float*>(X); a.n = n_points; a.num_tiles = p.num_tiles;
-  a.mode = mode;
+  const TcBufs b = carve(p, workspace);
+  TcArgs a = tc_args(net, p, b, X, n_points, mode, inv_n);
   a.J = static_cast<float*>(J); a.Jbar = static_cast<const float*>(Jbar);
   a.want_grad = (grad != nullptr) || (energy_grad != nullptr);
-  a.inv_n = (float)inv_n;
-  if (mode == 0) {
-    a.prog = prog->kind; a.n_q = pde_program_quantities(prog->kind);
-    if (env) {
-      a.env.kind = env->kind; a.env.lo = (float)env->lo; a.env.hi = (float)env->hi;
-      for (int i = 0; i < PDE_MAX_DIM; ++i) {
-        a.env.n_nodes[i] = env->n_nodes[i];
-        for (int k = 0; k < PDE_MAX_NODES; ++k) a.env.nodes[i][k] = (float)env->nodes[i][k];
-      }
-    }
-    a.alpha = (float)prog->alpha; a.beta_const = (float)prog->beta_const; a.energy_const = (float)prog->energy_const;
-    a.f = static_cast<const float*>(prog->f); a.beta = static_cast<const float*>(prog->beta);
-    a.energy = static_cast<const float*>(prog->energy); a.seed = static_cast<const float*>(seed);
-  }
-  a.partial = partial; a.psums = psums; a.stash = stash;
-  a.PP = p.PP; a.stash_f4 = p.stash_f4;
-  a.off_gW0 = p.off_gW0; a.off_gb0 = p.off_gb0; a.off_gW = p.off_gW; a.off_gwL = p.off_gwL; a.off_gbL = p.off_gbL;
+  if (mode == 0) set_program(a, env, prog, seed, inv_n);
+  ReduceArgs<float> r;
+  if (mode != 1 &&   // jets out: nothing to reduce
+      (rc = make_reduce_args<float>(p.g, b.partial, b.psums, p.grid, 0, a.n_q, false, static_cast<float*>(grad),
+                                    mode == 0 ? static_cast<float*>(sums) : nullptr,
+                                    mode == 0 ? static_cast<float*>(energy_grad) : nullptr, ex, &r)))
+    return rc;
+
+  if ((rc = launch_tc_pack(net, p, b.params, b.wimg, st))) return rc;
 #ifdef PDE_TC_TIMELINE
   a.dbg = timeline_buffer();
 #endif
@@ -2081,23 +2093,7 @@ static int tc_run(const pde_net* net, int order, int mode, const pde_envelope* e
 #ifdef PDE_TC_TIMELINE
   timeline_dump(a.dbg, st);
 #endif
-  if (mode == 1) return PDE_OK;   // jets out: nothing to reduce
-
-  ReduceArgs<float> r;
-  memset(&r, 0, sizeof(r));
-  r.partial = partial; r.psums = psums; r.PP = p.PP; r.grid = p.grid; r.n_lin = p.n_lin; r.D = p.D; r.H = p.H; r.Hp = HP;
-  r.n_q = a.n_q;
-  r.off_gW0 = p.off_gW0; r.off_gb0 = p.off_gb0; r.off_gW = p.off_gW; r.off_gwL = p.off_gwL; r.off_gbL = p.off_gbL;
-  r.n_params = p.n_params;
-  r.grad = static_cast<float*>(grad);
-  r.sums = (mode == 0) ? static_cast<float*>(sums) : nullptr;
-  r.energy_grad = (mode == 0) ? static_cast<float*>(energy_grad) : nullptr;
-  if (ex) {
-    if (mode != 0 || !r.grad || !r.sums || !r.energy_grad) return PDE_ERR_INVALID;
-    rc = comm_fill_args(ex->peers, PDE_F32, p.n_params + 1 + a.n_q, ex->slot_elems, ex->seq, &r.comm);
-    if (rc) return rc;
-    r.have_comm = 1;
-  }
+  if (mode == 1) return PDE_OK;
   if (launch_reduce<float>(st, r) != cudaSuccess) return PDE_ERR_CUDA;
   return PDE_OK;
 }
@@ -2112,106 +2108,57 @@ static int tc_pinn_split(const pde_net* net, const pde_envelope* env, const pde_
   SplitPlan sp;
   int rc = make_split_plan(net, n_points, &sp);
   if (rc) return rc;
-  for (int l = 0; l < sp.a.n_lin; ++l)
-    if (!net->W[l] || !net->b[l]) return PDE_ERR_INVALID;
+  if ((rc = check_ptrs(net))) return rc;
   if (!X || !workspace) return PDE_ERR_INVALID;
   if (workspace_bytes < sp.ws_total) return PDE_ERR_WORKSPACE;
   if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) return PDE_ERR_INVALID;
   const bool want_grad = (grad != nullptr) || (energy_grad != nullptr);
   unsigned char* wsb = static_cast<unsigned char*>(workspace);
-  const TcPlan& pa = sp.a;
-  float* params = reinterpret_cast<float*>(wsb);
-  unsigned char* wimg = wsb + pa.ws_params;
-  float* partial = reinterpret_cast<float*>(wsb + pa.ws_params + pa.ws_wimg);
-  double* psums_k = reinterpret_cast<double*>(wsb + pa.ws_params + pa.ws_wimg + pa.ws_partial);
-  float4* stash = reinterpret_cast<float4*>(wsb + pa.ws_params + pa.ws_wimg + pa.ws_partial + pa.ws_psums);
+  const TcBufs b = carve(sp.a, workspace);
   float* JA = reinterpret_cast<float*>(wsb + sp.off_JA);
   float* JB = reinterpret_cast<float*>(wsb + sp.off_JB);
   float* JbA = reinterpret_cast<float*>(wsb + sp.off_JbA);
   float* JbB = reinterpret_cast<float*>(wsb + sp.off_JbB);
   double* psums_pt = reinterpret_cast<double*>(wsb + sp.off_ps);
+  TcArgs pt;
+  memset(&pt, 0, sizeof(pt));
+  pt.X = static_cast<const float*>(X); pt.n = n_points;
+  set_program(pt, env, prog, seed, inv_n);
+  // With a gradient: pass A's reduction writes grad, pass B's adds to it and carries the sums, dE and the exchange.
+  // Without (value or dE only): one reduction of the sums over no gradient partials.
+  ReduceArgs<float> ra, rb;
+  if (!grad)
+    rc = make_reduce_args<float>(sp.a.g, b.partial, psums_pt, 0, sp.blocks, pt.n_q, false, nullptr,
+                                 static_cast<float*>(sums), static_cast<float*>(energy_grad), ex, &rb);
+  else if (!(rc = make_reduce_args<float>(sp.a.g, b.partial, psums_pt, sp.a.grid, sp.blocks, pt.n_q, false,
+                                          static_cast<float*>(grad), nullptr, nullptr, nullptr, &ra)))
+    rc = make_reduce_args<float>(sp.b.g, b.partial, psums_pt, sp.b.grid, sp.blocks, pt.n_q, true, static_cast<float*>(grad),
+                                 static_cast<float*>(sums), static_cast<float*>(energy_grad), ex, &rb);
+  if (rc) return rc;
 
-  TcPackArgs pk;
-  memset(&pk, 0, sizeof(pk));
-  for (int l = 0; l < pa.n_lin; ++l) { pk.W[l] = static_cast<const float*>(net->W[l]); pk.b[l] = static_cast<const float*>(net->b[l]); }
-  pk.n_lin = pa.n_lin; pk.D = pa.D; pk.H = pa.H; pk.params = params; pk.wimg = wimg;
-  tc_pack_kernel<<<32, 256, 0, st>>>(pk);
-  if (cudaGetLastError() != cudaSuccess) return PDE_ERR_CUDA;
-  count_launch();
-
+  if ((rc = launch_tc_pack(net, sp.a, b.params, b.wimg, st))) return rc;
   auto pass = [&](const TcPlan& p, int dir0, int mode, float* J, const float* Jbar) -> int {
-    TcArgs a;
-    memset(&a, 0, sizeof(a));
-    a.n_h = p.n_h; a.act = net->activation; a.H = p.H;
-    a.params = params; a.wimg = wimg;
-    a.X = static_cast<const float*>(X); a.n = n_points; a.num_tiles = p.num_tiles;
-    a.mode = mode; a.dir0 = dir0; a.J = J; a.Jbar = Jbar;
+    TcArgs a = tc_args(net, p, b, X, n_points, mode, inv_n);
+    a.dir0 = dir0; a.J = J; a.Jbar = Jbar;
     a.want_grad = mode == 2;
-    a.inv_n = (float)inv_n;
-    a.partial = partial; a.psums = psums_k; a.stash = stash;
-    a.PP = p.PP; a.stash_f4 = p.stash_f4;
-    a.off_gW0 = p.off_gW0; a.off_gb0 = p.off_gb0; a.off_gW = p.off_gW; a.off_gwL = p.off_gwL; a.off_gbL = p.off_gbL;
     if (launch_tc(p, a, st) != cudaSuccess) return PDE_ERR_CUDA;
     count_launch();
     return PDE_OK;
   };
   if ((rc = pass(sp.a, 0, 1, JA, nullptr))) return rc;
   if ((rc = pass(sp.b, 3, 1, JB, nullptr))) return rc;
-
-  TcArgs pt;
-  memset(&pt, 0, sizeof(pt));
-  pt.X = static_cast<const float*>(X); pt.n = n_points;
-  pt.prog = prog->kind; pt.n_q = pde_program_quantities(prog->kind);
-  if (env) {
-    pt.env.kind = env->kind; pt.env.lo = (float)env->lo; pt.env.hi = (float)env->hi;
-    for (int i = 0; i < PDE_MAX_DIM; ++i) {
-      pt.env.n_nodes[i] = env->n_nodes[i];
-      for (int k = 0; k < PDE_MAX_NODES; ++k) pt.env.nodes[i][k] = (float)env->nodes[i][k];
-    }
-  }
-  pt.alpha = (float)prog->alpha; pt.beta_const = (float)prog->beta_const; pt.energy_const = (float)prog->energy_const;
-  pt.inv_n = (float)inv_n;
-  pt.f = static_cast<const float*>(prog->f); pt.beta = static_cast<const float*>(prog->beta);
-  pt.energy = static_cast<const float*>(prog->energy); pt.seed = static_cast<const float*>(seed);
   pinn_split_kernel<<<sp.blocks, SPLIT_BLOCK, 0, st>>>(pt, JA, JB, want_grad ? JbA : nullptr, want_grad ? JbB : nullptr, psums_pt);
   if (cudaGetLastError() != cudaSuccess) return PDE_ERR_CUDA;
   count_launch();
   set_last_path(1);
 
-  auto reduce = [&](const TcPlan& p, bool first, bool last) -> int {
-    ReduceArgs<float> r;
-    memset(&r, 0, sizeof(r));
-    r.partial = partial; r.psums = psums_pt; r.psum_grid = sp.blocks; r.PP = p.PP; r.grid = p.grid; r.n_lin = p.n_lin; r.D = p.D; r.H = p.H;
-    r.Hp = HP; r.n_q = pt.n_q;
-    r.off_gW0 = p.off_gW0; r.off_gb0 = p.off_gb0; r.off_gW = p.off_gW; r.off_gwL = p.off_gwL; r.off_gbL = p.off_gbL;
-    r.n_params = p.n_params;
-    r.grad = static_cast<float*>(grad);
-    r.accumulate = first ? 0 : 1;
-    r.sums = last ? static_cast<float*>(sums) : nullptr;
-    r.energy_grad = last ? static_cast<float*>(energy_grad) : nullptr;
-    if (ex && last) {
-      if (!r.grad || !r.sums || !r.energy_grad) return PDE_ERR_INVALID;
-      int rc2 = comm_fill_args(ex->peers, PDE_F32, p.n_params + 1 + pt.n_q, ex->slot_elems, ex->seq, &r.comm);
-      if (rc2) return rc2;
-      r.have_comm = 1;
-    }
-    if (launch_reduce<float>(st, r) != cudaSuccess) return PDE_ERR_CUDA;
-    return PDE_OK;
-  };
-  if (!want_grad || !grad) {
-    // value only (or dE only): one reduction for the sums; a zero-sized gradient pass is not needed
-    ReduceArgs<float> r;
-    memset(&r, 0, sizeof(r));
-    r.partial = partial; r.psums = psums_pt; r.psum_grid = sp.blocks; r.PP = pa.PP; r.grid = 0; r.n_lin = pa.n_lin; r.D = pa.D; r.H = pa.H;
-    r.Hp = HP; r.n_q = pt.n_q; r.n_params = pa.n_params;
-    r.sums = static_cast<float*>(sums); r.energy_grad = static_cast<float*>(energy_grad);
-    if (launch_reduce<float>(st, r) != cudaSuccess) return PDE_ERR_CUDA;
-    return PDE_OK;
+  if (grad) {
+    if ((rc = pass(sp.a, 0, 2, nullptr, JbA))) return rc;
+    if (launch_reduce<float>(st, ra) != cudaSuccess) return PDE_ERR_CUDA;
+    if ((rc = pass(sp.b, 3, 2, nullptr, JbB))) return rc;
   }
-  if ((rc = pass(sp.a, 0, 2, nullptr, JbA))) return rc;
-  if ((rc = reduce(sp.a, true, false))) return rc;
-  if ((rc = pass(sp.b, 3, 2, nullptr, JbB))) return rc;
-  return reduce(sp.b, false, true);
+  if (launch_reduce<float>(st, rb) != cudaSuccess) return PDE_ERR_CUDA;
+  return PDE_OK;
 }
 
 int tc_residual_loss_grad(const pde_net* net, const pde_envelope* env, const pde_program* prog, const void* X,
