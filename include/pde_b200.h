@@ -52,8 +52,16 @@ enum {
   PDE_PROG_PINN = 1,     /* q0 = (alpha*Lap(u) + (beta-E)*u - f)^2                order 2 */
   PDE_PROG_DRM = 2,      /* q0 = alpha*|grad u|^2 - f*u                            order 1 */
   PDE_PROG_RAYLEIGH = 3, /* q0 = alpha*|grad u|^2 + beta*u^2 ; q1 = u^2            order 1 */
-  PDE_PROG_MSE = 4       /* q0 = (u - f)^2  (f NULL -> u^2)                        order 0 */
+  PDE_PROG_MSE = 4,      /* q0 = (u - f)^2  (f NULL -> u^2)                        order 0 */
+  PDE_PROG_FLUX = 5      /* q0 = (alpha*n.grad u + beta*u - f)^2 on box faces      order 1 */
 };
+
+/* Faces of the box [lo, hi]^dim for PDE_PROG_FLUX and pde_sample_faces_rhs: face k is x_{k/2} = lo (outward normal
+ * -e_{k/2}) when k is even and x_{k/2} = hi (normal +e_{k/2}) when k is odd.  A face set is a bit mask over bits
+ * 0 .. 2*dim-1.  A batch of n face points is popcount(mask) equal contiguous blocks, one per set bit in increasing bit
+ * order: point p lies on the face of set bit number p / (n / popcount(mask)).  The kernels need only the axis and the
+ * sign of the normal, never lo or hi.  With every face set (mask (1 << 2*dim) - 1) a pure-Neumann problem is
+ * accepted; its solution is determined only up to a constant. */
 
 /* A fully connected network [dim, H, ..., H, 1] with sin or tanh activations.
  * Replaces: SolutionNet / CriticNet (Poisson_Equations/Poisson_ND.py:11-46), FCN
@@ -82,10 +90,13 @@ typedef struct pde_envelope {
 
 /* Per-point residual program evaluated on the jets of u = B*net.
  * f, beta: optional device arrays of n values; energy: optional device scalar (trainable E,
- * KH_1D.py:218, QHO_2D_Energy.py:287-291), else energy_const. */
+ * KH_1D.py:218, QHO_2D_Energy.py:287-291), else energy_const.
+ * PDE_PROG_FLUX is the boundary-flux penalty of a Neumann (beta = 0) or Robin condition: f holds the prescribed data g
+ * (NULL: g = 0), beta (or beta_const) the Robin coefficient, `faces` the face mask of the points (layout above); the
+ * energy fields are ignored and dq/dE = 0.  The reference has no Neumann code (its README.md:23 advertises it). */
 typedef struct pde_program {
   int32_t kind;        /* PDE_PROG_* */
-  int32_t reserved;
+  int32_t faces;       /* PDE_PROG_FLUX: face mask, 1 .. (1 << 2*dim) - 1; ignored by every other program */
   double alpha;
   double beta_const;   /* used when beta == NULL */
   double energy_const; /* used when energy == NULL */
@@ -131,7 +142,9 @@ int pde_jets_backward(const pde_net* net, int32_t order, const void* X, int64_t 
  *   grad   : device (n_params) out or NULL — sum_k seed[k] * inv_n * sum_p dq_k(p)/dtheta
  *   energy_grad : device scalar out or NULL — same contraction for dq/dE
  *   seed   : device (K) or NULL (all ones) — dLoss/dmean_k, lets functions of means
- *            (Rayleigh quotient, WAN) and multi-GPU exact recombination share one kernel. */
+ *            (Rayleigh quotient, WAN) and multi-GPU exact recombination share one kernel.
+ * A PDE_PROG_FLUX call returns PDE_ERR_INVALID, before it enqueues anything, when faces == 0,
+ * faces >= 1 << 2*dim or n_points is not a multiple of popcount(faces); so does the _exchange variant below. */
 int pde_residual_loss_grad(const pde_net* net, const pde_envelope* env, const pde_program* prog,
                            const void* X, int64_t n_points, const void* seed, double inv_n,
                            void* sums, void* grad, void* energy_grad, void* workspace,
@@ -204,6 +217,19 @@ int pde_wan_scalars(int32_t dtype, int32_t kind, const void* means, const double
 int pde_sample_points_rhs(int32_t dtype, int32_t dim, int64_t n_points, double lo, double hi, uint64_t seed,
                           uint64_t offset, const void* offset_add, const double* k, double period,
                           const void* X_in, void* X, void* u_exact, void* f, void* stream);
+
+/* Face points with the manufactured Neumann data in the same pass.
+ * Replaces: the face draw of boundary_loss_dirichlet (Poisson_ND.py:130-141: X = rand(N, d) * L, X[:, i] = 0 or L),
+ * extended to a face mask (layout at pde_program above) and to the outward normal derivative of the manufactured
+ * solution of Poisson_ND.py:49-58.
+ *   X (popcount(faces) * n_per_face, dim) out: point p has exactly the coordinates pde_sample_points_rhs draws for
+ *     point index p with the same seed, offset and offset_add (same Philox counter, same half-open clamp), then the
+ *     face coordinate of its block set to lo or hi;
+ *   g: device (n) out or NULL (needs k and period): g = s (k_a pi / P) cos(k_a pi x_a / P) prod_{j != a} sin(k_j pi x_j / P),
+ *     s = -1 on the lo face and +1 on the hi face of axis a. */
+int pde_sample_faces_rhs(int32_t dtype, int32_t dim, int64_t n_per_face, int32_t faces, double lo, double hi,
+                         uint64_t seed, uint64_t offset, const void* offset_add, const double* k, double period, void* X,
+                         void* g, void* stream);
 
 /* Fused Adam over the flat gradient vector that pde_residual_loss_grad writes (parameters() order, a
  * trailing trainable energy scalar included when it is listed as the last tensor).

@@ -12,7 +12,7 @@ MAX_LINEAR, MAX_DIM, MAX_NODES, MAX_Q = 8, 5, 8, 4
 F32, F64 = 0, 1
 ACT_SIN, ACT_TANH = 0, 1
 ENV_NONE, ENV_POLY, ENV_EXPWIN = 0, 1, 2
-PROG_PINN, PROG_DRM, PROG_RAYLEIGH, PROG_MSE = 1, 2, 3, 4
+PROG_PINN, PROG_DRM, PROG_RAYLEIGH, PROG_MSE, PROG_FLUX = 1, 2, 3, 4, 5
 
 EXPORTS = [
     "pde_abi_version", "pde_strerror", "pde_param_count", "pde_jet_channels", "pde_program_quantities",
@@ -21,6 +21,7 @@ EXPORTS = [
     "pde_keep_best", "pde_peer_bytes", "pde_peer_alloc", "pde_peer_open", "pde_peer_close", "pde_peer_free",
     "pde_allreduce_oneshot", "pde_query_jets_path", "pde_set_kernel_path", "pde_kernel_path", "pde_last_kernel_path",
     "pde_launch_count", "pde_set_exchange_timeout", "pde_exchange_errors", "pde_residual_loss_grad_exchange", "pde_wan_scalars",
+    "pde_sample_faces_rhs",
 ]
 MAX_PEERS = 8
 
@@ -36,7 +37,7 @@ class Envelope(C.Structure):
 
 
 class Program(C.Structure):
-    _fields_ = [("kind", C.c_int32), ("reserved", C.c_int32), ("alpha", C.c_double), ("beta_const", C.c_double),
+    _fields_ = [("kind", C.c_int32), ("faces", C.c_int32), ("alpha", C.c_double), ("beta_const", C.c_double),
                 ("energy_const", C.c_double), ("f", C.c_void_p), ("beta", C.c_void_p), ("energy", C.c_void_p)]
 
 
@@ -100,6 +101,8 @@ def load():
     lib.pde_wan_pointwise.argtypes = [C.POINTER(Wan), vp, i64, vp, vp, vp, dbl, vp, vp, vp, vp, sz, vp]
     lib.pde_sample_points_rhs.argtypes = [i32, i32, i64, dbl, dbl, C.c_uint64, C.c_uint64, vp, C.POINTER(dbl), dbl, vp, vp,
                                           vp, vp, vp]
+    lib.pde_sample_faces_rhs.argtypes = [i32, i32, i64, i32, dbl, dbl, C.c_uint64, C.c_uint64, vp, C.POINTER(dbl), dbl, vp,
+                                         vp, vp]
     lib.pde_adam_step.argtypes = [C.POINTER(Adam), vp, vp, vp, vp, vp]
     lib.pde_keep_best.argtypes = [C.POINTER(Adam), vp, vp, vp, vp, vp, vp]
     lib.pde_peer_bytes.argtypes = [i32, i64, C.POINTER(sz)]

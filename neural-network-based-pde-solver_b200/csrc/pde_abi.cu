@@ -218,6 +218,7 @@ int run_net(const pde_net* net, int order, int mode, const pde_envelope* env, co
     a.inv_n = (T)inv_n;
     a.f = static_cast<const T*>(prog->f); a.beta = static_cast<const T*>(prog->beta);
     a.energy = static_cast<const T*>(prog->energy); a.seed = static_cast<const T*>(seed);
+    a.faces = prog->faces; a.face_n = flux_face_n(prog, n);
   }
   a.partial = partial; a.psums = psums; a.PP = p.g.PP;
   a.off_gW0 = p.g.off_gW0; a.off_gb0 = p.g.off_gb0; a.off_gW = p.g.off_gW; a.off_gwL = p.g.off_gwL; a.off_gbL = p.g.off_gbL;
@@ -279,7 +280,7 @@ int pde_jet_channels(int32_t dim, int32_t order) {
 
 int pde_program_quantities(int32_t kind) {
   switch (kind) {
-    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: return 1;
+    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: case PDE_PROG_FLUX: return 1;
     case PDE_PROG_RAYLEIGH: return 2;
     default: return PDE_ERR_INVALID;
   }
@@ -288,7 +289,7 @@ int pde_program_quantities(int32_t kind) {
 int pde_program_order(int32_t kind) {
   switch (kind) {
     case PDE_PROG_PINN: return 2;
-    case PDE_PROG_DRM: case PDE_PROG_RAYLEIGH: return 1;
+    case PDE_PROG_DRM: case PDE_PROG_RAYLEIGH: case PDE_PROG_FLUX: return 1;
     case PDE_PROG_MSE: return 0;
     default: return PDE_ERR_INVALID;
   }
@@ -343,6 +344,11 @@ static int residual_loss_grad_impl(const pde_net* net, const pde_envelope* env, 
   int rc = validate_env(env);
   if (rc) return rc;
   if (!sums && !grad && !energy_grad) return PDE_ERR_INVALID;
+  if (prog->kind == PDE_PROG_FLUX) {   // the face mask and the block layout of the points (include/pde_b200.h)
+    if (net->dim < 1 || net->dim > PDE_MAX_DIM) return PDE_ERR_UNSUPPORTED;
+    if (prog->faces <= 0 || prog->faces >= (1 << (2 * net->dim))) return PDE_ERR_INVALID;
+    if (n_points % __builtin_popcount((unsigned)prog->faces) != 0) return PDE_ERR_INVALID;
+  }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // Blackwell tensor-core path for the shapes it covers (fp32, H = 64 sin/tanh nets); it
   // declines with PDE_ERR_UNSUPPORTED and the generic SIMT kernel takes over.

@@ -35,6 +35,11 @@ inline int check_ptrs(const pde_net* net) {
   return PDE_OK;
 }
 
+// Points per face of a PDE_PROG_FLUX batch of n points (0 for every other program).  The mask is validated first.
+inline long long flux_face_n(const pde_program* prog, long long n) {
+  return prog->kind == PDE_PROG_FLUX ? n / __builtin_popcount((unsigned)prog->faces) : 0;
+}
+
 template <typename T>
 void fill_env(const pde_envelope* env, EnvDev<T>* e) {
   memset(e, 0, sizeof(*e));

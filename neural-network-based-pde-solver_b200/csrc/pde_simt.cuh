@@ -60,7 +60,21 @@ struct KArgs {
   T* partial;
   double* psums;
   long long PP, off_gW0, off_gb0, off_gW, off_gwL, off_gbL;
+  // PDE_PROG_FLUX: face mask and points per face (n / popcount(faces))
+  int faces;
+  long long face_n;
 };
+
+// Outward normal of the face that point gp of a PDE_PROG_FLUX batch lies on (include/pde_b200.h: one block of face_n
+// points per set bit of `faces`, in increasing bit order): axis in [0, dim), sign -1 (lo face) or +1 (hi face).
+// A subtraction walk over at most 2*dim - 1 blocks instead of a 64-bit division.
+__device__ __forceinline__ void flux_face(int faces, long long face_n, long long gp, int& axis, int& sign) {
+  unsigned m = (unsigned)faces;
+  for (long long r = gp; r >= face_n; r -= face_n) m &= m - 1u;
+  const int k = __ffs((int)m) - 1;
+  axis = k >> 1;
+  sign = (k & 1) ? 1 : -1;
+}
 
 // ---------------------------------------------------------------- small helpers
 template <typename T> __device__ __forceinline__ void ld4(const T* p, T (&v)[4]);
@@ -262,6 +276,20 @@ __device__ void program_point(const KArgs<T>& a, const T* x, long long gp, T (&n
     ub = T(2) * bt * u * w0 + T(2) * u * w1;
 #pragma unroll
     for (int i = 0; i < D; ++i) uib[i] = T(2) * a.alpha * ui[i] * w0;
+  } else if (ORDER == 1 && a.prog == 5) {  // boundary flux: r = alpha n.grad u + beta u - g
+    int ax, sg;
+    flux_face(a.faces, a.face_n, gp, ax, sg);
+    const T as = sg > 0 ? a.alpha : -a.alpha;
+    T un = T(0);
+#pragma unroll
+    for (int i = 0; i < D; ++i)
+      if (i == ax) un = ui[i];
+    const T r = as * un + bt * u - fv;
+    qs[0] += (double)(r * r);
+    const T rb = T(2) * r * w0;
+    ub = bt * rb;
+#pragma unroll
+    for (int i = 0; i < D; ++i) uib[i] = (i == ax) ? as * rb : T(0);
   } else {  // MSE on the value
     T r = u - fv;
     qs[0] += (double)(r * r);

@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <string.h>
 
 #include "../../include/pde_b200.h"
 #include "pde_launch.h"
@@ -34,6 +35,9 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 template <typename T> __device__ __forceinline__ T sin_(T x);
 template <> __device__ __forceinline__ float sin_<float>(float x) { return sinf(x); }
 template <> __device__ __forceinline__ double sin_<double>(double x) { return sin(x); }
+template <typename T> __device__ __forceinline__ T cos_(T x);
+template <> __device__ __forceinline__ float cos_<float>(float x) { return cosf(x); }
+template <> __device__ __forceinline__ double cos_<double>(double x) { return cos(x); }
 
 template <typename T> __device__ __forceinline__ T below_(T hi, T lo);
 template <> __device__ __forceinline__ float below_<float>(float hi, float lo) { return nextafterf(hi, lo); }
@@ -56,7 +60,31 @@ struct SampleArgs {
   void* X; void* u; void* f;
   const void* X_in;   // evaluate the manufactured solution at given points instead of sampling
   const long long* offset_add;   // device, optional: added to `offset` (e.g. the optimiser's step counter)
+  int faces;          // sample_faces_kernel: face mask, points per face, and the Neumann data out (the u slot is unused)
+  long long face_n;
+  void* g;
 };
+
+// The coordinates of point p: Philox counters (point index | coordinate group << 62, call offset), uniform in
+// [lo, hi) with the half-open interval kept through rounding (float: (hi - lo) * (1 - 2^-24) may round to hi - lo).
+template <typename T>
+__device__ __forceinline__ void draw_point(const SampleArgs& a, long long p, uint2 key, unsigned long long off, T (&x)[PDE_MAX_DIM]) {
+  if (sizeof(T) == 4) {
+    for (int c = 0; 4 * c < a.dim; ++c) {
+      const uint4 r = philox4x32_10(make_uint4((uint32_t)p, (uint32_t)(p >> 32) | ((uint32_t)c << 30), (uint32_t)off, (uint32_t)(off >> 32)), key);
+      const uint32_t rr[4] = {r.x, r.y, r.z, r.w};
+      for (int e = 0; e < 4 && 4 * c + e < a.dim; ++e) x[4 * c + e] = (T)(a.lo + (a.hi - a.lo) * (double)unit_f32(rr[e]));
+    }
+  } else {
+    for (int c = 0; 2 * c < a.dim; ++c) {
+      const uint4 r = philox4x32_10(make_uint4((uint32_t)p, (uint32_t)(p >> 32) | ((uint32_t)c << 30), (uint32_t)off, (uint32_t)(off >> 32)), key);
+      x[2 * c] = (T)(a.lo + (a.hi - a.lo) * unit_f64(r.x, r.y));
+      if (2 * c + 1 < a.dim) x[2 * c + 1] = (T)(a.lo + (a.hi - a.lo) * unit_f64(r.z, r.w));
+    }
+  }
+  for (int i = 0; i < a.dim; ++i)
+    if (x[i] >= (T)a.hi) x[i] = below_<T>((T)a.hi, (T)a.lo);
+}
 
 // One thread per point: coordinates from Philox counters (point index | coordinate group << 62, call offset),
 // written row-major; u* and f in the same pass.  HBM-bound: 4 (d + 2) bytes per point.
@@ -80,30 +108,44 @@ __global__ void sample_rhs_kernel(const SampleArgs a) {
     if (Xin) {
       for (int i = 0; i < a.dim; ++i) x[i] = Xin[p * a.dim + i];
     } else {
-      if (sizeof(T) == 4) {
-        for (int c = 0; 4 * c < a.dim; ++c) {
-          const uint4 r = philox4x32_10(make_uint4((uint32_t)p, (uint32_t)(p >> 32) | ((uint32_t)c << 30), (uint32_t)off, (uint32_t)(off >> 32)), key);
-          const uint32_t rr[4] = {r.x, r.y, r.z, r.w};
-          for (int e = 0; e < 4 && 4 * c + e < a.dim; ++e) x[4 * c + e] = (T)(a.lo + (a.hi - a.lo) * (double)unit_f32(rr[e]));
-        }
-      } else {
-        for (int c = 0; 2 * c < a.dim; ++c) {
-          const uint4 r = philox4x32_10(make_uint4((uint32_t)p, (uint32_t)(p >> 32) | ((uint32_t)c << 30), (uint32_t)off, (uint32_t)(off >> 32)), key);
-          x[2 * c] = (T)(a.lo + (a.hi - a.lo) * unit_f64(r.x, r.y));
-          if (2 * c + 1 < a.dim) x[2 * c + 1] = (T)(a.lo + (a.hi - a.lo) * unit_f64(r.z, r.w));
-        }
-      }
-      // the half-open interval survives rounding (float: (hi - lo) * (1 - 2^-24) may round to hi - lo)
-      for (int i = 0; i < a.dim; ++i) {
-        if (x[i] >= (T)a.hi) x[i] = below_<T>((T)a.hi, (T)a.lo);
-        X[p * a.dim + i] = x[i];
-      }
+      draw_point<T>(a, p, key, off, x);
+      for (int i = 0; i < a.dim; ++i) X[p * a.dim + i] = x[i];
     }
     if (a.have_k && (U || F)) {
       T u = T(1);
       for (int i = 0; i < a.dim; ++i) u *= sin_<T>((T)(a.k[i] * 3.14159265358979323846) * x[i] / (T)a.period);
       if (U) U[p] = u;
       if (F) F[p] = s * u;
+    }
+  }
+}
+
+// Face points (include/pde_b200.h, pde_sample_faces_rhs): the coordinates sample_rhs_kernel draws for the same point
+// index, the block's face coordinate set to lo or hi, and the outward normal derivative of u* in the same pass.
+// HBM-bound: 4 (d + 1) bytes per point.
+template <typename T>
+__global__ void sample_faces_kernel(const SampleArgs a) {
+  T* X = static_cast<T*>(a.X);
+  T* G = static_cast<T*>(a.g);
+  const uint2 key = make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32));
+  const unsigned long long off = a.offset + (a.offset_add ? (unsigned long long)*a.offset_add : 0ull);
+  for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < a.n; p += (long long)gridDim.x * blockDim.x) {
+    T x[PDE_MAX_DIM];
+    draw_point<T>(a, p, key, off, x);
+    int ax, sg;
+    pde::flux_face(a.faces, a.face_n, p, ax, sg);
+    for (int i = 0; i < a.dim; ++i) {
+      if (i == ax) x[i] = (T)(sg > 0 ? a.hi : a.lo);
+      X[p * a.dim + i] = x[i];
+    }
+    if (G) {
+      T v = T(1);
+      for (int i = 0; i < a.dim; ++i) {
+        const T w = (T)(a.k[i] * 3.14159265358979323846) / (T)a.period;
+        const T z = (T)(a.k[i] * 3.14159265358979323846) * x[i] / (T)a.period;
+        v *= (i == ax) ? w * cos_<T>(z) : sin_<T>(z);
+      }
+      G[p] = sg > 0 ? v : -v;
     }
   }
 }
@@ -258,6 +300,29 @@ int pde_sample_points_rhs(int32_t dtype, int32_t dim, int64_t n_points, double l
   const int block = 256, grid = grid_for(n_points, block);
   if (dtype == PDE_F32) sample_rhs_kernel<float><<<grid, block, 0, st>>>(a);
   else sample_rhs_kernel<double><<<grid, block, 0, st>>>(a);
+  pde::count_launch(1);
+  return cudaGetLastError() == cudaSuccess ? PDE_OK : PDE_ERR_CUDA;
+}
+
+int pde_sample_faces_rhs(int32_t dtype, int32_t dim, int64_t n_per_face, int32_t faces, double lo, double hi,
+                         uint64_t seed, uint64_t offset, const void* offset_add, const double* k, double period, void* X,
+                         void* g, void* stream) {
+  if (dtype != PDE_F32 && dtype != PDE_F64) return PDE_ERR_INVALID;
+  if (dim < 1 || dim > PDE_MAX_DIM) return PDE_ERR_UNSUPPORTED;
+  if (faces <= 0 || faces >= (1 << (2 * dim)) || n_per_face < 1 || !(hi > lo) || !X) return PDE_ERR_INVALID;
+  if (g && (!k || !(period > 0.0))) return PDE_ERR_INVALID;
+  SampleArgs a;
+  memset(&a, 0, sizeof(a));
+  a.dim = dim; a.n = n_per_face * __builtin_popcount((unsigned)faces); a.lo = lo; a.hi = hi;
+  a.period = period > 0.0 ? period : 1.0;
+  a.seed = seed; a.offset = offset; a.have_k = k ? 1 : 0;
+  for (int i = 0; i < PDE_MAX_DIM; ++i) a.k[i] = (k && i < dim) ? k[i] : 0.0;
+  a.X = X; a.g = g; a.offset_add = static_cast<const long long*>(offset_add);
+  a.faces = faces; a.face_n = n_per_face;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int block = 256, grid = grid_for(a.n, block);
+  if (dtype == PDE_F32) sample_faces_kernel<float><<<grid, block, 0, st>>>(a);
+  else sample_faces_kernel<double><<<grid, block, 0, st>>>(a);
   pde::count_launch(1);
   return cudaGetLastError() == cudaSuccess ? PDE_OK : PDE_ERR_CUDA;
 }

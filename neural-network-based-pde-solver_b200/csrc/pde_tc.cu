@@ -74,6 +74,10 @@ struct TcArgs {
   int mode;                     // 0: envelope + residual program; 1: network jets out (forward only); 2: jet cotangents in
   float* J;                     // mode 1: (n, C) network jets (value, first derivatives) out
   const float* Jbar;            // mode 2: (n, C) cotangents of the network jets in
+  // PDE_PROG_FLUX (order-1 instantiations only): face mask and points per face, read by the residual stage together
+  // with the point's global index (tile * 64 + tid)
+  int faces;
+  long long face_n;
 };
 
 // ---------------------------------------------------------------- per-element math
@@ -220,7 +224,7 @@ __device__ void envelope_point(const TcArgs& a, const float* x, float* out) {
   if constexpr (ORDER == 2) out[1 + D] = LB;
 }
 template <int D, int ORDER>
-__device__ void program_point_lap(const TcArgs& a, const float* env, const float* cst, float fv, float bt,
+__device__ void program_point_lap(const TcArgs& a, const float* env, const float* cst, float fv, float bt, long long gp,
                                   float (&nj)[1 + (ORDER >= 1 ? D : 0) + (ORDER == 2)], double (&qs)[4], double& gE) {
   constexpr int ND = (ORDER >= 1) ? D : 0;
   const float B = env[0];
@@ -272,6 +276,20 @@ __device__ void program_point_lap(const TcArgs& a, const float* env, const float
     ub = 2.f * bt * u * w0 + 2.f * u * w1;
 #pragma unroll
     for (int i = 0; i < D; ++i) uib[i] = 2.f * a.alpha * ui[i] * w0;
+  } else if (ORDER == 1 && a.prog == PDE_PROG_FLUX) {   // the order-0 / order-2 kernels keep their instruction stream
+    int ax, sg;
+    flux_face(a.faces, a.face_n, gp, ax, sg);
+    const float as = sg > 0 ? a.alpha : -a.alpha;
+    float un = 0.f;
+#pragma unroll
+    for (int i = 0; i < D; ++i)
+      if (i == ax) un = ui[i];
+    const float r = as * un + bt * u - fv;
+    qs[0] += (double)(r * r);
+    const float rb = 2.f * r * w0;
+    ub = bt * rb;
+#pragma unroll
+    for (int i = 0; i < D; ++i) uib[i] = (i == ax) ? as * rb : 0.f;
   } else {
     const float r = u - fv;
     qs[0] += (double)(r * r);
@@ -1223,7 +1241,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             double tq[4], tg;
             q_load(tq, tg);
             if (gp < a.n) {
-              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, nj, tq, tg);
+              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, tq, tg);
             } else {
 #pragma unroll
               for (int c = 0; c < C; ++c) nj[c] = 0.f;
@@ -1231,7 +1249,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             q_store(tq, tg);
           } else if constexpr (!SPLIT) {
             if (gp < a.n) {
-              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, nj, qs, gE);
+              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, qs, gE);
             } else {
 #pragma unroll
               for (int c = 0; c < C; ++c) nj[c] = 0.f;
@@ -1720,7 +1738,7 @@ __global__ void pinn_split_kernel(const TcArgs a, const float* JA, const float* 
     const float bt = a.beta ? a.beta[gp] : a.beta_const;
     float env[7];
     envelope_point<5, 2>(a, x, env);
-    program_point_lap<5, 2>(a, env, cst, fv, bt, nj, qs, gE);
+    program_point_lap<5, 2>(a, env, cst, fv, bt, gp, nj, qs, gE);
     if (JbarA) {
       // the value channel's cotangent goes to pass A only (the reverse sweep is linear in the cotangents)
       JbarA[gp * 5] = nj[0]; JbarA[gp * 5 + 1] = nj[1]; JbarA[gp * 5 + 2] = nj[2]; JbarA[gp * 5 + 3] = nj[3]; JbarA[gp * 5 + 4] = nj[6];
@@ -1997,6 +2015,7 @@ static void set_program(TcArgs& a, const pde_envelope* env, const pde_program* p
   a.inv_n = (float)inv_n;
   a.f = static_cast<const float*>(prog->f); a.beta = static_cast<const float*>(prog->beta);
   a.energy = static_cast<const float*>(prog->energy); a.seed = static_cast<const float*>(seed);
+  a.faces = prog->faces; a.face_n = flux_face_n(prog, a.n);
 }
 
 }  // namespace tc

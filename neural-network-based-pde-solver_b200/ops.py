@@ -366,15 +366,19 @@ def mlp_jets(model: nn.Module, X: torch.Tensor, order: int = 2) -> torch.Tensor:
 # ---------------------------------------------------------------------------------------------
 @dataclass
 class ProgramSpec:
+    """A residual program (pde_program).  ``faces``: face mask of a ``PROG_FLUX`` batch (include/pde_b200.h: one equal
+    block of points per set bit, face k = side k % 2 of axis k // 2); ignored by the other programs."""
     kind: int
     alpha: float = 1.0
     beta_const: float = 0.0
     energy_const: float = 0.0
+    faces: int = 0
 
     def to_c(self, f=None, beta=None, energy=None) -> L.Program:
         """The pde_program descriptor; ``f`` / ``beta`` / ``energy``: per-point (scalar) device tensors or None."""
         p = L.Program()
         p.kind, p.alpha, p.beta_const, p.energy_const = self.kind, self.alpha, self.beta_const, self.energy_const
+        p.faces = int(self.faces)
         p.f, p.beta, p.energy = _ptr(f), _ptr(beta), _ptr(energy)
         return p
 

@@ -123,6 +123,31 @@ def boundary_loss_dirichlet(model, L, N_b_per_face, dim, device, *, group=None):
     return sum(losses) / len(losses)
 
 
+def boundary_loss_neumann(model, L, N_b_per_face, dim, device, g=None, faces=None, *, group=None):
+    """mean over the selected faces of mean((du/dn - g)^2), fresh uniform face samples: the Neumann counterpart of
+    boundary_loss_dirichlet (Poisson_ND.py:130-141, same torch.rand face draws), one fused launch for all faces.
+
+    ``faces``: face mask, face k = (coordinate k // 2, side k % 2: 0 or L), default every face; ``g``: None (zero flux)
+    or a callable g(X) -> (N,) giving the prescribed outward normal derivative.  A Robin condition
+    alpha du/dn + kappa u = g is ``ops.residual_mean`` with ``ProgramSpec(PROG_FLUX, alpha, beta_const=kappa,
+    faces=mask)`` on the same blocked points."""
+    dtype = next(model.parameters()).dtype
+    mask = (1 << 2 * dim) - 1 if faces is None else int(faces)
+    if not 0 < mask < 1 << 2 * dim:
+        raise ValueError(f"faces must be a face mask in 1 .. {(1 << 2 * dim) - 1}")
+    blocks = []
+    for i in range(dim):
+        for at_L in (False, True):
+            if mask >> (2 * i + int(at_L)) & 1:
+                X = torch.rand(N_b_per_face, dim, device=device, dtype=dtype) * L
+                X[:, i] = L if at_L else 0.0
+                blocks.append(X)
+    X = torch.cat(blocks)
+    gv = None if g is None else g(X).reshape(-1)
+    # (with group, residual_mean counts the points of this rank on every rank)
+    return residual_mean(model, X, ProgramSpec(_lib.PROG_FLUX, faces=mask), _envelope(model, L), f=gv, group=group)
+
+
 def data_loss(model, X_data, u_data, L, *, group=None, n_global=None):
     """mean((u(X_data) - u_data)^2)   (Poisson_ND.py:230-232)."""
     return residual_mean(model, X_data, ProgramSpec(_lib.PROG_MSE), _envelope(model, L), f=u_data, group=group,

@@ -6,6 +6,7 @@ state on the CPU.  Here the same epoch is a fixed sequence of launches on one st
 
     pde_sample_points_rhs  (optional, when points are redrawn every epoch)
     pde_residual_loss_grad (the fused tcgen05 / SIMT loss step: sums, flat gradient)
+    pde_sample_faces_rhs + pde_residual_loss_grad per boundary term (Dirichlet penalty, Neumann flux), data / norm terms
     all-reduce of [grad | dE | sums]  (only with ``group``)
     pde_adam_step          (fused Adam on the flat gradient, parameters updated in place)
     pde_sample_points_rhs + pde_residual_loss_grad(value only) + pde_keep_best  (optional evaluation)
@@ -60,6 +61,38 @@ def sample_points_rhs(n, dim, L_box, ks=None, *, dtype=torch.float32, device="cu
     return Xout, u, f
 
 
+def all_faces(dim):
+    """The face mask with every face of [lo, hi]^dim set (include/pde_b200.h: face k = side k % 2 of axis k // 2)."""
+    return (1 << (2 * int(dim))) - 1
+
+
+def sample_faces_rhs(n_per_face, dim, L_box, faces=None, ks=None, *, dtype=torch.float32, device="cuda", seed=0, offset=0,
+                     lo=0.0, offset_add=None, out=None):
+    """(X, g): ``n_per_face`` uniform points on each face of the mask ``faces`` (default: all 2d faces) of
+    [lo, L_box]^dim, one contiguous block per set bit in increasing bit order, and with ``ks`` the outward normal
+    derivative g of the manufactured solution of Poisson_ND.py:49-58 at those points, in one launch
+    (pde_sample_faces_rhs).  Point p has the coordinates ``sample_points_rhs`` draws for point p with the same
+    seed / offset / offset_add, the block's face coordinate set to lo or L_box.  ``out=(X, g)``: write into existing
+    tensors (g may be None)."""
+    lib = L.load()
+    dev = torch.device(device)
+    mask = all_faces(dim) if faces is None else int(faces)
+    n = bin(mask).count("1") * int(n_per_face) if 0 < mask < (1 << 2 * dim) else 0
+    if out is not None:
+        X, g = out
+    else:
+        X = torch.empty(max(n, 1), dim, dtype=dtype, device=dev)
+        g = torch.empty(max(n, 1), dtype=dtype, device=dev) if ks is not None else None
+    karr = (C.c_double * dim)(*[float(k) for k in ks]) if ks is not None else None
+    with torch.cuda.device(dev):
+        L.check(lib.pde_sample_faces_rhs(L.F64 if X.dtype == torch.float64 else L.F32, dim, int(n_per_face), mask, float(lo),
+                                         float(L_box), int(seed), int(offset),
+                                         offset_add.data_ptr() if offset_add is not None else None, karr, float(L_box),
+                                         X.data_ptr(), g.data_ptr() if g is not None else None, _stream(dev)),
+                "pde_sample_faces_rhs")
+    return X, g
+
+
 def rank_offset(rank):
     """Philox counter offset of data-parallel rank ``rank``: bits 40.. of the counter's second half, far above any
     epoch count, so that every rank draws its own points (the reference is single-process; with the default seed
@@ -84,31 +117,27 @@ def _term_weights(weights, rb, has_data, pde=1.0):
 
 
 class _FacePoints:
-    """``n_boundary`` points split evenly over the 2d faces of [0, L]^dim (Poisson_ND.py:225), redrawn into ``X`` by
-    ``draw``: one uniform draw, then face k = (coordinate k // 2, side k % 2) gets that coordinate replaced by 0 or L
-    (:133-139).  Equal counts per face, so the mean over all face points is the mean of the per-face means."""
+    """``n_boundary // (2 dim)`` points on each face of the mask ``faces`` (default: all 2d faces) of [0, L]^dim
+    (Poisson_ND.py:225), redrawn into ``X`` by ``draw`` in one launch: a uniform draw in which face k = (coordinate
+    k // 2, side k % 2) gets that coordinate set to 0 or L (:133-139), and with ``ks`` the outward normal derivative
+    ``g`` of the manufactured solution.  Equal counts per face, so the mean over all face points is the mean of the
+    per-face means."""
     KEY = 0x5851F42D4C957F2D   # xor-ed into the seed: the face draws are independent of the interior draws
 
-    def __init__(self, n_boundary, dim, L_box, dtype, device):
-        per_face = max(1, int(n_boundary) // (2 * dim))
-        self.n, self.dim, self.L = 2 * dim * per_face, dim, float(L_box)
+    def __init__(self, n_boundary, dim, L_box, dtype, device, faces=None, ks=None, key=KEY):
+        self.per_face = max(1, int(n_boundary) // (2 * dim))
+        self.faces = all_faces(dim) if faces is None else int(faces)
+        self.n, self.dim, self.L, self.ks, self.key = bin(self.faces).count("1") * self.per_face, dim, float(L_box), ks, key
         self.X = torch.empty(self.n, dim, dtype=dtype, device=device)
-        keep = torch.ones(2 * dim, 1, dim, dtype=dtype, device=device)
-        put = torch.zeros(2 * dim, 1, dim, dtype=dtype, device=device)
-        for k in range(2 * dim):
-            keep[k, 0, k // 2] = 0.0
-            put[k, 0, k // 2] = self.L if k % 2 else 0.0
-        self._keep = keep.expand(-1, per_face, -1).reshape(self.n, dim).contiguous()
-        self._put = put.expand(-1, per_face, -1).reshape(self.n, dim).contiguous()
+        self.g = torch.empty(self.n, dtype=dtype, device=device) if ks is not None else None
 
     def draw(self, seed, offset, counter, advance=False):
         """Fresh face points from Philox block ``offset`` + ``counter`` (a device int64 draw counter, incremented
-        after the uniform draw when ``advance``)."""
-        sample_points_rhs(self.n, self.dim, self.L, None, dtype=self.X.dtype, device=self.X.device, seed=seed ^ self.KEY,
-                          offset=offset, offset_add=counter, out=(self.X, None, None))
+        after the draw when ``advance``)."""
+        sample_faces_rhs(self.per_face, self.dim, self.L, self.faces, self.ks, seed=seed ^ self.key, offset=offset,
+                         offset_add=counter, out=(self.X, self.g))
         if advance:
             counter.add_(1)
-        torch.addcmul(self._put, self.X, self._keep, out=self.X)
         return self.X
 
 
@@ -265,14 +294,20 @@ class FusedTrainer:
                the sampler's Philox counter block, ``rank_offset``) and the
                [grad | dE | sums] rows are summed over the ranks before Adam (exchange='nvlink': one kernel over
                peer memory; 'nccl': torch.distributed.all_reduce)
+    neumann_faces    face mask (face k = side k % 2 of axis k // 2, ``all_faces(dim)`` for every face) on which the
+               Neumann condition du/dn = du*/dn of the manufactured solution is imposed as the penalty term
+               mean((du/dn - g)^2), weight ``weight_neumann``, reported as ``terms['neumann']``: fresh face points every
+               epoch, n_boundary // (2d) per face, g from the same launch.  The Dirichlet ``bc`` penalty then covers the
+               other faces only.  Needs an 'RB' model (the 'FBC' envelope forces u = 0 on every face).
     """
 
     TERMS = TERMS
+    NEUMANN_KEY = 0x2545F4914F6CDD1D   # xor-ed into the seed: the Neumann face draws are independent of the others
 
     def __init__(self, model, L_box=2.0, ks=None, method='PINN', n_interior=20000, lr=1e-3, betas=(0.9, 0.999), eps=1e-8,
                  weight_pde=1.0, X=None, f=None, resample=False, seed=0, n_test=0, history=0, graph=True, group=None,
                  envelope: Optional[EnvelopeSpec] = None, exchange='nvlink', weights=None, n_boundary=4000, X_data=None,
-                 u_data=None, norm_mode='nontrivial'):
+                 u_data=None, norm_mode='nontrivial', neumann_faces=None, weight_neumann=1.0):
         from .poisson import _envelope
         self.lib = L.load()
         self.model, self.L, self.method, self.group = model, float(L_box), method, group
@@ -304,13 +339,24 @@ class FusedTrainer:
         rb = getattr(model, "bc_mode", "FBC") == 'RB' and envelope is None
         self.w = _term_weights(weights, rb, X_data is not None, pde=weight_pde)
         self.norm_mode = norm_mode
-        self.use = {'pde': True, 'bc': self.w['bc'] != 0.0, 'data': self.w['data'] != 0.0, 'norm': self.w['norm'] > 0.0}
+        self.neumann_faces = None if neumann_faces is None else int(neumann_faces)
+        dirichlet_faces = all_faces(self.dim)
+        if self.neumann_faces is not None:
+            if not rb:
+                raise ValueError("neumann_faces needs an 'RB' model without envelope: the 'FBC' envelope forces u = 0 "
+                                 "on every face")
+            if not 0 < self.neumann_faces < all_faces(self.dim) + 1:
+                raise ValueError(f"neumann_faces must be a face mask in 1 .. {all_faces(self.dim)}")
+            dirichlet_faces &= ~self.neumann_faces
+            self.w['neumann'] = float(weight_neumann)
+        self.use = {'pde': True, 'bc': self.w['bc'] != 0.0 and dirichlet_faces != 0, 'data': self.w['data'] != 0.0,
+                    'norm': self.w['norm'] > 0.0, 'neumann': self.neumann_faces is not None}
         if self.use['data'] and (X_data is None or u_data is None):
             raise ValueError("a data weight needs X_data and u_data")
         if self.use['norm'] and norm_mode == 'nontrivial' and group is not None:
             raise NotImplementedError("the 'nontrivial' norm term is a function of a global mean: not available with group "
                                       "(use norm_mode='l2' or weight 0)")
-        self.rows = [t for t in self.TERMS if self.use[t]]
+        self.rows = [t for t in self.TERMS + ('neumann',) if self.use[t]]
         self.net = _Net(model, self.X)
         self.params = [p for p in self.net.params]
         self.nparam = sum(p.numel() for p in self.params)
@@ -328,8 +374,13 @@ class FusedTrainer:
             self.total = torch.zeros(self.nparam + 2, dtype=self.dtype, device=self.dev)
             self.wvec = torch.tensor([self.w[t] for t in self.rows], dtype=self.dtype, device=self.dev)
         if self.use['bc']:
-            self.faces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev)
+            self.faces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev, faces=dirichlet_faces)
             self.nb, self.Xb = self.faces.n, self.faces.X
+        if self.use['neumann']:
+            self.nfaces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev, faces=self.neumann_faces,
+                                      ks=self.ks, key=self.NEUMANN_KEY)
+            self.nn, self.Xn, self.gn = self.nfaces.n, self.nfaces.X, self.nfaces.g
+            self.nspec = ProgramSpec(L.PROG_FLUX, alpha=1.0, faces=self.neumann_faces)
         if self.use['data']:
             self.Xd = X_data.detach().to(self.dtype).to(self.dev).contiguous()
             self.ud = u_data.detach().to(self.dtype).to(self.dev).reshape(-1).contiguous()
@@ -349,7 +400,8 @@ class FusedTrainer:
         self.hist_l2sq = torch.zeros(max(int(history), 0) if self.n_test else 0, dtype=self.dtype, device=self.dev)
         self._order = self.lib.pde_program_order(self.spec.kind)
         cnet = self.net.to_c([p.data for p in self.params])
-        n_big = max(self.n, self.n_test, getattr(self, "nb", 1), self.Xd.shape[0] if self.use['data'] else 1)
+        n_big = max(self.n, self.n_test, getattr(self, "nb", 1), getattr(self, "nn", 1),
+                    self.Xd.shape[0] if self.use['data'] else 1)
         self._ws = _ws_for(cnet, self._order, n_big, self.dev)
         self._graph = None
         self._use_graph = bool(graph)
@@ -378,6 +430,10 @@ class FusedTrainer:
             self._mse(cnet, cenv, self.faces.draw(self.seed, rank_offset(self.rank), step), None, 'bc')
         if self.use['data']:
             self._mse(cnet, cenv, self.Xd, self.ud, 'data')
+        if self.use['neumann']:
+            self.nfaces.draw(self.seed, rank_offset(self.rank), step)
+            _residual_row(cnet, cenv, self.nspec.to_c(f=self.gn), self.Xn, self.nn, 1.0 / (self.nn * self.world), self._ws,
+                          self.G[self.rows.index('neumann')], P)
         if self.use['norm']:
             if self.norm_mode == 'l2':
                 self._mse(cnet, cenv, self.X, None, 'norm')
@@ -453,8 +509,8 @@ class FusedTrainer:
 
     @property
     def terms(self):
-        """{'pde','bc','data','norm','total'} of the last evaluated epoch as 0-d device tensors
-        (what train_poisson_nd appends to its history, Poisson_ND.py:288-293)."""
+        """{'pde','bc','data','norm','total'} (and 'neumann' with ``neumann_faces``) of the last evaluated epoch as 0-d
+        device tensors (what train_poisson_nd appends to its history, Poisson_ND.py:288-293)."""
         self.check()
         out = {t: torch.zeros((), dtype=self.dtype, device=self.dev) for t in self.TERMS}
         out['pde'] = self._mean('pde', self.n)
@@ -465,6 +521,9 @@ class FusedTrainer:
         if self.use['norm']:
             out['norm'] = self._mean('norm', self.n) if self.norm_mode == 'l2' else self.norm_value
         out['total'] = sum(self.w[t] * out[t] for t in self.TERMS)
+        if self.use['neumann']:
+            out['neumann'] = self._mean('neumann', self.nn)
+            out['total'] = out['total'] + self.w['neumann'] * out['neumann']
         return out
 
     @property
