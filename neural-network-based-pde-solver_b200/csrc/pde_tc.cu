@@ -488,8 +488,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
   uint64_t* bar_wt = bar_chunk + 7;    // bulk copy of a W tile pair has landed (non-resident W only)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_chunk + 8);
   int* sTileEnd = reinterpret_cast<int*>(bar_chunk + 14);   // the epilogue's loop bound (see there)
-  // (bar_chunk + 9 is unused)
+  float* sXs = reinterpret_cast<float*>(bar_chunk + 9);    // 2^-K: the kernel's first-layer coordinates x' = 2^-K x (see there)
   float* sMx = reinterpret_cast<float*>(bar_chunk + 10);   // per-tile maximum cotangent of warps 0 and 1
+  // read where it is used: a register holding it across the tile loop would push the epilogue further into local memory
+  auto x_scale = [&]() {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(smem_u32(sXs)));
+    return v;
+  };
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int n_h = a.n_h;
@@ -506,6 +512,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
   // ---- one-time setup (all warps)
   for (int i = tid; i < D * 64 + n_h * 64; i += NTHREADS) sPar[i] = a.params[i];
   for (int i = tid; i < 64 + 1; i += NTHREADS) sWL[i] = a.params[D * 64 + n_h * 64 + i];
+  {
+    // per-warp maximum of |W0| (one entry per thread), for the epilogue's choice of K; sRed is free until the first
+    // tile's output layer
+    static_assert(D * 64 <= NTHREADS, "one W0 entry per thread");
+    const uint32_t m = __reduce_max_sync(0xffffffffu, __float_as_uint(tid < D * 64 ? fabsf(sW0t[tid]) : 0.f));
+    if (lane == 0) reinterpret_cast<uint32_t*>(sRed)[warp] = m;
+  }
   if (tid == 0 && a.mode == 0) {
     // loop-invariant scalars of the residual stage
     sWL[65] = a.energy ? a.energy[0] : a.energy_const;
@@ -1004,6 +1017,23 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
       }
     };
     if (tile_begin < tile_end) load_x(tile_begin);
+    // The kernel works in the coordinates x' = 2^-K x with first-layer weights W0' = 2^K W0, K = -round(log2 max|W0|)
+    // outside max|W0| in [2^-2, 2^2] and 0 inside (default initialisations): z = W0' x' + b is bit for bit W0 x + b, but
+    // the derivative channels carry 2^K and the Laplacian 2^2K, so that they stay O(max|W0'|) = O(1) and clear of the
+    // fp16 split's subnormal range whatever the box size (W0 ~ 1 / L), and the x^T operand of the first-layer gradient
+    // is O(|W0 x|) instead of O(L).  Every scaling is exact and undone where jets leave or cotangents enter the network
+    // (residual stage) and at the gW0 write.
+    {
+      uint32_t m = 0;
+      for (int w = 0; w < (D * 64 + 31) / 32; ++w) m = max(m, reinterpret_cast<const uint32_t*>(sRed)[w]);
+      const float mw = __uint_as_float(m);
+      // round(log2 max|W0|): the exponent, plus one when the significand is at least sqrt(2)
+      const int r = (int)((m >> 23) & 255u) - 127 + ((m & 0x7FFFFFu) >= 0x3504F3u ? 1 : 0);
+      const int k = (mw >= 0.25f && mw <= 4.f) || !(mw >= 1e-30f && mw <= 1e30f) ? 0 : -max(-60, min(60, r));
+      const float w_scale = __uint_as_float((uint32_t)(127 + k) << 23);
+      for (int i = tid; i < D * 64; i += NEPI * 32) sW0t[i] *= w_scale;
+      if (tid == 0) *sXs = __uint_as_float((uint32_t)(127 - k) << 23);
+    }
     // The epilogue is at its register limit and ptxas would keep the loop bound in local memory, whose reload misses L1
     // behind the stash traffic (~1 k cycles per tile): it is kept in shared memory instead.
     if (tid == 0) *sTileEnd = tile_end;
@@ -1034,10 +1064,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
       const float fv = stream_load_if(a.f ? a.f + base + tid : nullptr, pol_stream, in_tile && a.f != nullptr);
       const float bt_raw = stream_load_if(a.beta ? a.beta + base + tid : nullptr, pol_stream, in_tile && a.beta != nullptr);
       if (do_bwd) {
+        const float xs = x_scale();
         for (int i = tid; i < D * 32; i += NEPI * 32) {
-          const int j = i / 32, pp = 2 * (i % 32);   // row j of X^T, points pp, pp+1
+          const int j = i / 32, pp = 2 * (i % 32);   // row j of X'^T, points pp, pp+1
           uint32_t hi, lo;
-          split2(sX[pp * D + j], sX[(pp + 1) * D + j], hi, lo);
+          split2(sX[pp * D + j] * xs, sX[(pp + 1) * D + j] * xs, hi, lo);
           const uint32_t off = tile_off(j, pp >> 3) + ((pp & 7) << 1);
           sts32(sXTb + off, hi);
           sts32(sXTb + 1024 + off, lo);
@@ -1077,12 +1108,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
           tc_fence_after();
         }
         TS(20 + l);
-        float xr[2][D > 0 ? D : 1];   // first layer: this thread's point coordinates (loop-invariant)
+        float xr[2][D > 0 ? D : 1];   // first layer: this thread's point coordinates x' (loop-invariant)
         if constexpr (L0) {
+          const float xs = x_scale();
 #pragma unroll
           for (int r = 0; r < 2; ++r)
 #pragma unroll
-            for (int jd = 0; jd < D; ++jd) xr[r][jd] = sX[rows[r] * D + jd];
+            for (int jd = 0; jd < D; ++jd) xr[r][jd] = sX[rows[r] * D + jd] * xs;
         }
         float zr[C][4];  // raw accumulator fragments [channel][ (r0,u0) (r0,u0+1) (r1,u0) (r1,u0+1) ]; chunk j+1 is fetched while chunk j is processed
         float z[C][NE];  // this thread's elements
@@ -1220,6 +1252,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
 #pragma unroll
         for (int c = 0; c < C; ++c) nj[c] = sRed[tid * C + c] + sRed[(64 + tid) * C + c];
         nj[0] += sWL[64];
+        // jets in x' -> jets in x; after the program (or the cotangents read in), the same factors take cotangents of
+        // the jets in x to cotangents of the jets in x'
+        auto rescale = [&]() {
+          const float xs = x_scale();
+#pragma unroll
+          for (int i = 1; i <= ND; ++i) nj[i] *= xs;
+          if constexpr (LAP) nj[1 + ND] *= xs * xs;
+        };
+        rescale();
         bool programmed = false;
         if constexpr (ORDER <= 1 || SPLIT) {
           // jet modes (pde_jets_forward / pde_jets_backward): for order <= 1 the kernel's channels are the ABI's; the
@@ -1259,6 +1300,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             for (int c = 0; c < C; ++c) nj[c] = 0.f;   // split instantiations run in the jet modes only
           }
         }
+        rescale();
       }
       TS(2);
       if (!do_bwd) continue;
@@ -1285,26 +1327,31 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
         TSW(4);
         mx = fmaxf(sMx[0], sMx[1]);
         const float sm = adj_scale * mx;
-        if (mx > 1e-30f && mx < 3.0e38f && (adj_scale == 0.f || sm > 256.f || sm < 0.0625f)) {
+        // (cotangents down to 2^-118 are scaled: with an envelope that vanishes on a small box, u and every cotangent
+        // can be ~1e-24 while the gradients are still ordinary fp32 numbers)
+        if (mx > 1e-35f && mx < 3.0e38f && (adj_scale == 0.f || sm > 256.f || sm < 0.0625f)) {
           int ex = (int)((__float_as_uint(mx) >> 23) & 255u) - 126;       // mx = m 2^ex, m in [0.5, 1)
-          ex = max(-60, min(60, ex));
-          const float ns = __uint_as_float((uint32_t)(127 + 2 - ex) << 23);   // largest cotangent -> [2, 4)
+          ex = max(-116, min(60, ex));
+          const float ns = __uint_as_float((uint32_t)(127 + 2 - ex) << 23);   // largest cotangent -> [2, 4); ns <= 2^118
           if (adj_scale != 0.f) {
-            const float ratio = ns / adj_scale;
+            // the ratio ns / adj_scale may lie outside the fp32 range: applied as two exact factors, between which
+            // the sums stay between their old and new values
+            const int de = (int)(__float_as_uint(ns) >> 23) - (int)(__float_as_uint(adj_scale) >> 23);
+            const float r1 = __uint_as_float((uint32_t)(127 + de / 2) << 23), r2 = __uint_as_float((uint32_t)(127 + de - de / 2) << 23);
 #pragma unroll
             for (int i = 0; i < 3; ++i) {
 #pragma unroll
               for (int b = 0; b < 4; ++b)
 #pragma unroll
-                for (int e = 0; e < NE; ++e) accW[i][b][e] *= ratio;
+                for (int e = 0; e < NE; ++e) accW[i][b][e] = accW[i][b][e] * r1 * r2;
 #pragma unroll
-              for (int r = 0; r < 2; ++r) accB[i][r] *= ratio;
+              for (int r = 0; r < 2; ++r) accB[i][r] = accB[i][r] * r1 * r2;
             }
 #pragma unroll
-            for (int e = 0; e < NE; ++e) acc0[e] *= ratio;
+            for (int e = 0; e < NE; ++e) acc0[e] = acc0[e] * r1 * r2;
 #pragma unroll
-            for (int j = 0; j < 4; ++j) { gwl[j][0] *= ratio; gwl[j][1] *= ratio; }
-            gbl *= ratio;
+            for (int j = 0; j < 4; ++j) { gwl[j][0] = gwl[j][0] * r1 * r2; gwl[j][1] = gwl[j][1] * r1 * r2; }
+            gbl = gbl * r1 * r2;
           }
           adj_scale = ns;
         }
@@ -1651,11 +1698,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
         }
       }
       if (h == 0) {
-        // columns cq, cq+1 of [gW0 (D cols) | gb0]
+        // columns cq, cq+1 of [gW0 (D cols) | gb0]; the kernel's gradient is the one of W0' = 2^K W0
+        const float wk = 1.f / x_scale();   // 2^K, exact
 #pragma unroll
         for (int e = 0; e < NE; ++e) {
           const int col = cq + (e & 1), o = rows[e >> 1];
-          if (col < D) part[a.off_gW0 + o * D + col] = acc0[e] * inv;
+          if (col < D) part[a.off_gW0 + o * D + col] = acc0[e] * inv * wk;
           else if (col == D) part[a.off_gb0 + o] = acc0[e] * inv;
         }
       }
