@@ -53,8 +53,11 @@ enum {
   PDE_PROG_DRM = 2,      /* q0 = alpha*|grad u|^2 - f*u                            order 1 */
   PDE_PROG_RAYLEIGH = 3, /* q0 = alpha*|grad u|^2 + beta*u^2 ; q1 = u^2            order 1 */
   PDE_PROG_MSE = 4,      /* q0 = (u - f)^2  (f NULL -> u^2)                        order 0 */
-  PDE_PROG_FLUX = 5      /* q0 = (alpha*n.grad u + beta*u - f)^2 on box faces      order 1 */
+  PDE_PROG_FLUX = 5,     /* q0 = (alpha*n.grad u + beta*u - f)^2 on box faces      order 1 */
+  PDE_PROG_RITZ_VALUE = 7 /* q0 = beta*u^2/2 - g*u, g = f (f NULL -> alpha)        order 0 */
 };
+/* Kind 6 is not assigned: the library has always answered PDE_ERR_INVALID for it, and stays so for callers that
+ * check that answer. */
 
 /* Faces of the box [lo, hi]^dim for PDE_PROG_FLUX and pde_sample_faces_rhs: face k is x_{k/2} = lo (outward normal
  * -e_{k/2}) when k is even and x_{k/2} = hi (normal +e_{k/2}) when k is odd.  A face set is a bit mask over bits
@@ -93,7 +96,13 @@ typedef struct pde_envelope {
  * KH_1D.py:218, QHO_2D_Energy.py:287-291), else energy_const.
  * PDE_PROG_FLUX is the boundary-flux penalty of a Neumann (beta = 0) or Robin condition: f holds the prescribed data g
  * (NULL: g = 0), beta (or beta_const) the Robin coefficient, `faces` the face mask of the points (layout above); the
- * energy fields are ignored and dq/dE = 0.  The reference has no Neumann code (its README.md:23 advertises it). */
+ * energy fields are ignored and dq/dE = 0.  The reference has no Neumann code (its README.md:23 advertises it).
+ * PDE_PROG_RITZ_VALUE is the value-only term of a Deep Ritz functional (DESIGN.md §3.4b): q0 = beta*u^2/2 - g*u with
+ * beta from `beta` (or beta_const) and g from f, or the constant alpha when f is NULL; `faces` and the energy fields
+ * are ignored and dq/dE = 0.  It needs no normal, so the points may lie on any boundary.  Its uses: the Robin /
+ * Neumann boundary energy (beta = kappa, f = g on boundary points; the reference has no counterpart, its
+ * drm_energy_loss, Poisson_ND.py:98-103, is the interior half of the same functional) and the integral of u for a
+ * mean constraint (beta = 0, f = NULL, alpha = -1: q0 = u, with the caller's seed). */
 typedef struct pde_program {
   int32_t kind;        /* PDE_PROG_* */
   int32_t faces;       /* PDE_PROG_FLUX: face mask, 1 .. (1 << 2*dim) - 1; ignored by every other program */

@@ -280,7 +280,7 @@ int pde_jet_channels(int32_t dim, int32_t order) {
 
 int pde_program_quantities(int32_t kind) {
   switch (kind) {
-    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: case PDE_PROG_FLUX: return 1;
+    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: case PDE_PROG_FLUX: case PDE_PROG_RITZ_VALUE: return 1;
     case PDE_PROG_RAYLEIGH: return 2;
     default: return PDE_ERR_INVALID;
   }
@@ -290,7 +290,7 @@ int pde_program_order(int32_t kind) {
   switch (kind) {
     case PDE_PROG_PINN: return 2;
     case PDE_PROG_DRM: case PDE_PROG_RAYLEIGH: case PDE_PROG_FLUX: return 1;
-    case PDE_PROG_MSE: return 0;
+    case PDE_PROG_MSE: case PDE_PROG_RITZ_VALUE: return 0;
     default: return PDE_ERR_INVALID;
   }
 }

@@ -290,6 +290,10 @@ __device__ void program_point(const KArgs<T>& a, const T* x, long long gp, T (&n
     ub = bt * rb;
 #pragma unroll
     for (int i = 0; i < D; ++i) uib[i] = (i == ax) ? as * rb : T(0);
+  } else if (ORDER == 0 && a.prog == 7) {  // Ritz value term: q = beta u^2 / 2 - g u, g = f or alpha
+    const T g = a.f ? fv : a.alpha;
+    qs[0] += (double)(T(0.5) * bt * u * u - g * u);
+    ub = (bt * u - g) * w0;
   } else {  // MSE on the value
     T r = u - fv;
     qs[0] += (double)(r * r);

@@ -290,6 +290,10 @@ __device__ void program_point_lap(const TcArgs& a, const float* env, const float
     ub = bt * rb;
 #pragma unroll
     for (int i = 0; i < D; ++i) uib[i] = (i == ax) ? as * rb : 0.f;
+  } else if (ORDER == 0 && a.prog == PDE_PROG_RITZ_VALUE) {   // the order-1 / order-2 kernels keep their instruction stream
+    const float g = a.f ? fv : a.alpha;
+    qs[0] += (double)(0.5f * bt * u * u - g * u);
+    ub = (bt * u - g) * w0;
   } else {
     const float r = u - fv;
     qs[0] += (double)(r * r);

@@ -367,7 +367,8 @@ def mlp_jets(model: nn.Module, X: torch.Tensor, order: int = 2) -> torch.Tensor:
 @dataclass
 class ProgramSpec:
     """A residual program (pde_program).  ``faces``: face mask of a ``PROG_FLUX`` batch (include/pde_b200.h: one equal
-    block of points per set bit, face k = side k % 2 of axis k // 2); ignored by the other programs."""
+    block of points per set bit, face k = side k % 2 of axis k // 2); ignored by the other programs.  ``PROG_RITZ_VALUE``
+    reads ``alpha`` as the constant g when ``f`` is None."""
     kind: int
     alpha: float = 1.0
     beta_const: float = 0.0

@@ -131,6 +131,33 @@ def boundary_loss_neumann(model, L, N_b_per_face, dim, device, g=None, faces=Non
     or a callable g(X) -> (N,) giving the prescribed outward normal derivative.  A Robin condition
     alpha du/dn + kappa u = g is ``ops.residual_mean`` with ``ProgramSpec(PROG_FLUX, alpha, beta_const=kappa,
     faces=mask)`` on the same blocked points."""
+    X, mask = _face_batch(model, L, N_b_per_face, dim, device, faces)
+    gv = None if g is None else g(X).reshape(-1)
+    # (with group, residual_mean counts the points of this rank on every rank)
+    return residual_mean(model, X, ProgramSpec(_lib.PROG_FLUX, faces=mask), _envelope(model, L), f=gv, group=group)
+
+
+def boundary_energy_neumann(model, L, N_b_per_face, dim, device, g=None, kappa=0.0, faces=None, *, group=None):
+    """(popcount(faces) / L) mean(kappa u^2 / 2 - g u) on fresh uniform face samples: the boundary integral
+    oint (kappa u^2 / 2 - g u) ds of the Deep Ritz functional divided by |Omega| = L^dim, so that
+    ``drm_energy_loss(...) + boundary_energy_neumann(...)`` is E[u] / |Omega| on the box (DESIGN.md §3.4b).  The Ritz
+    counterpart of boundary_loss_neumann: the same face draws, one launch for all faces (PROG_RITZ_VALUE).
+
+    The minimiser of that sum satisfies du/dn + kappa u = g on the faces of the mask (Neumann for kappa = 0) with no
+    penalty weight.  Faces outside the mask get the natural condition du/dn = 0 in this form, unless another term (a
+    Dirichlet penalty) constrains them.  ``g``: None (g = 0) or a callable g(X) -> (N,); ``faces``: face mask, face
+    k = (coordinate k // 2, side k % 2: 0 or L), default every face."""
+    X, mask = _face_batch(model, L, N_b_per_face, dim, device, faces)
+    gv = None if g is None else g(X).reshape(-1)
+    # alpha is the constant g when f is NULL: 0 here
+    spec = ProgramSpec(_lib.PROG_RITZ_VALUE, alpha=0.0, beta_const=float(kappa))
+    e = residual_mean(model, X, spec, _envelope(model, L), f=gv, group=group)
+    return e * (bin(mask).count("1") / L)
+
+
+def _face_batch(model, L, N_b_per_face, dim, device, faces):
+    """(X, mask): ``N_b_per_face`` torch.rand points on each face of the mask (default every face) in the order of
+    boundary_loss_dirichlet (Poisson_ND.py:130-141), one block per set bit in increasing bit order."""
     dtype = next(model.parameters()).dtype
     mask = (1 << 2 * dim) - 1 if faces is None else int(faces)
     if not 0 < mask < 1 << 2 * dim:
@@ -142,10 +169,16 @@ def boundary_loss_neumann(model, L, N_b_per_face, dim, device, g=None, faces=Non
                 X = torch.rand(N_b_per_face, dim, device=device, dtype=dtype) * L
                 X[:, i] = L if at_L else 0.0
                 blocks.append(X)
-    X = torch.cat(blocks)
-    gv = None if g is None else g(X).reshape(-1)
-    # (with group, residual_mean counts the points of this rank on every rank)
-    return residual_mean(model, X, ProgramSpec(_lib.PROG_FLUX, faces=mask), _envelope(model, L), f=gv, group=group)
+    return torch.cat(blocks), mask
+
+
+def mean_value_loss(model, X, L, c=0.0, *, group=None, n_global=None):
+    """(mean_X u - c)^2: the constraint that fixes the additive constant of a pure-Neumann problem (DESIGN.md §3.4b).
+    One residual call of PROG_RITZ_VALUE with q = u (beta = 0, f = None, alpha = -1); autograd supplies the factor
+    2 (m - c) for its gradient, which is exact under ``group`` because the mean m is recombined over the ranks first."""
+    m = residual_mean(model, X, ProgramSpec(_lib.PROG_RITZ_VALUE, alpha=-1.0), _envelope(model, L), group=group,
+                      n_global=n_global)
+    return (m - c) ** 2
 
 
 def data_loss(model, X_data, u_data, L, *, group=None, n_global=None):

@@ -19,6 +19,7 @@ reference's arithmetic (Adam: torch.optim.Adam defaults, single-tensor formula).
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional, Sequence
 
 import torch
@@ -299,6 +300,15 @@ class FusedTrainer:
                mean((du/dn - g)^2), weight ``weight_neumann``, reported as ``terms['neumann']``: fresh face points every
                epoch, n_boundary // (2d) per face, g from the same launch.  The Dirichlet ``bc`` penalty then covers the
                other faces only.  Needs an 'RB' model (the 'FBC' envelope forces u = 0 on every face).
+    robin_kappa      kappa of the Robin condition du/dn + kappa u = g on the ``neumann_faces`` (0: Neumann), in either
+               form; g = du*/dn + kappa u* on the face points (u* from one sample_points_rhs launch on those points)
+    neumann_form     'penalty': the row above (PROG_FLUX, beta = kappa); 'ritz' (method='DRM' only): the boundary term
+               of the Deep Ritz functional, mean(kappa u^2 / 2 - g u) on the same face points (PROG_RITZ_VALUE), with
+               the weight the functional fixes, the pde weight * popcount(neumann_faces) / L (DESIGN.md §3.4b);
+               ``weight_neumann`` (default 1) is for the penalty form only
+    mean_value       add the row 'mean' = (mean_X u - c*)^2 on the interior points, weight ``weight_mean``, with c* the
+               exact mean of u* over the box: it fixes the additive constant of a pure-Neumann problem
+               (``neumann_faces=all_faces(dim)``).  Not available with ``group``.
     """
 
     TERMS = TERMS
@@ -307,7 +317,8 @@ class FusedTrainer:
     def __init__(self, model, L_box=2.0, ks=None, method='PINN', n_interior=20000, lr=1e-3, betas=(0.9, 0.999), eps=1e-8,
                  weight_pde=1.0, X=None, f=None, resample=False, seed=0, n_test=0, history=0, graph=True, group=None,
                  envelope: Optional[EnvelopeSpec] = None, exchange='nvlink', weights=None, n_boundary=4000, X_data=None,
-                 u_data=None, norm_mode='nontrivial', neumann_faces=None, weight_neumann=1.0):
+                 u_data=None, norm_mode='nontrivial', neumann_faces=None, weight_neumann=None, neumann_form='penalty',
+                 robin_kappa=0.0, mean_value=False, weight_mean=1.0):
         from .poisson import _envelope
         self.lib = L.load()
         self.model, self.L, self.method, self.group = model, float(L_box), method, group
@@ -315,6 +326,18 @@ class FusedTrainer:
         self.dev, self.dtype = p0.device, p0.dtype
         if method not in ('PINN', 'DRM'):
             raise ValueError("method must be one of {'PINN','DRM'}")
+        if neumann_form not in ('penalty', 'ritz'):
+            raise ValueError("neumann_form must be 'penalty' or 'ritz'")
+        if neumann_form == 'ritz':
+            if method != 'DRM' or neumann_faces is None:
+                raise ValueError("neumann_form='ritz' is the boundary term of the Deep Ritz functional: it needs "
+                                 "method='DRM' and neumann_faces")
+            if weight_neumann is not None:
+                raise ValueError("the Ritz boundary term has the weight the functional fixes; weight_neumann is for "
+                                 "neumann_form='penalty'")
+        if mean_value and group is not None:
+            raise NotImplementedError("the mean-value constraint is a function of a global mean: not available with "
+                                      "group")
         if norm_mode not in ('nontrivial', 'l2'):
             raise ValueError("norm mode should be 'nontrivial' or 'l2'")
         self.env = envelope if envelope is not None else _envelope(model, L_box)
@@ -348,15 +371,23 @@ class FusedTrainer:
             if not 0 < self.neumann_faces < all_faces(self.dim) + 1:
                 raise ValueError(f"neumann_faces must be a face mask in 1 .. {all_faces(self.dim)}")
             dirichlet_faces &= ~self.neumann_faces
-            self.w['neumann'] = float(weight_neumann)
+            if neumann_form == 'ritz':    # the boundary integral over |Omega|: popcount faces of area L^(d-1) / L^d
+                self.w['neumann'] = self.w['pde'] * bin(self.neumann_faces).count("1") / self.L
+            else:
+                self.w['neumann'] = 1.0 if weight_neumann is None else float(weight_neumann)
+        self.neumann_form, self.kappa = neumann_form, float(robin_kappa)
+        if mean_value:
+            self.w['mean'] = float(weight_mean)
+            # c* = mean of u* = prod_i sin(k_i pi x_i / L) over [0, L]^d
+            self.c_mean = math.prod((1.0 - math.cos(k * math.pi)) / (k * math.pi) for k in self.ks)
         self.use = {'pde': True, 'bc': self.w['bc'] != 0.0 and dirichlet_faces != 0, 'data': self.w['data'] != 0.0,
-                    'norm': self.w['norm'] > 0.0, 'neumann': self.neumann_faces is not None}
+                    'norm': self.w['norm'] > 0.0, 'neumann': self.neumann_faces is not None, 'mean': bool(mean_value)}
         if self.use['data'] and (X_data is None or u_data is None):
             raise ValueError("a data weight needs X_data and u_data")
         if self.use['norm'] and norm_mode == 'nontrivial' and group is not None:
             raise NotImplementedError("the 'nontrivial' norm term is a function of a global mean: not available with group "
                                       "(use norm_mode='l2' or weight 0)")
-        self.rows = [t for t in self.TERMS + ('neumann',) if self.use[t]]
+        self.rows = [t for t in self.TERMS + ('neumann', 'mean') if self.use[t]]
         self.net = _Net(model, self.X)
         self.params = [p for p in self.net.params]
         self.nparam = sum(p.numel() for p in self.params)
@@ -380,7 +411,12 @@ class FusedTrainer:
             self.nfaces = _FacePoints(n_boundary, self.dim, self.L, self.dtype, self.dev, faces=self.neumann_faces,
                                       ks=self.ks, key=self.NEUMANN_KEY)
             self.nn, self.Xn, self.gn = self.nfaces.n, self.nfaces.X, self.nfaces.g
-            self.nspec = ProgramSpec(L.PROG_FLUX, alpha=1.0, faces=self.neumann_faces)
+            if neumann_form == 'ritz':
+                self.nspec = ProgramSpec(L.PROG_RITZ_VALUE, alpha=0.0, beta_const=self.kappa)
+            else:
+                self.nspec = ProgramSpec(L.PROG_FLUX, alpha=1.0, beta_const=self.kappa, faces=self.neumann_faces)
+            if self.kappa != 0.0:
+                self.un = torch.empty(self.nn, dtype=self.dtype, device=self.dev)    # u* on the face points
         if self.use['data']:
             self.Xd = X_data.detach().to(self.dtype).to(self.dev).contiguous()
             self.ud = u_data.detach().to(self.dtype).to(self.dev).reshape(-1).contiguous()
@@ -388,6 +424,11 @@ class FusedTrainer:
             self.nsum = torch.zeros(1, dtype=self.dtype, device=self.dev)
             self.nseed = torch.ones(1, dtype=self.dtype, device=self.dev)
             self.norm_value = torch.zeros((), dtype=self.dtype, device=self.dev)
+        if self.use['mean']:
+            self.msum = torch.zeros(1, dtype=self.dtype, device=self.dev)
+            self.mseed = torch.ones(1, dtype=self.dtype, device=self.dev)
+            self.mean_term = torch.zeros((), dtype=self.dtype, device=self.dev)
+            self.mspec = ProgramSpec(L.PROG_RITZ_VALUE, alpha=-1.0)     # q = u
         self.n_test = int(n_test)
         if self.n_test:
             self.Xt = torch.empty(self.n_test, self.dim, dtype=self.dtype, device=self.dev)
@@ -432,6 +473,9 @@ class FusedTrainer:
             self._mse(cnet, cenv, self.Xd, self.ud, 'data')
         if self.use['neumann']:
             self.nfaces.draw(self.seed, rank_offset(self.rank), step)
+            if self.kappa != 0.0:     # g = du*/dn + kappa u*
+                sample_points_rhs(0, 0, self.L, self.ks, X=self.Xn, out=(None, self.un, None))
+                self.gn.add_(self.un, alpha=self.kappa)
             _residual_row(cnet, cenv, self.nspec.to_c(f=self.gn), self.Xn, self.nn, 1.0 / (self.nn * self.world), self._ws,
                           self.G[self.rows.index('neumann')], P)
         if self.use['norm']:
@@ -444,6 +488,15 @@ class FusedTrainer:
                 torch.neg(torch.reciprocal((m + 1e-8) ** 2), out=self.nseed)
                 self._mse(cnet, cenv, self.X, None, 'norm', seed=self.nseed)
                 self.norm_value.copy_(torch.reciprocal(m + 1e-8)[0])
+        if self.use['mean']:
+            # (m - c*)^2, m = mean u: the mean first, then the reverse sweep seeded with 2 (m - c*)
+            row_m = self.G[self.rows.index('mean')]
+            _residual_row(cnet, cenv, self.mspec.to_c(), self.X, self.n, inv_n, self._ws, None, P, sums=self.msum,
+                          want_grad=False)
+            dm = self.msum * inv_n - self.c_mean
+            torch.mul(dm, 2.0, out=self.mseed)
+            _residual_row(cnet, cenv, self.mspec.to_c(), self.X, self.n, inv_n, self._ws, row_m, P, seed=self.mseed)
+            self.mean_term.copy_((dm * dm)[0])
         if self._ar is not None:
             if fused_ar is None:
                 self._ar.all_reduce_(self.G.view(-1))
@@ -509,8 +562,9 @@ class FusedTrainer:
 
     @property
     def terms(self):
-        """{'pde','bc','data','norm','total'} (and 'neumann' with ``neumann_faces``) of the last evaluated epoch as 0-d
-        device tensors (what train_poisson_nd appends to its history, Poisson_ND.py:288-293)."""
+        """{'pde','bc','data','norm','total'} (and 'neumann' with ``neumann_faces``: the row's mean in either form,
+        'mean' with ``mean_value``) of the last evaluated epoch as 0-d device tensors (what train_poisson_nd appends to
+        its history, Poisson_ND.py:288-293); 'total' includes every term with its weight."""
         self.check()
         out = {t: torch.zeros((), dtype=self.dtype, device=self.dev) for t in self.TERMS}
         out['pde'] = self._mean('pde', self.n)
@@ -524,6 +578,9 @@ class FusedTrainer:
         if self.use['neumann']:
             out['neumann'] = self._mean('neumann', self.nn)
             out['total'] = out['total'] + self.w['neumann'] * out['neumann']
+        if self.use['mean']:
+            out['mean'] = self.mean_term
+            out['total'] = out['total'] + self.w['mean'] * out['mean']
         return out
 
     @property
