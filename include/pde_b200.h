@@ -54,10 +54,11 @@ enum {
   PDE_PROG_RAYLEIGH = 3, /* q0 = alpha*|grad u|^2 + beta*u^2 ; q1 = u^2            order 1 */
   PDE_PROG_MSE = 4,      /* q0 = (u - f)^2  (f NULL -> u^2)                        order 0 */
   PDE_PROG_FLUX = 5,     /* q0 = (alpha*n.grad u + beta*u - f)^2 on box faces      order 1 */
-  PDE_PROG_RITZ_VALUE = 7 /* q0 = beta*u^2/2 - g*u, g = f (f NULL -> alpha)        order 0 */
+  PDE_PROG_RITZ_VALUE = 7, /* q0 = beta*u^2/2 - g*u, g = f (f NULL -> alpha)       order 0 */
+  PDE_PROG_PARABOLIC = 9   /* q0 = (du/dt + alpha*Lap_x(u) + (beta-E)*u - f)^2, t = x_{dim-1}  order 2 */
 };
-/* Kind 6 is not assigned: the library has always answered PDE_ERR_INVALID for it, and stays so for callers that
- * check that answer. */
+/* Kinds 6 and 8 are not assigned: the library has always answered PDE_ERR_INVALID for them, and stays so for callers
+ * that check that answer. */
 
 /* Faces of the box [lo, hi]^dim for PDE_PROG_FLUX and pde_sample_faces_rhs: face k is x_{k/2} = lo (outward normal
  * -e_{k/2}) when k is even and x_{k/2} = hi (normal +e_{k/2}) when k is odd.  A face set is a bit mask over bits
@@ -102,7 +103,15 @@ typedef struct pde_envelope {
  * are ignored and dq/dE = 0.  It needs no normal, so the points may lie on any boundary.  Its uses: the Robin /
  * Neumann boundary energy (beta = kappa, f = g on boundary points; the reference has no counterpart, its
  * drm_energy_loss, Poisson_ND.py:98-103, is the interior half of the same functional) and the integral of u for a
- * mean constraint (beta = 0, f = NULL, alpha = -1: q0 = u, with the caller's seed). */
+ * mean constraint (beta = 0, f = NULL, alpha = -1: q0 = u, with the caller's seed).
+ * PDE_PROG_PARABOLIC is the space-time residual of a parabolic equation (DESIGN.md §3.4c).  The LAST coordinate is time:
+ * x = (x_0 .. x_{dim-2}, t), dim = 2..5, and Lap_x = sum_{i < dim-1} d^2/dx_i^2 is the spatial Laplacian.  beta, E and
+ * f are as for PDE_PROG_PINN (per-point or constant beta, energy pointer or constant, f NULL -> 0), dq/dE = -2 r u.  The
+ * heat equation u_t = kappa Lap_x u + s is alpha = -kappa, beta = 0, f = s.  In the face layout above the spatial faces
+ * are the mask (1 << 2*(dim-1)) - 1 and the initial face t = lo is bit 2*(dim-1): initial and boundary data are
+ * PDE_PROG_MSE (or PDE_PROG_FLUX) calls on such points.  The program uses the jets of order 2, so
+ * pde_workspace_bytes(net, 2, n) covers it on both kernel families, and it has as many jet channels as PDE_PROG_PINN at
+ * the same dim. */
 typedef struct pde_program {
   int32_t kind;        /* PDE_PROG_* */
   int32_t faces;       /* PDE_PROG_FLUX: face mask, 1 .. (1 << 2*dim) - 1; ignored by every other program */
@@ -153,7 +162,11 @@ int pde_jets_backward(const pde_net* net, int32_t order, const void* X, int64_t 
  *   seed   : device (K) or NULL (all ones) — dLoss/dmean_k, lets functions of means
  *            (Rayleigh quotient, WAN) and multi-GPU exact recombination share one kernel.
  * A PDE_PROG_FLUX call returns PDE_ERR_INVALID, before it enqueues anything, when faces == 0,
- * faces >= 1 << 2*dim or n_points is not a multiple of popcount(faces); so does the _exchange variant below. */
+ * faces >= 1 << 2*dim or n_points is not a multiple of popcount(faces); so does the _exchange variant below.
+ * A PDE_PROG_PARABOLIC call returns PDE_ERR_INVALID, before it enqueues anything, when dim < 2 (there is no spatial
+ * axis) or when env is non-NULL with a kind other than PDE_ENV_NONE or any n_nodes[i] != 0: every envelope vanishes at
+ * both ends of every axis, the time axis included, which is wrong for an initial-value problem.  So does the _exchange
+ * variant below. */
 int pde_residual_loss_grad(const pde_net* net, const pde_envelope* env, const pde_program* prog,
                            const void* X, int64_t n_points, const void* seed, double inv_n,
                            void* sums, void* grad, void* energy_grad, void* workspace,

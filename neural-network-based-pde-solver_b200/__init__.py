@@ -13,9 +13,10 @@ from ._lib import PdeError, load as load_library
 from .ops import (NO_ENVELOPE, EnvelopeSpec, ProgramSpec, WanSpec, all_reduce_grads, frozen_jets, mlp_jets,
                   residual_means, wan_means)
 from . import poisson
+from . import heat
 from . import schrodinger
 from . import train
 from . import comm
 
 __all__ = ["PdeError", "load_library", "EnvelopeSpec", "ProgramSpec", "WanSpec", "NO_ENVELOPE", "mlp_jets",
-           "residual_means", "wan_means", "frozen_jets", "all_reduce_grads", "poisson", "schrodinger", "train", "comm"]
+           "residual_means", "wan_means", "frozen_jets", "all_reduce_grads", "poisson", "heat", "schrodinger", "train", "comm"]

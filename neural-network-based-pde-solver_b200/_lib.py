@@ -13,6 +13,7 @@ F32, F64 = 0, 1
 ACT_SIN, ACT_TANH = 0, 1
 ENV_NONE, ENV_POLY, ENV_EXPWIN = 0, 1, 2
 PROG_PINN, PROG_DRM, PROG_RAYLEIGH, PROG_MSE, PROG_FLUX, PROG_RITZ_VALUE = 1, 2, 3, 4, 5, 7   # (6 is not assigned)
+PROG_PARABOLIC = 9   # (8 is not assigned)
 
 EXPORTS = [
     "pde_abi_version", "pde_strerror", "pde_param_count", "pde_jet_channels", "pde_program_quantities",

@@ -280,7 +280,9 @@ int pde_jet_channels(int32_t dim, int32_t order) {
 
 int pde_program_quantities(int32_t kind) {
   switch (kind) {
-    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: case PDE_PROG_FLUX: case PDE_PROG_RITZ_VALUE: return 1;
+    case PDE_PROG_PINN: case PDE_PROG_DRM: case PDE_PROG_MSE: case PDE_PROG_FLUX: case PDE_PROG_RITZ_VALUE:
+    case PDE_PROG_PARABOLIC:
+      return 1;
     case PDE_PROG_RAYLEIGH: return 2;
     default: return PDE_ERR_INVALID;
   }
@@ -288,7 +290,7 @@ int pde_program_quantities(int32_t kind) {
 
 int pde_program_order(int32_t kind) {
   switch (kind) {
-    case PDE_PROG_PINN: return 2;
+    case PDE_PROG_PINN: case PDE_PROG_PARABOLIC: return 2;
     case PDE_PROG_DRM: case PDE_PROG_RAYLEIGH: case PDE_PROG_FLUX: return 1;
     case PDE_PROG_MSE: case PDE_PROG_RITZ_VALUE: return 0;
     default: return PDE_ERR_INVALID;
@@ -348,6 +350,14 @@ static int residual_loss_grad_impl(const pde_net* net, const pde_envelope* env, 
     if (net->dim < 1 || net->dim > PDE_MAX_DIM) return PDE_ERR_UNSUPPORTED;
     if (prog->faces <= 0 || prog->faces >= (1 << (2 * net->dim))) return PDE_ERR_INVALID;
     if (n_points % __builtin_popcount((unsigned)prog->faces) != 0) return PDE_ERR_INVALID;
+  }
+  if (prog->kind == PDE_PROG_PARABOLIC) {   // a spatial axis besides time, and no envelope (include/pde_b200.h)
+    if (net->dim < 2) return PDE_ERR_INVALID;
+    if (env) {
+      if (env->kind != PDE_ENV_NONE) return PDE_ERR_INVALID;
+      for (int i = 0; i < PDE_MAX_DIM; ++i)
+        if (env->n_nodes[i] != 0) return PDE_ERR_INVALID;
+    }
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // Blackwell tensor-core path for the shapes it covers (fp32, H = 64 sin/tanh nets); it

@@ -247,16 +247,24 @@ __device__ void program_point(const KArgs<T>& a, const T* x, long long gp, T (&n
   T ub = T(0), uib[D], uiib[D];
 #pragma unroll
   for (int i = 0; i < D; ++i) { uib[i] = T(0); uiib[i] = T(0); }
-  if (a.prog == 1) {  // PINN
+  if (a.prog == 1 || (ORDER == 2 && a.prog == 9)) {
+    // PINN; parabolic (order 2 only): time t = x_{D-1} leaves the Laplacian and r gains u_t
+    const bool par = ORDER == 2 && a.prog == 9;
     T lap = T(0);
 #pragma unroll
-    for (int i = 0; i < D; ++i) lap += uii[i];
+    for (int i = 0; i < D; ++i)
+      if (i < D - 1 || !par) lap += uii[i];
     T r = a.alpha * lap + (bt - E) * u - fv;
+    if (par) r += ui[D - 1];
     qs[0] += (double)(r * r);
     T rb = T(2) * r * w0;
     ub = (bt - E) * rb;
 #pragma unroll
     for (int i = 0; i < D; ++i) uiib[i] = a.alpha * rb;
+    if (par) {
+      uiib[D - 1] = T(0);
+      uib[D - 1] = rb;
+    }
     gE += (double)(-u * rb);
   } else if (a.prog == 2) {  // Deep Ritz
     T g2 = T(0);

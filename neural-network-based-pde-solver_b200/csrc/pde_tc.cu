@@ -223,10 +223,28 @@ __device__ void envelope_point(const TcArgs& a, const float* x, float* out) {
   }
   if constexpr (ORDER == 2) out[1 + D] = LB;
 }
-template <int D, int ORDER>
+// NLAP < D (parabolic instantiations, order 2): the Laplacian channel carries the sum over the first NLAP = D - 1
+// directions only, Lap_x u, and derivative channel D is du/dt.  Those instantiations run PDE_PROG_PARABOLIC alone, with
+// no envelope (the library refuses one for that program), so u = N0.
+template <int D, int ORDER, int NLAP = D>
 __device__ void program_point_lap(const TcArgs& a, const float* env, const float* cst, float fv, float bt, long long gp,
                                   float (&nj)[1 + (ORDER >= 1 ? D : 0) + (ORDER == 2)], double (&qs)[4], double& gE) {
   constexpr int ND = (ORDER >= 1) ? D : 0;
+  if constexpr (NLAP < ND) {
+    static_assert(ORDER == 2 && NLAP == D - 1, "parabolic instantiations: order 2, time is the last direction");
+    const float E = cst[0], w0 = cst[1];
+    const float u = nj[0];
+    const float r = nj[D] + a.alpha * nj[1 + ND] + (bt - E) * u - fv;
+    qs[0] += (double)(r * r);
+    const float rb = 2.f * r * w0;
+    nj[0] = (bt - E) * rb;
+#pragma unroll
+    for (int i = 0; i < D - 1; ++i) nj[1 + i] = 0.f;
+    nj[D] = rb;
+    nj[1 + ND] = a.alpha * rb;
+    gE += (double)(-u * rb);
+    return;
+  }
   const float B = env[0];
   float Bi[D], LB = 0.f;
 #pragma unroll
@@ -463,9 +481,14 @@ __device__ __forceinline__ bool elect_one() {
 // NDIR < D: dimension-split instantiation — jets along the NDIR directions dir0 .. dir0+NDIR-1 only (value, NDIR first
 // derivatives, the partial Laplacian over those directions); jet modes only.  The 5-D PINN step, whose 7 channels do
 // not fit on chip, is two such passes (3 + 2 directions) around a pointwise residual kernel (tc_pinn_split).
-template <int D, int ORDER, int ACT, int NDIR = D>
+// NLAP < NDIR (order 2, NLAP = D - 1): the Laplacian channel sums over the first NLAP derivative directions only, so the
+// last derivative channel is du/dt and the Laplacian channel Lap_x u (PDE_PROG_PARABOLIC; residual mode only).  Same
+// channels, stash and shared-memory plan as the NLAP = NDIR instantiation; the sums S = sum z_i^2 below are guarded by
+// `i < NLAP`, which the unrolled loops resolve at compile time.
+template <int D, int ORDER, int ACT, int NDIR = D, int NLAP = NDIR>
 __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
   constexpr int ND = (ORDER >= 1) ? NDIR : 0;
+  static_assert(NLAP == NDIR || (ORDER == 2 && NDIR == D && NLAP == D - 1), "restricted Laplacian: order 2, time last");
   constexpr bool SPLIT = (NDIR != D);
   const int dir0 = SPLIT ? a.dir0 : 0;
   constexpr int LAP = (ORDER == 2) ? 1 : 0;
@@ -1184,7 +1207,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
               for (int i = 0; i < ND; ++i) {
                 const f32x2 Z = pk2(z[1 + i][e], z[1 + i][e + 1]);
                 unpk2(mul2(S1, Z), av[1 + i][e], av[1 + i][e + 1]);
-                S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
+                if (i < NLAP) S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
               }
               if constexpr (LAP)
                 unpk2(fma2(S1, pk2(z[1 + ND][e], z[1 + ND][e + 1]), mul2(pk2(s2a, s2b), S)), av[1 + ND][e], av[1 + ND][e + 1]);
@@ -1286,7 +1309,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             double tq[4], tg;
             q_load(tq, tg);
             if (gp < a.n) {
-              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, tq, tg);
+              program_point_lap<D, ORDER, NLAP>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, tq, tg);
             } else {
 #pragma unroll
               for (int c = 0; c < C; ++c) nj[c] = 0.f;
@@ -1294,7 +1317,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
             q_store(tq, tg);
           } else if constexpr (!SPLIT) {
             if (gp < a.n) {
-              program_point_lap<D, ORDER>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, qs, gE);
+              program_point_lap<D, ORDER, NLAP>(a, sNb + tid * C, sWL + 65, fv, a.beta ? bt_raw : a.beta_const, gp, nj, qs, gE);
             } else {
 #pragma unroll
               for (int c = 0; c < C; ++c) nj[c] = 0.f;
@@ -1447,7 +1470,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
               for (int i = 0; i < ND; ++i) {
                 const f32x2 Z = pk2(zp[1 + i][e], zp[1 + i][e + 1]);
                 unpk2(mul2(S1, Z), ap[1 + i][e], ap[1 + i][e + 1]);
-                S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
+                if (i < NLAP) S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
               }
               if constexpr (LAP)
                 unpk2(fma2(S1, pk2(zp[1 + ND][e], zp[1 + ND][e + 1]), mul2(pk2(s2a, s2b), S)), ap[1 + ND][e], ap[1 + ND][e + 1]);
@@ -1522,10 +1545,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_kernel(const TcArgs a) {
                   const f32x2 Z = pk2(zj[1 + i][e], zj[1 + i][e + 1]);
                   const f32x2 AB = pk2(ab[1 + i][e], ab[1 + i][e + 1]);
                   const f32x2 S2Z = mul2(S2, Z);
-                  T0 = fma2(S2Z, AB, T0);
-                  S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
+                  T0 = fma2(S2Z, AB, T0);   // every a_i = s'(z0) z_i depends on z0, Laplacian direction or not
+                  if (i < NLAP) S = (i == 0) ? mul2(Z, Z) : fma2(Z, Z, S);
                   f32x2 Ti = mul2(S1, AB);
-                  if constexpr (LAP) Ti = fma2(add2(S2Z, S2Z), ABL, Ti);
+                  if constexpr (LAP) {
+                    if (i < NLAP) Ti = fma2(add2(S2Z, S2Z), ABL, Ti);
+                  }
                   unpk2(Ti, zb[1 + i][e], zb[1 + i][e + 1]);
                 }
                 if constexpr (LAP) {
@@ -1863,22 +1888,24 @@ __global__ void tc_pack_kernel(const TcPackArgs a) {
 struct TcPlan {
   int D, order, C, NV, n_lin, n_h, H, grid, num_tiles, sms;
   int ndir;   // derivative directions of this launch (= D except in the dimension-split passes)
+  int nlap;   // leading derivative directions summed into the Laplacian channel (= ndir except PDE_PROG_PARABOLIC: D - 1)
   size_t smem_bytes;
   GradLayout g;
   long long stash_f4;
   size_t ws_params, ws_wimg, ws_partial, ws_psums, ws_stash, ws_total;
 };
 
-template <int D, int ORDER, int ACT, int NDIR = D>
+template <int D, int ORDER, int ACT, int NDIR = D, int NLAP = NDIR>
 static cudaError_t launch_one(const TcPlan& p, const TcArgs& a, cudaStream_t st) {
   constexpr int C = 1 + (ORDER >= 1 ? NDIR : 0) + (ORDER == 2);
   if constexpr (C > MAXC) {
     return cudaErrorInvalidValue;
   } else {
     const int smem = SmemMap<D, C>::total;
-    cudaError_t err = cudaFuncSetAttribute(tc_kernel<D, ORDER, ACT, NDIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    cudaError_t err =
+        cudaFuncSetAttribute(tc_kernel<D, ORDER, ACT, NDIR, NLAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (err != cudaSuccess) return err;
-    tc_kernel<D, ORDER, ACT, NDIR><<<p.grid, NTHREADS, smem, st>>>(a);
+    tc_kernel<D, ORDER, ACT, NDIR, NLAP><<<p.grid, NTHREADS, smem, st>>>(a);
     return cudaGetLastError();
   }
 }
@@ -1889,6 +1916,16 @@ static cudaError_t launch_act(const TcPlan& p, const TcArgs& a, cudaStream_t st)
 #if !defined(PDE_TC_ONLY_CFG2) && !defined(PDE_TC_ONLY_SMALL)
     if (p.D == 5 && p.order == 2 && p.ndir == 3) return launch_one<5, 2, ACT, 3>(p, a, st);
     if (p.D == 5 && p.order == 2 && p.ndir == 2) return launch_one<5, 2, ACT, 2>(p, a, st);
+#endif
+    return cudaErrorInvalidValue;
+  }
+  if (p.nlap != p.ndir) {   // PDE_PROG_PARABOLIC: the Laplacian over the spatial directions 0 .. D-2
+#if !defined(PDE_TC_ONLY_CFG2) && !defined(PDE_TC_ONLY_SMALL)
+    if (p.order == 2 && p.nlap == p.D - 1) {
+      if (p.D == 2) return launch_one<2, 2, ACT, 2, 1>(p, a, st);
+      if (p.D == 3) return launch_one<3, 2, ACT, 3, 2>(p, a, st);
+      if (p.D == 4) return launch_one<4, 2, ACT, 4, 3>(p, a, st);
+    }
 #endif
     return cudaErrorInvalidValue;
   }
@@ -1986,7 +2023,7 @@ static bool shape_ok(const pde_net* net, int order, long long n, int ndir = -1) 
   return n >= 4096;   // below that the launch is latency bound and the generic kernel is as fast
 }
 
-static int make_plan(const pde_net* net, int order, long long n, TcPlan* pl, int ndir = -1) {
+static int make_plan(const pde_net* net, int order, long long n, TcPlan* pl, int ndir = -1, int nlap = -1) {
   if (!shape_ok(net, order, n, ndir)) return PDE_ERR_UNSUPPORTED;
   const DevInfo dv = device_info();
   if (!dv.ok) return PDE_ERR_NO_DEVICE;
@@ -1996,6 +2033,7 @@ static int make_plan(const pde_net* net, int order, long long n, TcPlan* pl, int
   p.sms = dv.sms;
   p.D = net->dim; p.order = order;
   p.ndir = ndir < 0 ? p.D : ndir;
+  p.nlap = nlap < 0 ? p.ndir : nlap;
   p.C = 1 + (order >= 1 ? p.ndir : 0) + (order == 2);
   p.NV = 1 + p.C;
   p.n_lin = net->n_linear; p.n_h = p.n_lin - 1; p.H = net->widths[1];
@@ -2104,15 +2142,21 @@ static int make_split_plan(const pde_net* net, long long n, SplitPlan* sp) {
   return PDE_OK;
 }
 
+// Laplacian directions of a program's order-2 plan: the spatial ones (all but the last) for PDE_PROG_PARABOLIC, else all.
+static int lap_dirs(const pde_net* net, const pde_program* prog) {
+  return (net && prog && prog->kind == PDE_PROG_PARABOLIC) ? net->dim - 1 : -1;
+}
+
 bool tc_supported(const pde_net* net, const pde_program* prog, long long n_points) {
   if (!program_ok(prog)) return false;
   const int order = pde_program_order(prog->kind);
   if (split_shape(net, order)) {
+    if (prog->kind != PDE_PROG_PINN) return false;   // the split passes serve the PINN step only (tc_residual_loss_grad)
     SplitPlan sp;
     return make_split_plan(net, n_points, &sp) == PDE_OK;
   }
   tc::TcPlan p;
-  return tc::make_plan(net, order, n_points, &p) == PDE_OK;
+  return tc::make_plan(net, order, n_points, &p, -1, lap_dirs(net, prog)) == PDE_OK;
 }
 
 int tc_workspace_bytes(const pde_net* net, int order, long long n_points, size_t* bytes) {
@@ -2136,7 +2180,7 @@ static int tc_run(const pde_net* net, int order, int mode, const pde_envelope* e
                   void* energy_grad, void* workspace, size_t workspace_bytes, cudaStream_t st, const ExchangeReq* ex = nullptr) {
   using namespace tc;
   TcPlan p;
-  int rc = make_plan(net, order, n_points, &p);
+  int rc = make_plan(net, order, n_points, &p, -1, mode == 0 ? lap_dirs(net, prog) : -1);
   if (rc) return rc;
   if ((rc = check_ptrs(net))) return rc;
   if (!X || !workspace) return PDE_ERR_INVALID;
