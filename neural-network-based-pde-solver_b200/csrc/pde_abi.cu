@@ -107,6 +107,9 @@ int make_plan(const pde_net* net, int order, long long n, Plan* pl) {
   int regs_alloc = (regs + 7) & ~7;
   int max_threads_regs = (65536 / regs_alloc) & ~31;
   if (max_threads_regs > 1024) max_threads_regs = 1024;
+  // The runtime's own limit for this kernel is below that estimate for some register counts (197 registers: the
+  // estimate allows 320 threads, a launch of 320 or 300 fails); a block larger than it does not launch at all.
+  if (ki.max_threads > 0 && max_threads_regs > ki.max_threads) max_threads_regs = ki.max_threads & ~31;
 
   const int budget1 = dv.smem_optin;                              // one CTA per SM
   const int budget2 = (dv.smem_optin + 1024) / 2 - 1024;          // two CTAs per SM

@@ -7,9 +7,13 @@ namespace pde {
 template <typename T, int D, int ORDER>
 static KernelInfo info_one() {
   cudaFuncAttributes at;
-  KernelInfo k;
-  k.fn = reinterpret_cast<const void*>(&net_kernel<T, D, ORDER>);
-  k.regs = (cudaFuncGetAttributes(&at, net_kernel<T, D, ORDER>) == cudaSuccess) ? at.numRegs : 255;
+  KernelInfo k{reinterpret_cast<const void*>(&net_kernel<T, D, ORDER>), 255, 0};
+  if (cudaFuncGetAttributes(&at, net_kernel<T, D, ORDER>) == cudaSuccess) {
+    k.regs = at.numRegs;
+    k.max_threads = at.maxThreadsPerBlock;
+  } else {
+    cudaGetLastError();
+  }
   return k;
 }
 
@@ -35,7 +39,7 @@ static KernelInfo info_one() {
 
 template <typename T>
 static KernelInfo net_kernel_info_impl(int dim, int order) {
-  KernelInfo k{nullptr, 0};
+  KernelInfo k{nullptr, 0, 0};
   if (dim < 1 || dim > 5 || order < 0 || order > 2) return k;
   PDE_DISPATCH(T, dim, order, (k = info_one<T, D, O>()));
   return k;

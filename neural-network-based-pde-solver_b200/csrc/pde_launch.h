@@ -98,6 +98,7 @@ int make_reduce_args(const GradLayout& g, const T* partial, const double* psums,
 struct KernelInfo {
   const void* fn;
   int regs;
+  int max_threads;   // cudaFuncAttributes::maxThreadsPerBlock, the largest block a launch accepts (0: unknown)
 };
 
 // kernel handle for (dim, order); nullptr if out of range

@@ -257,6 +257,57 @@ def rayleigh_program(U, d, a=1.0, beta=None):
     return (q1, q2), (U1, U2)
 
 
+def face_blocks(faces, n):
+    """Axis and outward sign of each point of a blocked face batch of n points (include/pde_b200.h): face k is axis
+    k // 2, sign -1 (lo) for even k and +1 (hi) for odd k; one block of n / popcount(faces) points per set bit, in
+    increasing bit order.  Returns (axis, sign), each (n,)."""
+    ks = [k for k in range(faces.bit_length()) if faces >> k & 1]
+    per = n // len(ks)
+    assert per * len(ks) == n, "n must be a multiple of popcount(faces)"
+    k = np.repeat(np.array(ks), per)
+    return k // 2, np.where(k % 2 == 1, 1.0, -1.0)
+
+
+def flux_program(U, d, faces, f=None, alpha=1.0, beta=None):
+    """q = (alpha·s·∂_a u + beta·u − f)² on a blocked face batch (PDE_PROG_FLUX, layout of face_blocks).
+    Returns q (N,1) and ∂(Σq)/∂U; the program has no dq/dE."""
+    u = U[:, 0:1]
+    ax, s = face_blocks(faces, U.shape[0])
+    rows = np.arange(U.shape[0])
+    un = (s * U[rows, 1 + ax]).reshape(-1, 1)
+    bt = 0.0 if beta is None else beta
+    r = alpha * un + bt * u - (0.0 if f is None else f)
+    Ubar = np.zeros_like(U)
+    Ubar[:, 0:1] = 2.0 * r * bt
+    Ubar[rows, 1 + ax] = (2.0 * r * alpha).reshape(-1) * s
+    return r * r, Ubar
+
+
+def ritz_value_program(U, f=None, alpha=0.0, beta=None):
+    """q = ½·beta·u² − g·u with g = f, or the constant alpha when f is None (PDE_PROG_RITZ_VALUE, order 0).
+    Returns q (N,1) and ∂(Σq)/∂U; the program has no dq/dE."""
+    u = U[:, 0:1]
+    bt = 0.0 if beta is None else beta
+    g = alpha if f is None else f
+    Ubar = np.zeros_like(U)
+    Ubar[:, 0:1] = bt * u - g
+    return 0.5 * bt * u * u - g * u, Ubar
+
+
+def parabolic_program(U, d, f=None, alpha=-1.0, beta=None, E=0.0):
+    """q = (∂_{d−1}u + alpha·Σ_{i<d−1} ∂²_i u + (beta−E)·u − f)², time the last coordinate (PDE_PROG_PARABOLIC, order 2).
+    Returns q (N,1), ∂(Σq)/∂U and ∂(Σq)/∂E = Σ −2 r u."""
+    u = U[:, 0:1]
+    lap = np.sum(U[:, 1 + d:2 * d], axis=1, keepdims=True)
+    bt = 0.0 if beta is None else beta
+    r = U[:, d:d + 1] + alpha * lap + (bt - E) * u - (0.0 if f is None else f)
+    Ubar = np.zeros_like(U)
+    Ubar[:, 0:1] = 2.0 * r * (bt - E)
+    Ubar[:, d:d + 1] = 2.0 * r
+    Ubar[:, 1 + d:2 * d] = 2.0 * r * alpha
+    return r * r, Ubar, float(np.sum(-2.0 * r * u))
+
+
 def bump_weight(X, lo, hi, eps_den=0.0, I1=0.210987):
     """WAN cut-off w = Π φ(t_i), φ(t)=exp(1/(t²−1+eps_den))/I1 for |t|<1 else 0, and ∇w.
 

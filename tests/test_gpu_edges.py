@@ -6,7 +6,9 @@ shapes the other parity tests use stay well inside that envelope; here the ABI i
 structs, every output buffer and the workspace belong to the test (so they can be poisoned), and the reference is the
 float64 numpy oracle (oracle/jets_numpy).  The cases sit where kernels go wrong: one hidden layer, width 1 (padded to 8
 units) and 256 (two warps per point, W streamed in K-chunks), the deepest net, tile tails, tensor-core options that the
-reference shapes never reach, and the decline edges between the two kernel families.
+reference shapes never reach, and the decline edges between the two kernel families.  Every program of the header runs
+here: PINN, DRM, RAYLEIGH and MSE, the boundary flux (FLUX, on the blocked face layout), the Ritz value term (RITZ) and
+the space-time parabolic residual (PARABOLIC), the last three also with the fields the header says they ignore (g).
 
 Bars: 1e-10 in fp64 and 1e-5 in fp32 (conftest.BASE_TOL), on the sums, on every parameter gradient
 (conftest.assert_grads_close) and on dE.  Inputs of fp32 cases are fp32-representable, so the oracle sees exactly
@@ -25,9 +27,10 @@ pytestmark = pytest.mark.gpu
 
 PAD = 16            # elements past the end of every output buffer; a call must leave them as they were
 POISON = 0xFF       # all-ones bytes: NaN in fp32 and fp64
-PINN, DRM, RAYLEIGH, MSE = 1, 2, 3, 4
-ORDER = {PINN: 2, DRM: 1, RAYLEIGH: 1, MSE: 0}
-NQ = {PINN: 1, DRM: 1, RAYLEIGH: 2, MSE: 1}
+PINN, DRM, RAYLEIGH, MSE, FLUX, RITZ, PARABOLIC = 1, 2, 3, 4, 5, 7, 9
+ORDER = {PINN: 2, DRM: 1, RAYLEIGH: 1, MSE: 0, FLUX: 1, RITZ: 0, PARABOLIC: 2}
+NQ = {PINN: 1, DRM: 1, RAYLEIGH: 2, MSE: 1, FLUX: 1, RITZ: 1, PARABOLIC: 1}
+NAME = {PINN: "pinn", DRM: "drm", RAYLEIGH: "ray", MSE: "mse", FLUX: "flux", RITZ: "ritz", PARABOLIC: "par"}
 SIN, TANH = O.SIN, O.TANH
 F32, F64 = torch.float32, torch.float64
 
@@ -142,11 +145,11 @@ def _workspace(net, order, n, fill):
 class _Case:
     """Points, per-point arrays and program of one pde_residual_loss_grad call (float64 host copies + device copies)."""
 
-    def __init__(self, net, env, kind, X, alpha=1.0, f=None, beta=None, beta_const=0.0, E=0.0, energy_ptr=False):
+    def __init__(self, net, env, kind, X, alpha=1.0, f=None, beta=None, beta_const=0.0, E=0.0, energy_ptr=False, faces=0):
         L, _ = _lib()
         dt = net.dtype
         self.net, self.env_c, self.env = net, env[0], env[1]
-        self.kind, self.alpha = kind, alpha
+        self.kind, self.alpha, self.faces = kind, alpha, faces
         self.X = _rnd(X, dt)
         self.n = self.X.shape[0]
         self.f = None if f is None else _rnd(np.asarray(f).reshape(-1, 1), dt)
@@ -157,7 +160,7 @@ class _Case:
         self.bd = None if beta is None else _dev(self.beta.reshape(-1), dt)
         self.Ed = _dev(np.array([self.E]), dt) if energy_ptr else None
         p = L.Program()
-        p.kind, p.alpha, p.beta_const = kind, alpha, self.beta_const
+        p.kind, p.faces, p.alpha, p.beta_const = kind, faces, alpha, self.beta_const
         p.energy_const = 0.0 if energy_ptr else self.E      # with the pointer the constant must not be read
         p.f, p.beta, p.energy = _ptr(self.fd), _ptr(self.bd), _ptr(self.Ed)
         self.prog = p
@@ -212,6 +215,16 @@ class _Case:
             elif kind == RAYLEIGH:
                 (q1, q2), (U1, U2) = O.rayleigh_program(U, d, a, beta)
                 qs, Ub = [q1, q2], w[0] * U1 + w[1] * U2
+            elif kind == FLUX:      # no dq/dE: dE must come back as exactly 0
+                q, U0 = O.flux_program(U, d, self.faces, self.f, a, beta)
+                qs, Ub = [q], w[0] * U0
+            elif kind == RITZ:
+                q, U0 = O.ritz_value_program(U, self.f, a, beta)
+                qs, Ub = [q], w[0] * U0
+            elif kind == PARABOLIC:
+                q, U0, dE0 = O.parabolic_program(U, d, self.f, alpha=a, beta=beta, E=self.E)
+                qs, Ub = [q], w[0] * U0
+                dE, dEs = w[0] * dE0, abs(w[0]) * float(np.sum(np.abs(U0[:, d:d + 1] * u)))   # U0[:, d] = 2 r
             else:
                 r = u - f
                 qs = [r * r]
@@ -247,38 +260,46 @@ HS = (1, 2, 3, 4, 5, 8, 63, 64, 65, 127, 128, 200, 255, 256)
 def test_planner_covers_the_advertised_envelope():
     """pde_workspace_bytes plans, and pde_query_path names a kernel family for, every shape include/pde_b200.h admits:
     both dtypes, dim 1..5, order 0..2, 2..8 Linear layers, widths from 1 to 256 around every padding and chunk edge —
-    at one point and at 8192, with the kernel family chosen automatically and forced onto the tensor cores."""
+    at one point and at 8192, with the kernel family chosen automatically and forced onto the tensor cores.  Every
+    program of each order is asked: MSE and RITZ (order 0), DRM and FLUX on all 2d faces (order 1), PINN and, from
+    d = 2, PARABOLIC (order 2).  The tensor-core kernel has no 5-D parabolic pass, so there PARABOLIC answers 0."""
     L, lib = _lib()
-    progs = {0: MSE, 1: DRM, 2: PINN}
+    progs = {0: (MSE, RITZ), 1: (DRM, FLUX), 2: (PINN, PARABOLIC)}
     refused = []
     for which in ("auto", "tc"):
         with _path(which):
             for dt in (L.F32, L.F64):
                 for d in range(1, 6):
                     for order in range(3):
-                        prog = L.Program()
-                        prog.kind = progs[order]
-                        for nl in range(2, 9):
-                            for H in HS:
-                                net = L.Net()
-                                net.dtype, net.dim, net.n_linear, net.activation = dt, d, nl, L.ACT_SIN
-                                net.widths[0] = d
-                                for l in range(1, nl):
-                                    net.widths[l] = H
-                                net.widths[nl] = 1
-                                for n in (1, 8192):
-                                    nb = C.c_size_t(0)
-                                    rc = lib.pde_workspace_bytes(C.byref(net), order, n, C.byref(nb))
-                                    path = lib.pde_query_path(C.byref(net), C.byref(prog), n)
-                                    if rc != 0 or nb.value == 0 or path not in (0, 1):
-                                        refused.append(("f64" if dt == L.F64 else "f32", f"d={d}", f"order={order}",
-                                                        f"n_linear={nl}", f"H={H}", f"n={n}", which, rc, path))
+                        for kind in progs[order]:
+                            if kind == PARABOLIC and d == 1:
+                                continue
+                            prog = L.Program()
+                            prog.kind = kind
+                            prog.faces = (1 << 2 * d) - 1 if kind == FLUX else 0
+                            for nl in range(2, 9):
+                                for H in HS:
+                                    net = L.Net()
+                                    net.dtype, net.dim, net.n_linear, net.activation = dt, d, nl, L.ACT_SIN
+                                    net.widths[0] = d
+                                    for l in range(1, nl):
+                                        net.widths[l] = H
+                                    net.widths[nl] = 1
+                                    for n in (1, 8192):
+                                        nb = C.c_size_t(0)
+                                        rc = lib.pde_workspace_bytes(C.byref(net), order, n, C.byref(nb))
+                                        path = lib.pde_query_path(C.byref(net), C.byref(prog), n)
+                                        ok = (0,) if kind == PARABOLIC and d == 5 else (0, 1)
+                                        if rc != 0 or nb.value == 0 or path not in ok:
+                                            refused.append(("f64" if dt == L.F64 else "f32", f"d={d}", NAME[kind],
+                                                            f"n_linear={nl}", f"H={H}", f"n={n}", which, rc, path))
     assert not refused, f"{len(refused)} shapes inside the header's envelope refused: {refused}"
 
 
 # ================================================================================================ (b) generic kernel
 # dtype, d, n_linear, H, activation, program, envelope (kind, lo, hi, nodes), N, energy through the pointer
 ENV_POLY02 = (O.ENV_POLY, 0.0, 2.0, ())
+ENV_NONE02 = (O.ENV_NONE, 0.0, 2.0, ())
 GENERIC = [
     (F64, 5, 8, 256, SIN, PINN, ENV_POLY02, 7, True),          # the widest, deepest fp64 order-2 net: KC below default
     (F64, 5, 8, 255, TANH, RAYLEIGH, ENV_POLY02, 2, False),
@@ -296,16 +317,48 @@ GENERIC = [
     (F32, 3, 8, 5, TANH, MSE, ENV_POLY02, 1, False),
     (F32, 1, 3, 256, TANH, RAYLEIGH, ENV_POLY02, 1000, False),
     (F32, 2, 8, 255, SIN, DRM, (O.ENV_EXPWIN, 0.0, 2.0, ()), 149, False),
+    # FLUX: one point per face (N = 2d), a single face (149 is prime), five and eight faces of 1000 points
+    (F64, 5, 8, 256, TANH, FLUX, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(8), (), _cheb(3))), 10, False),
+    (F32, 2, 2, 1, SIN, FLUX, ENV_NONE02, 149, False),
+    (F64, 3, 2, 3, TANH, FLUX, (O.ENV_POLY, -2.0, 2.0, (_cheb(8), [0.5])), 1000, False),
+    (F32, 4, 8, 255, SIN, FLUX, ENV_NONE02, 1000, False),
+    # RITZ: f = NULL (g = alpha) at odd N
+    (F64, 5, 8, 256, SIN, RITZ, (O.ENV_POLY, 0.0, 2.0, ((), _cheb(8, 0.0, 2.0))), 1000, False),
+    (F32, 3, 2, 1, TANH, RITZ, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(3), _cheb(8), ())), 1000, False),
+    (F64, 1, 8, 3, TANH, RITZ, ENV_POLY02, 1, False),
+    (F32, 2, 2, 255, SIN, RITZ, ENV_NONE02, 7, False),
+    # PARABOLIC: no envelope (the library refuses one)
+    (F64, 5, 8, 256, SIN, PARABOLIC, ENV_NONE02, 7, True),
+    (F64, 2, 2, 1, TANH, PARABOLIC, ENV_NONE02, 1000, True),
+    (F32, 3, 8, 3, SIN, PARABOLIC, ENV_NONE02, 1, False),
+    (F32, 4, 2, 255, TANH, PARABOLIC, ENV_NONE02, 1000, True),
 ]
 
 
 def _ids(cases):
-    return ["-".join(str(v).replace("torch.", "") for v in (c[0], f"d{c[1]}", f"nl{c[2]}", f"H{c[3]}",
-                                                             {PINN: "pinn", DRM: "drm", RAYLEIGH: "ray", MSE: "mse"}[c[5]],
+    return ["-".join(str(v).replace("torch.", "") for v in (c[0], f"d{c[1]}", f"nl{c[2]}", f"H{c[3]}", NAME[c[5]],
                                                              f"n{c[7]}")) for c in cases]
 
 
+def _flux_mask(d, N):
+    """The face mask with the most faces whose count divides N (of those, the top bits): a FLUX batch of N points is
+    popcount(mask) equal blocks."""
+    p = max(k for k in range(1, 2 * d + 1) if N % k == 0)
+    return ((1 << 2 * d) - 1) ^ ((1 << (2 * d - p)) - 1)
+
+
+def _on_faces(X, faces, lo, hi):
+    """Puts each block of a FLUX batch on its face: the face coordinate of the block's points set to lo or hi."""
+    ax, s = O.face_blocks(faces, X.shape[0])
+    X[np.arange(X.shape[0]), ax] = np.where(s > 0, hi, lo)
+    return X
+
+
 def _case(dtype, d, nl, H, act, kind, env, N, energy_ptr, seed=0):
+    """One call of program `kind`.  PINN, DRM and MSE get white-noise f, PINN and RAYLEIGH per-point beta.  FLUX, RITZ
+    and PARABOLIC get one-signed f (see test_tc_tile_edges_vs_oracle for why): FLUX on the faces of _flux_mask(d, N)
+    with a per-point Robin beta on tanh nets and a constant one on sin nets; RITZ with beta >= 0 chosen the same way and
+    f = NULL (g = alpha) when N is odd; PARABOLIC with alpha < 0, per-point beta and no envelope."""
     rng = np.random.default_rng(seed + 1000 * d + 10 * nl + H + N)
     Ws, bs = _rand_net(rng, d, H, nl, dtype)
     net = _Net(Ws, bs, act, dtype)
@@ -313,9 +366,24 @@ def _case(dtype, d, nl, H, act, kind, env, N, energy_ptr, seed=0):
     X = _points(rng, N, d, lo + 0.05 * (hi - lo), hi - 0.05 * (hi - lo))
     f = rng.normal(size=N) if kind in (PINN, DRM, MSE) else None
     beta = rng.uniform(0.5, 1.5, N) if kind in (PINN, RAYLEIGH) else None
-    alpha = {PINN: -0.5, DRM: 0.5, RAYLEIGH: 0.75, MSE: 1.0}[kind]
-    return _Case(net, _envelope(kind_e, lo, hi, nodes, dtype), kind, X, alpha=alpha, f=f, beta=beta, E=0.375,
-                 energy_ptr=energy_ptr)
+    alpha = {PINN: -0.5, DRM: 0.5, RAYLEIGH: 0.75, MSE: 1.0, FLUX: 0.75, RITZ: -1.25, PARABOLIC: -0.375}[kind]
+    beta_const, faces = 0.0, 0
+    if kind in (FLUX, RITZ, PARABOLIC):
+        f = rng.uniform(1.0, 2.0, N)
+        if kind == PARABOLIC:
+            assert kind_e == O.ENV_NONE and not nodes, "PARABOLIC takes no envelope"
+            beta = rng.uniform(0.5, 1.5, N)
+        elif act == TANH:
+            beta = rng.uniform(0.0 if kind == RITZ else 0.5, 1.5, N)
+        else:
+            beta_const = 0.8
+        if kind == RITZ and N % 2:
+            f = None
+        if kind == FLUX:
+            faces = _flux_mask(d, N)
+            X = _on_faces(X, faces, lo, hi)
+    return _Case(net, _envelope(kind_e, lo, hi, nodes, dtype), kind, X, alpha=alpha, f=f, beta=beta,
+                 beta_const=beta_const, E=0.375, energy_ptr=energy_ptr, faces=faces)
 
 
 @pytest.mark.parametrize("dtype,d,nl,H,act,kind,env,N,energy_ptr", GENERIC, ids=_ids(GENERIC))
@@ -325,6 +393,24 @@ def test_generic_kernel_at_the_edges_vs_oracle(dtype, d, nl, H, act, kind, env, 
         got = case.run()
     assert got["path"] == 0
     _assert_matches_oracle(case, got, case.oracle(), f"generic {case.net.c.dim}-D nl{nl} H{H} n{N}")
+
+
+@pytest.mark.parametrize("order", [0, 1, 2])
+@pytest.mark.parametrize("dtype", [F64, F32], ids=["float64", "float32"])
+def test_generic_kernel_launches_its_largest_tiles(dtype, order):
+    """With 64 points per SM the generic kernel's plan takes the largest point tile that shared memory and the block
+    size of the kernel allow, which the point counts above rarely reach.  Every dim at widths of 25, 50 and 64 thread
+    groups per point (H = 100, 200, 256) must launch there and match the oracle.  (The fp32 order-2 4-D kernel uses 197
+    registers: a plan that sized its blocks from the register count alone picked 320 threads, which do not launch.)"""
+    kind = {0: MSE, 1: DRM, 2: PINN}[order]
+    N = 64 * _sms()
+    for d in range(1, 6):
+        for H in (100, 200, 256):
+            case = _case(dtype, d, 2, H, TANH, kind, ENV_POLY02, N, False, seed=7)
+            with _path("simt"):
+                got = case.run()
+            assert got["path"] == 0
+            _assert_matches_oracle(case, got, case.oracle(), f"generic {NAME[kind]} {d}-D H{H} n{N}")
 
 
 # dtype, d, n_linear, H, activation, order, N
@@ -394,6 +480,30 @@ TC = [
     # the 5-D split with everything it evaluates on its own: EXPWIN, nodes, per-point beta, energy pointer, seed
     (5, 4, 48, TANH, PINN, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(2), (), _cheb(8), [0.5], _cheb(3))), 3000, True, [0.3]),
     (5, 5, 64, SIN, PINN, (O.ENV_POLY, -2.0, 2.0, ((), _cheb(4))), 700, False, [-1.75]),
+    # the fused residual step at width 1 and one unit below a full K-chunk
+    (3, 4, 1, SIN, PINN, ENV_POLY02, 1000, True, None),
+    (2, 3, 63, TANH, PINN, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(3), ())), 1500, True, [0.3]),
+    (3, 5, 1, TANH, DRM, ENV_POLY02, 1000, False, None),
+    (4, 4, 63, SIN, DRM, ENV_POLY02, 800, False, [-1.75]),
+    # FLUX (order 1): narrow and odd widths, 2..4 hidden layers, nodes, the face walk across tiles and CTAs
+    (3, 3, 1, SIN, FLUX, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(8), (), _cheb(3))), 1200, False, None),
+    (2, 4, 17, TANH, FLUX, (O.ENV_POLY, -2.0, 2.0, (_cheb(5), [0.25])), 1000, False, [0.3]),
+    (4, 5, 63, SIN, FLUX, ENV_NONE02, 777, False, None),
+    (1, 5, 64, TANH, FLUX, ENV_POLY02, 2000, False, [-1.75]),
+    (5, 3, 3, TANH, FLUX, ENV_NONE02, 4000, False, None),
+    # RITZ (order 0)
+    (3, 3, 3, TANH, RITZ, (O.ENV_POLY, -2.0, 2.0, (_cheb(8), _cheb(2), ())), 1500, False, None),
+    (5, 4, 63, SIN, RITZ, (O.ENV_EXPWIN, -2.0, 2.0, ((), _cheb(4), (), (), _cheb(8))), 999, False, [0.3]),
+    (2, 5, 1, TANH, RITZ, ENV_NONE02, 2000, False, None),
+    (4, 3, 17, SIN, RITZ, ENV_POLY02, 777, False, [-1.75]),
+    (1, 4, 64, TANH, RITZ, (O.ENV_EXPWIN, -2.0, 2.0, (_cheb(8),)), 1001, False, None),
+    # PARABOLIC (the NLAP = d - 1 instantiations), energy through the pointer
+    (2, 3, 1, TANH, PARABOLIC, ENV_NONE02, 1000, True, None),
+    (3, 4, 63, SIN, PARABOLIC, ENV_NONE02, 1500, True, [0.3]),
+    (4, 5, 17, TANH, PARABOLIC, ENV_NONE02, 2000, True, None),
+    (3, 5, 3, SIN, PARABOLIC, ENV_NONE02, 777, True, [-1.75]),
+    (2, 4, 64, SIN, PARABOLIC, ENV_NONE02, 3000, False, None),
+    (4, 3, 64, TANH, PARABOLIC, ENV_NONE02, 1200, True, [0.3]),
 ]
 
 
@@ -444,6 +554,44 @@ def test_tc_tile_edges_vs_oracle(d, tiles):
     _assert_matches_oracle(case, got, case.oracle(), f"tc {d}-D n{N}")
 
 
+@pytest.mark.parametrize("tiles", list(TILE_EDGES))
+@pytest.mark.parametrize("kind", [RITZ, FLUX, PARABOLIC], ids=[NAME[k] for k in (RITZ, FLUX, PARABOLIC)])
+def test_tc_tile_edges_of_the_boundary_and_parabolic_programs_vs_oracle(kind, tiles):
+    """The tile edges of test_tc_tile_edges_vs_oracle at d = 3 for RITZ, FLUX and PARABOLIC, with one-signed data.
+
+    RITZ keeps the exact tail check: the appended point has two coordinates on the POLY boundary and f = 0, so u = 0 and
+    its cotangent beta u - f is 0.  FLUX runs on the mask with the most faces whose count divides N (N follows the SM
+    count and may be prime; the mask is in every message), and PARABOLIC without an envelope; for those two a point
+    more would change the face layout or contribute, so they are compared with the oracle only."""
+    d = 3
+    N = TILE_EDGES[tiles](_sms())
+    rng = np.random.default_rng(20 + kind + 1000 * d + N)
+    Ws, bs = _rand_net(rng, d, 64, 5, F32)
+    net = _Net(Ws, bs, TANH, F32)
+    faces = _flux_mask(d, N) if kind == FLUX else 0
+    env = _envelope(O.ENV_NONE if kind == PARABOLIC else O.ENV_POLY, 0.0, 2.0, (), F32)
+    X = _points(rng, N, d)
+    if kind == FLUX:
+        X = _on_faces(X, faces, 0.0, 2.0)
+    f, beta = rng.uniform(1.0, 2.0, N), rng.uniform(0.5, 1.5, N)
+    alpha = {RITZ: -1.25, FLUX: 0.75, PARABOLIC: -0.375}[kind]
+    case = _Case(net, env, kind, X, alpha=alpha, f=f, beta=beta, E=0.375, energy_ptr=True, faces=faces)
+    what = f"tc {NAME[kind]} {d}-D n{N} faces={faces:#b}"
+    with _path("tc"):
+        got = case.run()
+        if kind == RITZ:
+            inert = np.ones((1, d))
+            inert[0, :2] = 0.0
+            padded = _Case(net, env, kind, np.concatenate([X, inert]), alpha=alpha, f=np.append(f, 0.0),
+                           beta=np.append(beta, 1.0), E=0.375, energy_ptr=True)
+            more = padded.run(inv_n=1.0 / N)
+            assert more["path"] == 1
+            for k, n in (("sums", 1), ("grad", net.n_params), ("dE", 1)):
+                assert torch.equal(_bytes(more[k], n), _bytes(got[k], n)), k
+    assert got["path"] == 1, what
+    _assert_matches_oracle(case, got, case.oracle(), what)
+
+
 # n_linear, H, expected family at 8192 points (automatic choice)
 DECLINE = [(3, 64, 1), (5, 64, 1), (2, 64, 0), (6, 64, 0), (4, 65, 0)]
 
@@ -461,18 +609,38 @@ def test_tc_decline_edges(nl, H, family):
     _assert_matches_oracle(case, got, case.oracle(), f"auto nl{nl} H{H}")
 
 
+# d, n_linear, H, expected family at 8192 points (automatic choice)
+PARABOLIC_DECLINE = [(3, 4, 64, 1), (2, 2, 64, 0), (2, 6, 64, 0), (2, 4, 65, 0), (5, 4, 64, 0)]
+
+
+@pytest.mark.parametrize("d,nl,H,family", PARABOLIC_DECLINE)
+def test_tc_decline_edges_of_the_parabolic_program(d, nl, H, family):
+    """PARABOLIC declines like PINN (one hidden layer, five, or width 65) and also at d = 5, where the tensor-core
+    kernel has no split pass for it: the generic kernel serves those calls and every call matches the oracle."""
+    case = _case(F32, d, nl, H, SIN, PARABOLIC, ENV_NONE02, 8192, True, seed=3)
+    with _path("auto"):
+        assert case.query_path() == family
+        got = case.run()
+    assert got["path"] == family
+    _assert_matches_oracle(case, got, case.oracle(), f"auto parabolic d{d} nl{nl} H{H}")
+
+
 # ================================================================================================ (d) seed and inv_n
 # family, dtype, d, n_linear, H, program, N, seed
 LINEAR = [("simt", F64, 2, 3, 20, RAYLEIGH, 500, [0.3, -2.0]), ("simt", F32, 1, 4, 33, PINN, 300, [0.3]),
           ("tc", F32, 3, 5, 64, PINN, 5000, [0.3]), ("tc", F32, 2, 4, 64, RAYLEIGH, 3000, [0.3, -2.0]),
-          ("tc", F32, 5, 5, 64, PINN, 2000, [0.3])]
+          ("tc", F32, 5, 5, 64, PINN, 2000, [0.3]),
+          ("simt", F64, 3, 4, 20, FLUX, 600, [0.3]), ("simt", F32, 2, 3, 33, RITZ, 300, [-2.0]),
+          ("simt", F64, 3, 3, 20, PARABOLIC, 500, [0.3]), ("tc", F32, 3, 5, 64, FLUX, 3000, [0.3]),
+          ("tc", F32, 2, 4, 17, RITZ, 3000, [-2.0]), ("tc", F32, 3, 4, 64, PARABOLIC, 5000, [0.3])]
 
 
 @pytest.mark.parametrize("family,dtype,d,nl,H,kind,N,seed", LINEAR)
 def test_seed_and_inv_n_are_linear(family, dtype, d, nl, H, kind, N, seed):
     """With a seed s and an arbitrary inv_n the gradient and dE are inv_n n sum_k s_k (those of seed e_k, inv_n = 1/n),
     the NULL seed is the all-ones seed, and the sums do not depend on either, bit for bit."""
-    case = _case(dtype, d, nl, H, SIN, kind, ENV_POLY02, N, kind == PINN, seed=4)
+    case = _case(dtype, d, nl, H, SIN, kind, ENV_NONE02 if kind == PARABOLIC else ENV_POLY02, N,
+                 kind in (PINN, PARABOLIC), seed=4)
     inv_n = 0.625 / N
     K = NQ[kind]
     with _path(family):
@@ -489,7 +657,7 @@ def test_seed_and_inv_n_are_linear(family, dtype, d, nl, H, kind, N, seed):
     assert float((sum(g) - base["grad"].double()).abs().max()) <= tol * scale
     want = inv_n * N * sum(float(sk) * gk for sk, gk in zip(s, g))
     assert float((got["grad"].double() - want).abs().max()) <= tol * scale * inv_n * N * max(abs(s))
-    if kind == PINN:
+    if kind in (PINN, PARABOLIC):
         dE1 = float(units[0]["dE"][0])
         assert float(base["dE"][0]) == pytest.approx(dE1, rel=tol, abs=0)
         assert float(got["dE"][0]) == pytest.approx(inv_n * N * float(s[0]) * dE1, rel=tol, abs=0)
@@ -498,27 +666,52 @@ def test_seed_and_inv_n_are_linear(family, dtype, d, nl, H, kind, N, seed):
 # ================================================================================================ (e) output contract
 # family, dtype, d, n_linear, H, program, N
 CONTRACT = [("simt", F64, 2, 3, 20, PINN, 300), ("simt", F32, 1, 4, 256, RAYLEIGH, 149), ("tc", F32, 3, 5, 64, PINN, 1000),
-            ("tc", F32, 2, 4, 64, RAYLEIGH, 5000), ("tc", F32, 5, 5, 64, PINN, 500)]
+            ("tc", F32, 2, 4, 64, RAYLEIGH, 5000), ("tc", F32, 5, 5, 64, PINN, 500),
+            ("simt", F64, 3, 4, 20, FLUX, 300), ("simt", F32, 2, 8, 256, RITZ, 149), ("simt", F64, 4, 3, 20, PARABOLIC, 300),
+            ("tc", F32, 3, 5, 64, FLUX, 996), ("tc", F32, 2, 3, 63, RITZ, 1000), ("tc", F32, 3, 4, 64, PARABOLIC, 1000)]
 
 
 @pytest.mark.parametrize("family,dtype,d,nl,H,kind,N", CONTRACT)
 def test_residual_outputs_and_workspace_carry_no_state(family, dtype, d, nl, H, kind, N):
     """sums, grad and energy_grad are pure outputs and the workspace holds nothing across calls: with every byte of
     them NaN beforehand the results are bit-identical to a run on zeroed buffers, nothing past their ends is written,
-    and grad = NULL with energy_grad set still gives the same dE and sums."""
-    case = _case(dtype, d, nl, H, TANH, kind, ENV_POLY02, N, kind == PINN, seed=5)
+    grad = NULL with energy_grad set still gives the same dE and sums (that call still runs the reverse sweep), and the
+    sums-only call (grad and energy_grad NULL, no reverse sweep) gives the same sums."""
+    case = _case(dtype, d, nl, H, TANH, kind, ENV_NONE02 if kind == PARABOLIC else ENV_POLY02, N,
+                 kind in (PINN, PARABOLIC), seed=5)
     K = NQ[kind]
     with _path(family):
         clean = case.run(fill=0)
         dirty = case.run(fill=POISON)
         no_grad = case.run(fill=POISON, grad=False)
-    assert clean["path"] == dirty["path"] == no_grad["path"] == (1 if family == "tc" else 0)
-    assert clean["intact"] and dirty["intact"] and no_grad["intact"]
+        sums_only = case.run(fill=POISON, grad=False, dE=False)
+    assert clean["path"] == dirty["path"] == no_grad["path"] == sums_only["path"] == (1 if family == "tc" else 0)
+    assert clean["intact"] and dirty["intact"] and no_grad["intact"] and sums_only["intact"]
     for k, n in (("sums", K), ("grad", case.net.n_params), ("dE", 1)):
         assert torch.equal(_bytes(dirty[k], n), _bytes(clean[k], n)), k
     assert torch.equal(_bytes(no_grad["sums"], K), _bytes(clean["sums"], K))
     assert torch.equal(_bytes(no_grad["dE"], 1), _bytes(clean["dE"], 1))
+    assert torch.equal(_bytes(sums_only["sums"], K), _bytes(clean["sums"], K))
     assert torch.isfinite(clean["grad"]).all() and torch.isfinite(clean["sums"]).all()
+
+
+@pytest.mark.parametrize("kind", [RITZ, FLUX, PARABOLIC, PINN, DRM], ids=[NAME[k] for k in (RITZ, FLUX, PARABOLIC, PINN, DRM)])
+def test_tc_sums_only_call_over_three_tiles_per_cta(kind):
+    """Without grad and energy_grad the tensor-core kernel runs forward only, and the two-slot W plan has to bring the
+    first hidden layer's weights back for every tile by itself: over three tiles per CTA (and a tail) the sums must be
+    bit-identical to the training call's — for the order-0 RITZ and order-1 FLUX branches, the PARABOLIC (NLAP = d - 1)
+    instantiation and, at these widths, PINN and DRM."""
+    N = 64 * _sms() * 3 + 29
+    env = ENV_NONE02 if kind == PARABOLIC else ENV_POLY02
+    case = _case(F32, 3, 5, 64, SIN, kind, env, N, kind in (PINN, PARABOLIC), seed=9)
+    with _path("tc"):
+        train = case.run(fill=POISON)
+        sums_only = case.run(fill=POISON, grad=False, dE=False)
+    assert train["path"] == sums_only["path"] == 1
+    assert train["intact"] and sums_only["intact"]
+    assert torch.isfinite(train["sums"]).all() and torch.isfinite(train["grad"]).all()
+    assert torch.equal(_bytes(sums_only["sums"], 1), _bytes(train["sums"], 1)), (float(sums_only["sums"][0]),
+                                                                                  float(train["sums"][0]))
 
 
 @pytest.mark.parametrize("family,dtype,d,nl,H,order,N", [("simt", F64, 3, 4, 20, 2, 300), ("simt", F32, 2, 2, 256, 1, 149),
@@ -538,6 +731,70 @@ def test_jets_outputs_and_workspace_carry_no_state(family, dtype, d, nl, H, orde
     assert torch.equal(_bytes(Jd, Jd.numel()), _bytes(Jc, Jc.numel()))
     assert torch.equal(_bytes(gd, gd.numel()), _bytes(gc, gc.numel()))
     assert torch.isfinite(Jc).all() and torch.isfinite(gc).all()
+
+
+# ================================================================================================ (g) ignored fields
+def _same_outputs(a, b, n_params, what):
+    for k, n in (("sums", 1), ("grad", n_params), ("dE", 1)):
+        assert torch.equal(_bytes(a[k], n), _bytes(b[k], n)), f"{what}: {k}"
+
+
+# family, dtype, d, n_linear, H, N
+IGNORED = [("simt", F64, 3, 3, 20, 300), ("tc", F32, 3, 4, 64, 1200)]
+
+
+@pytest.mark.parametrize("family,dtype,d,nl,H,N", IGNORED, ids=[c[0] for c in IGNORED])
+@pytest.mark.parametrize("kind", [FLUX, RITZ], ids=[NAME[k] for k in (FLUX, RITZ)])
+def test_energy_fields_are_ignored_by_flux_and_ritz(kind, family, dtype, d, nl, H, N):
+    """FLUX and RITZ ignore the energy fields and have dq/dE = 0: with `energy` pointing at NaN and energy_const = NaN,
+    sums and grad are bit-identical to a call with energy = NULL, and energy_grad is written as exactly 0 over a
+    NaN-filled buffer."""
+    case = _case(dtype, d, nl, H, TANH, kind, ENV_POLY02, N, False, seed=11)
+    with _path(family):
+        base = case.run(fill=POISON)
+        nan = _dev(np.array([np.nan]), dtype)
+        case.prog.energy, case.prog.energy_const = nan.data_ptr(), float("nan")
+        got = case.run(fill=POISON)
+    assert base["path"] == got["path"] == (1 if family == "tc" else 0)
+    assert got["intact"]
+    for k, n in (("sums", 1), ("grad", case.net.n_params)):
+        assert torch.equal(_bytes(got[k], n), _bytes(base[k], n)), k
+    assert float(got["dE"][0]) == 0.0 and float(base["dE"][0]) == 0.0, (float(got["dE"][0]), float(base["dE"][0]))
+
+
+@pytest.mark.parametrize("family,dtype,d,nl,H,N", IGNORED, ids=[c[0] for c in IGNORED])
+@pytest.mark.parametrize("kind", [PINN, RITZ, PARABOLIC], ids=[NAME[k] for k in (PINN, RITZ, PARABOLIC)])
+def test_face_mask_is_ignored_by_every_program_but_flux(kind, family, dtype, d, nl, H, N):
+    """`faces` is read by FLUX alone: a mask of 0x155 (not even a valid mask at d = 3) leaves sums, grad and dE
+    bit-identical to faces = 0."""
+    env = ENV_NONE02 if kind == PARABOLIC else ENV_POLY02
+    case = _case(dtype, d, nl, H, SIN, kind, env, N, kind != RITZ, seed=12)
+    with _path(family):
+        base = case.run(fill=POISON)
+        case.prog.faces = 0x155
+        got = case.run(fill=POISON)
+    assert base["path"] == got["path"] == (1 if family == "tc" else 0)
+    assert got["intact"]
+    _same_outputs(got, base, case.net.n_params, f"{NAME[kind]} faces=0x155")
+
+
+@pytest.mark.parametrize("family,dtype,d,nl,H,N", IGNORED, ids=[c[0] for c in IGNORED])
+def test_ritz_constant_g_is_alpha(family, dtype, d, nl, H, N):
+    """RITZ with f = NULL uses g = alpha: bit-identical to f = an array of that constant (with alpha = NaN, which a
+    call with f must not read)."""
+    c = -1.25
+    base = _case(dtype, d, nl, H, TANH, RITZ, ENV_POLY02, N + 1, False, seed=13)     # N + 1 odd: f = NULL
+    assert base.f is None
+    base.prog.alpha = c
+    with_f = _Case(base.net, (base.env_c, base.env), RITZ, base.X, alpha=float("nan"), f=np.full(base.n, c), beta=base.beta,
+                   beta_const=base.beta_const, E=base.E)
+    with _path(family):
+        a = base.run(fill=POISON)
+        b = with_f.run(fill=POISON)
+    assert a["path"] == b["path"] == (1 if family == "tc" else 0)
+    assert a["intact"] and b["intact"]
+    _same_outputs(a, b, base.net.n_params, "f = NULL, alpha = c vs f = c")
+    assert torch.isfinite(a["grad"]).all() and torch.isfinite(a["sums"]).all()
 
 
 # ================================================================================================ (f) WAN pointwise

@@ -489,3 +489,81 @@ def test_reference_spread_is_recorded_for_every_fixture():
     # losses and gradient tensors: a one-ulp perturbation moves nothing by more than ~1e-12 relative to the tensor's
     # largest entry, so no float64 bar is loosened on conditioning grounds
     assert worst < 1e-12, worst
+
+
+# ---------------------------------------------------------------- the flux, Ritz-value and parabolic programs
+def _program_cases():
+    """(program, d, bc, beta, f, faces) over d = 1..5 (parabolic 2..5), both envelopes, per-point and constant beta, f
+    given and None; the flux program on one face, on all 2d faces and on a sparse mask of both ends of the face bits."""
+    out = []
+    for prog in ("flux", "ritz", "parabolic"):
+        for d in range(2 if prog == "parabolic" else 1, 6):
+            masks = {"one": 1 << (3 * d % (2 * d)), "all": (1 << 2 * d) - 1} if prog == "flux" else {"": 0}
+            if prog == "flux" and d == 5:
+                masks["sparse"] = 0b1000000001
+            for bc in ("FBC", "RB"):
+                for beta in ("point", "const"):
+                    for f in ("f", "nof"):
+                        for mname, faces in masks.items():
+                            out.append(pytest.param(prog, d, bc, beta, f, faces,
+                                                    id="-".join(x for x in (prog, f"d{d}", bc, beta, f, mname) if x)))
+    return out
+
+
+@pytest.mark.parametrize("prog,d,bc,beta,f,faces", _program_cases())
+def test_numpy_programs_match_the_autograd_specifications(prog, d, bc, beta, f, faces):
+    """oracle/jets_numpy's flux_program, ritz_value_program and parabolic_program through _loss_and_grads equal the
+    float64 nested-autograd specifications the GPU suites are checked against (tests/flux_oracle, ritz_oracle,
+    heat_oracle): the mean, every parameter gradient and, for the parabolic program, d mean / dE."""
+    from flux_oracle import flux_loss
+    from heat_oracle import parabolic_loss
+    from ritz_oracle import ritz_value_loss
+    rng = np.random.default_rng([("flux", "ritz", "parabolic").index(prog), d, bc == "FBC", beta == "point", f == "f", faces])
+    L, H, act = 2.0, 10, (O.TANH if d % 2 else O.SIN)
+    widths = [d, H, H, 1]
+    Ws = [rng.uniform(-1, 1, (o, i)) / math.sqrt(i) for i, o in zip(widths[:-1], widths[1:])]
+    bs = [rng.uniform(-0.5, 0.5, o) for o in widths[1:]]
+    nf = bin(faces).count("1")
+    N = 6 * nf if prog == "flux" else 23
+    X = rng.uniform(0.1 * L, 0.9 * L, (N, d))
+    if prog == "flux":      # the face coordinate of each block on its side of the box
+        ax, s = O.face_blocks(faces, N)
+        X[np.arange(N), ax] = np.where(s > 0, L, 0.0)
+    bt = rng.uniform(0.5, 1.5, (N, 1)) if beta == "point" else 0.625
+    fv = rng.normal(size=(N, 1)) if f == "f" else None
+    alpha = {"flux": 0.75, "ritz": -1.25, "parabolic": -0.3}[prog]
+    E = 0.375
+    env = {"kind": O.ENV_POLY if bc == "FBC" else O.ENV_NONE, "lo": 0.0, "hi": L}
+    order = {"flux": 1, "ritz": 0, "parabolic": 2}[prog]
+
+    def program(U):
+        dE = 0.0
+        if prog == "flux":
+            q, Ub = O.flux_program(U, d, faces, fv, alpha, bt)
+        elif prog == "ritz":
+            q, Ub = O.ritz_value_program(U, fv, alpha, bt)
+        else:
+            q, Ub, dE = O.parabolic_program(U, d, fv, alpha, bt, E)
+        return float(q.mean()), Ub / N, dE / N
+
+    loss, gWs, gbs, dE = O._loss_and_grads(Ws, bs, X, act, order, env, program)
+
+    net = AR.build_mlp(widths, "tanh" if act == O.TANH else "sin", torch.float64)
+    AR.load_params(net, Ws, bs)
+    Xt = torch.tensor(X).requires_grad_(prog != "ritz")
+    bt_t = torch.tensor(bt) if beta == "point" else bt
+    f_t = None if fv is None else torch.tensor(fv)
+    Et = torch.tensor(E, dtype=torch.float64, requires_grad=True)
+    if prog == "flux":
+        spec = flux_loss(net, Xt, faces, f_t, L, bc, alpha=alpha, kappa=bt_t)
+    elif prog == "ritz":
+        spec = ritz_value_loss(net, Xt, f_t, L, bc, kappa=bt_t, alpha=alpha)
+    else:
+        spec = parabolic_loss(net, Xt, f_t, alpha, bt_t, Et, L, bc)
+    spec.backward()
+    ps = [p.grad.numpy() for p in net.parameters()]
+    tol = 1e-12
+    assert abs(loss - float(spec.detach())) <= tol * max(1.0, abs(float(spec.detach()))), (loss, float(spec.detach()))
+    assert_grads_close((gWs, gbs), (ps[0::2], ps[1::2]), tol, f"{prog} d{d} {bc}")
+    if prog == "parabolic":
+        assert abs(dE - float(Et.grad)) <= tol * max(1.0, abs(float(Et.grad))), (dE, float(Et.grad))
